@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU baseline arm (rank 0 only)
+    python bench.py ... --dump-outputs DIR                    # also write the lists the last timed step returned, DIR/*.npy
+
+Each timed region of the headline runs exactly K steps.  The steps cycle through a pool of 4 seeded query batches, so
+the inputs, and which batch the last timed step runs, depend only on the arguments.
 
 HEADLINE (BASELINE.json `metric`, first half): hybrid top-100 queries/sec — BM25 + cosine + reciprocal rank fusion
 over a 768-dim bf16 corpus with a 1M-term Zipf vocabulary, 256 queries per step.  The corpus is the largest one
@@ -30,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 DIM, TOPK, BATCH, VOCAB, QTERMS, RRF_K = 768, 100, 256, 1_000_000, 8, 60
 N_DOCS_TOTAL = 50_000_000
@@ -271,6 +276,9 @@ def time_hybrid(ix, dev, cdf, dist, steps, warmup, rank, local_rank, sample_cloc
     barrier()
     ms = allmax(ev0.elapsed_time(ev1))
     launches = ix.launch_count() - l0
+    # what the last timed step returned, copied before the leg timings below reuse the output buffers
+    last_out = (d_out[0].cpu().numpy().view(np.uint32), d_rrf.cpu().numpy(),
+                d_out[1].cpu().numpy().view(np.uint32), d_out[2].cpu().numpy().view(np.uint32))
     clocks = sampler.stop() if (rank == 0 and sample_clocks) else None
     # ---- end-to-end leg: pinned host buffers through the blocking C-ABI call ----
     for i in range(warmup):
@@ -297,7 +305,7 @@ def time_hybrid(ix, dev, cdf, dist, steps, warmup, rank, local_rank, sample_cloc
         ix.set_option("comm_debug_skip_gather", 0)
     step_host(0)  # leave the result of pool entry 0 in the host buffers for the verification
     return {"ms_total": ms, "e2e_s": e2e_s, "launches": launches, "clocks": clocks, "ms_cos": ms_cos, "ms_bm25": ms_bm,
-            "h2d": BATCH * DIM * 4 + BATCH * QTERMS * 4 + (BATCH + 1) * 4, "d2h": BATCH * TOPK * 16,
+            "h2d": BATCH * DIM * 4 + BATCH * QTERMS * 4 + (BATCH + 1) * 4, "d2h": BATCH * TOPK * 16, "last_out": last_out,
             "pool_q": pool, "pool_t": terms, "host_out": (h_out[0].numpy().view(np.uint32).copy(), h_rrf.numpy().copy(),
                                                          h_out[1].numpy().view(np.uint32).copy(), h_out[2].numpy().view(np.uint32).copy())}
 
@@ -364,10 +372,20 @@ def cpu_hybrid_rate(setup, n_total, threads, n_batches, warm=1):
         O.hybrid_batch_fast(rows, pool[i % 4], corp["term_offsets"], corp["doc_ids"], w, terms[i % 4], TOPK, RRF_K, threads)
     t0 = time.perf_counter()
     for i in range(n_batches):
-        O.hybrid_batch_fast(rows, pool[i % 4], corp["term_offsets"], corp["doc_ids"], w, terms[i % 4], TOPK, RRF_K, threads)
+        out = O.hybrid_batch_fast(rows, pool[i % 4], corp["term_offsets"], corp["doc_ids"], w, terms[i % 4], TOPK, RRF_K, threads)
     dt = time.perf_counter() - t0
     scale = n_total / rows.shape[0]
-    return n_batches * BATCH / (dt * scale), dt
+    return n_batches * BATCH / (dt * scale), dt, out
+
+
+def dump_outputs(out_dir, ids, rrf, rank_cos, rank_bm25):
+    """--dump-outputs: the lists one hybrid batch returns to its caller (BATCH x TOPK each), as .npy files that two
+    builds can be compared by.  Doc ids and ranks are written as float64, which holds every uint32 exactly."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a, dt in (("hybrid_ids", ids, np.float64), ("hybrid_rrf", rrf, np.float32),
+                        ("hybrid_rank_cosine", rank_cos, np.float64), ("hybrid_rank_bm25", rank_bm25, np.float64)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(dt))
 
 
 def run_reference(args, rank):
@@ -379,7 +397,9 @@ def run_reference(args, rank):
     threads = O.host_threads()
     slice_docs = args.cpu_slice
     setup = cpu_hybrid_setup(slice_docs, threads)
-    val, dt = cpu_hybrid_rate(setup, args.docs, threads, args.steps, warm=max(1, min(args.warmup, 2)))
+    val, dt, last_out = cpu_hybrid_rate(setup, args.docs, threads, args.steps, warm=max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_out)
     sample = ("%d steps; a step = one %d-query batch scored against a %d-document slice (1/%d of the corpus), scaled by the "
               "corpus/slice ratio; %d OpenMP threads on '%s'" % (args.steps, BATCH, slice_docs, args.docs // slice_docs, threads, _cpu_model()))
     print(json.dumps({
@@ -473,7 +493,10 @@ def main():
     ap.add_argument("--no-verify", action="store_true", help="skip the full-size oracle comparison of the timed output")
     ap.add_argument("--repeats", type=int, default=3, help="timed regions of `steps` steps; the median is reported")
     ap.add_argument("--exchange", default=DEFAULT_EXCHANGE, choices=["nccl", "p2p"], help="transport of the local top-k lists at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -519,6 +542,8 @@ def main():
     e2e_value = n_queries / statistics.median([r["e2e_s"] for r in runs])
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *res["last_out"])
         ms_cos, ms_bm = res["ms_cos"], res["ms_bm25"]
         flops = 2.0 * n_local * DIM * BATCH
         tf = flops / (ms_cos * 1e-3) / 1e12
@@ -533,9 +558,9 @@ def main():
             import oracle as O
             threads = O.host_threads()
             setup = cpu_hybrid_setup(args.cpu_slice, threads)
-            v, dt = cpu_hybrid_rate(setup, args.docs, threads, 4)
+            v, dt, _ = cpu_hybrid_rate(setup, args.docs, threads, 4)
             nb = max(2, min(40, int(12.0 / max(dt / 4, 1e-3))))
-            v, dt = cpu_hybrid_rate(setup, args.docs, threads, nb, warm=0)
+            v, dt, _ = cpu_hybrid_rate(setup, args.docs, threads, nb, warm=0)
             cpu = {"value": v, "unit": UNIT, "cores": threads, "kind": "port",
                    "sample": "%d batches of %d queries against a %d-document slice (1/%d of the corpus) in %.1f s, scaled by the corpus/slice "
                              "ratio; %d OpenMP threads on '%s' (self-written CPU oracle port: no reference implementation of this path exists)"

@@ -47,6 +47,32 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_reference_arm_dumps_the_last_timed_step(tmp_path):
+    # step i scores query batch i % 4: 1 and 5 steps end on the same batch, 2 steps on another
+    import numpy as np
+    dumps = {}
+    for steps in (1, 5, 2):
+        d = tmp_path / str(steps)
+        r = _run(["--impl", "reference", "--steps", str(steps), "--warmup", "1", "--docs", "400000", "--cpu-slice", "20000",
+                  "--dump-outputs", str(d)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        dumps[steps] = {n: np.load(d / (n + ".npy")) for n in ("hybrid_ids", "hybrid_rrf", "hybrid_rank_cosine", "hybrid_rank_bm25")}
+    for steps in (1, 5, 2):
+        a = dumps[steps]
+        assert a["hybrid_rrf"].dtype == np.float32 and a["hybrid_ids"].dtype == np.float64
+        assert all(v.shape == (256, 100) for v in a.values())
+        assert np.all(a["hybrid_ids"] < 20000) and np.all(np.diff(a["hybrid_rrf"], axis=1) <= 0)
+        assert np.all((a["hybrid_rank_cosine"] >= 0) & (a["hybrid_rank_cosine"] <= 100))
+    assert all(np.array_equal(dumps[1][n], dumps[5][n]) for n in dumps[1])
+    assert not np.array_equal(dumps[1]["hybrid_ids"], dumps[2]["hybrid_ids"])
+
+
+def test_steps_must_be_positive():
+    r = _run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_gpu_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():
