@@ -105,6 +105,17 @@ oi_status oi_index_load_bm25(oi_index *h, const uint64_t *term_offsets, const ui
                              const uint32_t *tfs, const uint32_t *doc_len, uint32_t n_terms);
 /* build the synthetic shard-local CSR on the device (SPEC §9); zipf_cdf[vocab] from the host */
 oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vocab, const double *zipf_cdf);
+/* posts -> this shard's BM25 part, on the device: post i = texts[offsets[i] .. offsets[i+1]) (host memory),
+ * n_posts == the shard's n_docs, doc ids local in input order.  Tokenizer = SPEC §6; vocabulary = the distinct tokens
+ * in ascending byte order, term id = rank in it; doc_len = token count; tf = occurrences of the term in the post
+ * (SPEC §3).  Leaves the index exactly as oi_index_load_bm25 with the host IndexBuilder's CSR would: follow with
+ * oi_index_bm25_finalize.  out_n_terms / out_vocab_bytes size the buffers of oi_index_read_vocabulary.  A corpus
+ * without any token is OI_ERR_INVALID_ARG (an index needs a term).  Any failure leaves the index without a BM25 part. */
+oi_status oi_index_build_bm25_text(oi_index *h, const uint8_t *texts, const uint64_t *offsets, uint64_t n_posts,
+                                   uint32_t *out_n_terms, uint64_t *out_vocab_bytes);
+/* the vocabulary of the last oi_index_build_bm25_text: term t = bytes[offsets[t] .. offsets[t+1]), offsets[n_terms+1].
+ * OI_ERR_STATE when the BM25 part did not come from text. */
+oi_status oi_index_read_vocabulary(oi_index *h, uint8_t *bytes, uint64_t *offsets);
 /* this shard's df per term and sum of doc lengths, to be summed over shards by the host */
 oi_status oi_index_bm25_local_stats(oi_index *h, uint32_t *df_out, uint64_t *sum_doc_len,
                                     uint64_t *n_postings);

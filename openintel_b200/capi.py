@@ -69,6 +69,8 @@ def load_library():
         "oi_index_read_embeddings": (st, [H, _vp, C.c_uint64, C.c_uint64]),
         "oi_index_load_bm25": (st, [H, _u64p, _u32p, _u32p, _u32p, C.c_uint32]),
         "oi_index_synth_bm25": (st, [H, C.c_uint64, C.c_uint32, _vp]),
+        "oi_index_build_bm25_text": (st, [H, _vp, _u64p, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
+        "oi_index_read_vocabulary": (st, [H, _vp, _u64p]),
         "oi_index_bm25_local_stats": (st, [H, _u32p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "oi_index_bm25_finalize": (st, [H, C.POINTER(Bm25Params)]),
         "oi_index_read_bm25": (st, [H, _u64p, _u32p, _u32p, _u32p, _f32p]),
@@ -179,6 +181,19 @@ class GpuIndex:
         assert len(cdf) == vocab
         self.n_terms = vocab
         self._ck(self.L.oi_index_synth_bm25(self.h, seed, vocab, _addr(cdf)))
+
+    def build_bm25_text(self, texts):
+        """posts (str or bytes, one per document) -> this shard's BM25 part, tokenized and indexed on the device
+        (oi_index_build_bm25_text); follow with bm25_finalize.  Returns the vocabulary: term id i = list[i]."""
+        blob, offs = pack_texts(texts)
+        nt, nb = C.c_uint32(), C.c_uint64()
+        self._ck(self.L.oi_index_build_bm25_text(self.h, _addr(blob), _addr(offs), len(offs) - 1, C.byref(nt), C.byref(nb)))
+        self.n_terms = nt.value
+        vb = np.empty(max(nb.value, 1), dtype=np.uint8)
+        vo = np.empty(self.n_terms + 1, dtype=np.uint64)
+        self._ck(self.L.oi_index_read_vocabulary(self.h, _addr(vb), _addr(vo)))
+        raw = vb.tobytes()
+        return [raw[vo[t]:vo[t + 1]].decode("ascii") for t in range(self.n_terms)]
 
     def bm25_local_stats(self):
         df = np.empty(self.n_terms, dtype=np.uint32)
@@ -301,8 +316,8 @@ class GpuIndex:
 
 
 def pack_texts(texts):
-    """list of str -> (UTF-8 blob u8[], offsets u64[n + 1]) as the lexicon entry points take them"""
-    raw = [t.encode("utf-8") for t in texts]
+    """list of str (encoded as UTF-8) or bytes -> (blob u8[], offsets u64[n + 1]) as the text entry points take them"""
+    raw = [t.encode("utf-8") if isinstance(t, str) else bytes(t) for t in texts]
     offs = np.zeros(len(raw) + 1, dtype=np.uint64)
     offs[1:] = np.cumsum([len(r) for r in raw])
     blob = np.frombuffer(b"".join(raw) or b"\0", dtype=np.uint8).copy()

@@ -948,6 +948,8 @@ unsigned grid_for(u64 n, int threads, int num_sms) {
   } while (0)
 
 void oi_bm25_free(oi_index *h) {
+  cudaFree(h->d_vocab); cudaFree(h->d_vocab_off);
+  h->d_vocab = nullptr; h->d_vocab_off = nullptr; h->vocab_bytes = 0;
   OiBm25 *b = h->bm25;
   if (!b) return;
   cudaFree(b->d_term_off); cudaFree(b->d_doc_ids); cudaFree(b->d_tfs); cudaFree(b->d_doc_len); cudaFree(b->d_w);
@@ -1034,6 +1036,26 @@ extern "C" oi_status oi_index_load_bm25(oi_index *h, const uint64_t *term_offset
     return h->fail(OI_ERR_INVALID_ARG, "posting %llu: doc id %u outside the shard", (unsigned long long)pb, doc_ids[pb]);
   }
   return bm25_alloc_workspace(h, b);
+}
+
+oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 *d_term_off, uint32_t *d_doc_ids,
+                        uint32_t *d_tfs, uint32_t *d_doc_len) {
+  oi_bm25_free(h);
+  OiBm25 *b = new OiBm25();
+  h->bm25 = b;
+  b->n_terms = n_terms;
+  b->n_postings = n_postings;
+  b->d_term_off = d_term_off;
+  b->d_doc_ids = d_doc_ids;
+  b->d_tfs = d_tfs;
+  b->d_doc_len = d_doc_len;
+  oi_status s = OI_OK;
+  const cudaError_t e = cudaMalloc(&b->d_w, (n_postings ? n_postings : 1) * sizeof(float));
+  if (e != cudaSuccess)
+    s = h->fail(e == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA, "cudaMalloc(weights) failed: %s", cudaGetErrorString(e));
+  if (s == OI_OK) s = bm25_alloc_workspace(h, b);
+  if (s != OI_OK) oi_bm25_free(h);
+  return s;
 }
 
 extern "C" oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vocab, const double *zipf_cdf) {

@@ -85,6 +85,11 @@ struct oi_index {
   int bm25_items_per_warp = 0; // tuning: work items per warp the super-range count aims for (0 = default 16)
   int bm25_no_cold_bound = 0;  // tests: disable the cold-start bound (group maxima) of the selection pass
   int bm25_stage_slots = -1;  // tuning: staged 64-posting chunks per warp (-1 = default, 0 = none)
+  // vocabulary of a BM25 part built from text (text_index.cu): term t = d_vocab[d_vocab_off[t] .. d_vocab_off[t + 1]);
+  // NULL when the BM25 part came from a CSR.  Freed with the BM25 part (oi_bm25_free).
+  uint8_t *d_vocab = nullptr;
+  u64 *d_vocab_off = nullptr;
+  uint64_t vocab_bytes = 0;
 
   // multi-GPU
   OiComm *comm = nullptr;
@@ -98,6 +103,11 @@ struct oi_index {
 
 // bm25.cu
 void oi_bm25_free(oi_index *h);
+// installs a CSR that already lives on the device (text_index.cu) as the BM25 part, as oi_index_load_bm25 leaves it;
+// the arrays become the index's.  On failure they are freed and the index has no BM25 part.
+oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 *d_term_off, uint32_t *d_doc_ids,
+                        uint32_t *d_tfs, uint32_t *d_doc_len);
+uint32_t oi_bm25_n_terms(const oi_index *h);  // 0 = no BM25 part
 uint32_t *oi_bm25_stage_terms(oi_index *h);  // device staging for the host call's flat term array
 uint32_t *oi_bm25_stage_offs(oi_index *h);
 // prep -> blocked scoring -> merge: shard-local sorted key lists d_out_keys[nq][k] (global doc ids)

@@ -24,6 +24,7 @@
 #include <string>
 
 #include "internal.h"
+#include "oi_tokenize.cuh"
 
 namespace {
 
@@ -58,24 +59,6 @@ struct LexSlot { unsigned long long lo, hi; uint32_t flags, pad; };  // flags: 1
 constexpr int kLexSlots = 128;
 __host__ __device__ __forceinline__ uint32_t lex_hash(unsigned long long lo, unsigned long long hi) {
   return (uint32_t)(((lo ^ (hi * 0x9E3779B97F4A7C15ull)) * 0x3CDFA3C5131A5AF7ull) >> 57);
-}
-
-enum { CLS_SEP = 0, CLS_SKIP = -1, CLS_I_THEN_SEP = -2 };  // > 0: a token byte (the lowered char)
-
-// class of byte position i of text[0..len): token char (> 0), separator, transparent, or the
-// 'i' of U+0130 (a token char that also ends the token)
-__device__ __forceinline__ int classify(const uint8_t *t, long long i, long long len) {
-  const uint8_t b = t[i];
-  if (b < 0x80) {
-    if (b >= 'A' && b <= 'Z') return b + 32;
-    if ((b >= 'a' && b <= 'z') || (b >= '0' && b <= '9')) return b;
-    return CLS_SEP;
-  }
-  if (b == 0xE2 && i + 2 < len && t[i + 1] == 0x84 && t[i + 2] == 0xAA) return 'k';
-  if (b == 0x84 && i >= 1 && i + 1 < len && t[i - 1] == 0xE2 && t[i + 1] == 0xAA) return CLS_SKIP;
-  if (b == 0xAA && i >= 2 && t[i - 2] == 0xE2 && t[i - 1] == 0x84) return CLS_SKIP;
-  if (b == 0xC4 && i + 1 < len && t[i + 1] == 0xB0) return CLS_I_THEN_SEP;
-  return CLS_SEP;
 }
 
 constexpr int kStageBytes = 4096;  // per warp: posts up to this many bytes are tokenized from shared memory
@@ -131,7 +114,7 @@ __global__ void __launch_bounds__(256) lexicon_kernel(const uint8_t *texts, cons
       for (long long c0 = 0; c0 < len; c0 += 32) {
         const long long i = c0 + lane;
         const uint32_t b = i < len ? (uint32_t)t[i] : 0x20u;
-        const bool tok = ((b | 0x20u) - 'a') < 26u || (b - '0') < 10u;
+        const bool tok = oi_ascii_token_byte(b);
         const uint32_t m = __ballot_sync(0xFFFFFFFFu, tok);
         const uint32_t starts = m & ~((m << 1) | carry);
         carry = m >> 31;
@@ -159,7 +142,7 @@ __global__ void __launch_bounds__(256) lexicon_kernel(const uint8_t *texts, cons
           if (run) n += lead;
           run = run && lead == 4u;
         }
-        const bool more = run && (((b16 | 0x20u) - 'a') < 26u || (b16 - '0') < 10u);  // a 17th token byte
+        const bool more = run && oi_ascii_token_byte(b16);  // a 17th token byte
         const long long left = len - i;
         if (more && left > 16) continue;  // longer than 16 bytes: cannot match a list word
         if ((long long)n > left) n = (uint32_t)left;

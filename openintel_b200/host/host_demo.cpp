@@ -42,8 +42,9 @@ static int store_mode(int argc, char **argv) {
   const size_t k = std::stoul(argv[5]);
   const uint32_t dim = store.dim();
   if (qemb.size() != qtexts.size() * dim) throw std::runtime_error("query embedding file size mismatch");
-  IndexBuilder ix;
-  const auto search = lift_index(store, ix, 0, (uint32_t)k, (uint32_t)std::max<size_t>(qtexts.size(), 1));
+  Vocabulary vocab;
+  std::vector<std::string> post_ids;
+  const auto search = lift_index(store, vocab, post_ids, 0, (uint32_t)k, (uint32_t)std::max<size_t>(qtexts.size(), 1));
   std::vector<SearchQuery> queries;
   for (size_t j = 0; j < qtexts.size(); ++j) {
     SearchQuery q;
@@ -53,7 +54,7 @@ static int store_mode(int argc, char **argv) {
     const float nrm = std::sqrt(ss);
     if (nrm > 0.0f)
       for (float &v : q.embedding) v /= nrm;
-    q.terms = ix.query_terms(qtexts[j]);
+    q.terms = vocab.query_terms(qtexts[j]);
     queries.push_back(std::move(q));
   }
   const HybridSearch &port = *search;
@@ -61,8 +62,8 @@ static int store_mode(int argc, char **argv) {
   for (size_t j = 0; j < hits.size(); ++j)
     for (size_t i = 0; i < hits[j].size(); ++i)
       std::printf("hit %zu %zu %u %.9g %u %u %s\n", j, i, hits[j][i].doc_id, hits[j][i].rrf, hits[j][i].rank_cosine, hits[j][i].rank_bm25,
-                  ix.post_ids()[hits[j][i].doc_id].c_str());
-  std::printf("store %llu posts dim %u terms %u\n", (unsigned long long)store.n_posts(), dim, ix.n_terms());
+                  post_ids[hits[j][i].doc_id].c_str());
+  std::printf("store %llu posts dim %u terms %u\n", (unsigned long long)store.n_posts(), dim, vocab.size());
   return 0;
 }
 

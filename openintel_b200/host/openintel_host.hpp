@@ -7,7 +7,8 @@
 //   PostAnalyzer           <- src/domain/ports/post_analyzer.rs:7-11 (one signal per post, input order)
 //   HybridSearch           <- new port in the same shape (the reference has no search port: SURVEY.md §0)
 //   tokenize()             <- src/adapters/analyzer/lexicon.rs:54-58
-//   IndexBuilder           <- SURVEY.md §8(f) row 1: posts -> vocabulary + CSR postings + doc lengths
+//   IndexBuilder           <- SURVEY.md §8(f) row 1: posts -> vocabulary + CSR postings + doc lengths (host reference)
+//   Vocabulary             <- the vocabulary of an index built from text on the device (GpuHybridSearch's text form)
 // Header-only; compute happens in libopenintel_gpu.so.  No CPU scoring path exists here either.
 #pragma once
 #include <algorithm>
@@ -107,6 +108,19 @@ inline std::vector<std::string> tokenize(std::string_view text) {
   return out;
 }
 
+// query text -> term ids: unknown tokens (term_id gives OI_NO_DOC) dropped, duplicates dropped in first-seen order (SPEC
+// §3 counts a term once and scores at most the first 64 DISTINCT known terms; the library de-duplicates too, this keeps
+// the arrays small)
+template <class TermId>
+inline std::vector<uint32_t> query_terms_of(std::string_view text, TermId &&term_id) {
+  std::vector<uint32_t> out;
+  tokenize(text, [&](std::string_view t) {
+    const uint32_t id = term_id(t);
+    if (id != OI_NO_DOC && std::find(out.begin(), out.end(), id) == out.end()) out.push_back(id);
+  });
+  return out;
+}
+
 // ---- index builder -------------------------------------------------------------------------------
 // Posts in, CSR inverted index out: dense doc ids in input order, exact-token vocabulary (no stemming,
 // no stop words: src/domain/dip.rs:261-272 idiom), term ids = lexicographic rank of the token.
@@ -177,15 +191,9 @@ class IndexBuilder {
     auto it = std::lower_bound(vocab_.begin(), vocab_.end(), token, [](const std::string &a, std::string_view b) { return std::string_view(a) < b; });
     return (it != vocab_.end() && std::string_view(*it) == token) ? (uint32_t)(it - vocab_.begin()) : OI_NO_DOC;
   }
-  // query text -> term ids: unknown tokens dropped, duplicates dropped in first-seen order (SPEC §3 counts a term once
-  // and scores at most the first 64 DISTINCT known terms; the library de-duplicates too, this keeps the arrays small)
+  // query text -> term ids (query_terms_of)
   std::vector<uint32_t> query_terms(std::string_view text) const {
-    std::vector<uint32_t> out;
-    tokenize(text, [&](std::string_view t) {
-      const uint32_t id = term_id(t);
-      if (id != OI_NO_DOC && std::find(out.begin(), out.end(), id) == out.end()) out.push_back(id);
-    });
-    return out;
+    return query_terms_of(text, [&](std::string_view t) { return term_id(t); });
   }
 
  private:
@@ -198,6 +206,33 @@ class IndexBuilder {
   bool finished_ = false;
 };
 
+// The vocabulary of an index built from text on the device (oi_index_build_bm25_text): term t = bytes[offsets[t] ..
+// offsets[t + 1]), ascending byte order.  Maps query text to term ids with IndexBuilder's rules.
+class Vocabulary {
+ public:
+  uint32_t size() const { return offsets_.empty() ? 0 : (uint32_t)(offsets_.size() - 1); }
+  std::string_view term(uint32_t t) const {
+    return std::string_view(reinterpret_cast<const char *>(bytes_.data()) + offsets_.at(t), offsets_.at(t + 1) - offsets_[t]);
+  }
+  // term id of a token, or OI_NO_DOC when the token is not in the vocabulary
+  uint32_t term_id(std::string_view token) const {
+    uint32_t lo = 0, hi = size();
+    while (lo < hi) {
+      const uint32_t mid = lo + (hi - lo) / 2;
+      if (term(mid) < token) lo = mid + 1; else hi = mid;
+    }
+    return (lo < size() && term(lo) == token) ? lo : OI_NO_DOC;
+  }
+  std::vector<uint32_t> query_terms(std::string_view text) const {
+    return query_terms_of(text, [&](std::string_view t) { return term_id(t); });
+  }
+
+ private:
+  friend class GpuHybridSearch;
+  std::vector<uint8_t> bytes_;
+  std::vector<uint64_t> offsets_;
+};
+
 // ---- adapters over the C ABI ---------------------------------------------------------------------
 class GpuHybridSearch final : public HybridSearch {
  public:
@@ -206,21 +241,24 @@ class GpuHybridSearch final : public HybridSearch {
                   uint32_t max_batch = 64, uint32_t rrf_k = 60, float k1 = 1.2f, float b = 0.75f)
       : dim_(dim), rrf_k_(rrf_k) {
     ix.finish();
-    oi_index_desc d{};
-    d.struct_size = sizeof(d);
-    d.device = device; d.n_docs = ix.n_docs(); d.doc_base = 0; d.dim = dim; d.dtype = dtype; d.max_k = max_k; d.max_batch = max_batch;
-    if (oi_index_create(&d, &h_) != OI_OK) throw DomainError::source_failure("gpu-search", oi_last_error(nullptr));
-    try {
-      ck(oi_index_load_embeddings(h_, embeddings, 0, ix.n_docs()));
+    open(device, ix.n_docs(), dim, dtype, embeddings, max_k, max_batch, [&] {
       ck(oi_index_load_bm25(h_, ix.term_offsets().data(), ix.doc_ids().data(), ix.tfs().data(), ix.doc_len().data(), ix.n_terms()));
-      oi_bm25_params p{};
-      p.struct_size = sizeof(p);
-      p.k1 = k1; p.b = b; p.avgdl = 0.0f; p.n_docs_global = 0; p.global_df = nullptr;
-      ck(oi_index_bm25_finalize(h_, &p));
-    } catch (...) {
-      oi_index_destroy(h_);
-      throw;
-    }
+    }, k1, b);
+  }
+  // the same index with its BM25 part built on the device from the posts' text: post i = texts[offsets[i] ..
+  // offsets[i + 1]); `vocab` receives the vocabulary (what IndexBuilder::vocabulary() would hold)
+  GpuHybridSearch(int device, uint32_t dim, uint32_t dtype, const void *embeddings, const uint8_t *texts, const uint64_t *offsets,
+                  uint64_t n_posts, Vocabulary &vocab, uint32_t max_k = 100, uint32_t max_batch = 64, uint32_t rrf_k = 60,
+                  float k1 = 1.2f, float b = 0.75f)
+      : dim_(dim), rrf_k_(rrf_k) {
+    open(device, n_posts, dim, dtype, embeddings, max_k, max_batch, [&] {
+      uint32_t n_terms = 0;
+      uint64_t n_bytes = 0;
+      ck(oi_index_build_bm25_text(h_, texts, offsets, n_posts, &n_terms, &n_bytes));
+      vocab.bytes_.resize(n_bytes);
+      vocab.offsets_.resize((size_t)n_terms + 1);
+      ck(oi_index_read_vocabulary(h_, vocab.bytes_.data(), vocab.offsets_.data()));
+    }, k1, b);
   }
   ~GpuHybridSearch() override { oi_index_destroy(h_); }
   GpuHybridSearch(const GpuHybridSearch &) = delete;
@@ -256,6 +294,26 @@ class GpuHybridSearch final : public HybridSearch {
  private:
   void ck(oi_status s) const {
     if (s != OI_OK) throw DomainError::source_failure("gpu-search", oi_last_error(h_));
+  }
+  // creates the index, loads the embeddings, runs `load_bm25` and finalizes; destroys the index on any failure
+  template <class LoadBm25>
+  void open(int device, uint64_t n_docs, uint32_t dim, uint32_t dtype, const void *embeddings, uint32_t max_k, uint32_t max_batch,
+            LoadBm25 &&load_bm25, float k1, float b) {
+    oi_index_desc d{};
+    d.struct_size = sizeof(d);
+    d.device = device; d.n_docs = n_docs; d.doc_base = 0; d.dim = dim; d.dtype = dtype; d.max_k = max_k; d.max_batch = max_batch;
+    if (oi_index_create(&d, &h_) != OI_OK) throw DomainError::source_failure("gpu-search", oi_last_error(nullptr));
+    try {
+      ck(oi_index_load_embeddings(h_, embeddings, 0, n_docs));
+      load_bm25();
+      oi_bm25_params p{};
+      p.struct_size = sizeof(p);
+      p.k1 = k1; p.b = b; p.avgdl = 0.0f; p.n_docs_global = 0; p.global_df = nullptr;
+      ck(oi_index_bm25_finalize(h_, &p));
+    } catch (...) {
+      oi_index_destroy(h_);
+      throw;
+    }
   }
   oi_index *h_ = nullptr;
   uint32_t dim_, rrf_k_;

@@ -156,14 +156,25 @@ class SqlitePostStore {
   uint64_t n_posts_ = 0;
 };
 
-// store -> (vocabulary + CSR in `ix`, normalised embeddings) -> GPU index.  `ix` stays alive with the caller: it
-// maps query text to term ids (IndexBuilder::query_terms) and doc ids back to post ids (post_ids()).
-inline std::unique_ptr<GpuHybridSearch> lift_index(const SqlitePostStore &store, IndexBuilder &ix, int device = 0, uint32_t max_k = 100,
-                                                   uint32_t max_batch = 16, std::vector<float> *rows_out = nullptr) {
-  store.for_each_post([&](const SocialPost &p) { ix.add(p); });
-  ix.finish();
+// store -> GPU index: the posts' text goes to the device in one packed blob, where the vocabulary and the CSR are built
+// (oi_index_build_bm25_text); the normalised embeddings are loaded next to them.  `vocab` maps query text to term ids
+// (Vocabulary::query_terms) and `post_ids` doc ids back to post ids; both stay with the caller.
+inline std::unique_ptr<GpuHybridSearch> lift_index(const SqlitePostStore &store, Vocabulary &vocab, std::vector<std::string> &post_ids,
+                                                   int device = 0, uint32_t max_k = 100, uint32_t max_batch = 16,
+                                                   std::vector<float> *rows_out = nullptr) {
+  std::string blob;
+  std::vector<uint64_t> offs{0};
+  post_ids.clear();
+  store.for_each_post([&](const SocialPost &p) {
+    blob += p.text;
+    offs.push_back(blob.size());
+    post_ids.push_back(p.id);
+  });
+  if (blob.empty()) blob.push_back('\0');  // a valid pointer for a store without text
   std::vector<float> rows = store.embeddings();
-  auto gs = std::make_unique<GpuHybridSearch>(device, store.dim(), (uint32_t)OI_DTYPE_F32, rows.data(), ix, max_k, max_batch);
+  auto gs = std::make_unique<GpuHybridSearch>(device, store.dim(), (uint32_t)OI_DTYPE_F32, rows.data(),
+                                              reinterpret_cast<const uint8_t *>(blob.data()), offs.data(), offs.size() - 1, vocab,
+                                              max_k, max_batch);
   if (rows_out) *rows_out = std::move(rows);
   return gs;
 }

@@ -73,7 +73,7 @@ class IndexBuilder:
     __del__ = close
 
     def add(self, texts):
-        raw = [t.encode("utf-8") for t in texts]
+        raw = [t.encode("utf-8") if isinstance(t, str) else bytes(t) for t in texts]
         offs = np.zeros(len(raw) + 1, dtype=np.uint64)
         offs[1:] = np.cumsum([len(r) for r in raw])
         blob = b"".join(raw) or b"\0"

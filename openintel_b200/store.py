@@ -7,9 +7,12 @@ engagement}` (src/domain/entities/social_post.rs:30-38), `PostText::parse` (trim
 at most 10 000 chars: social_post.rs:7-23), `SourceKind {Reddit, Bluesky}` rendered as
 "reddit" / "bluesky" (src/domain/values/source_kind.rs:5-20) -- plus one embedding per post.
 
-    store  --posts, in doc_id order-->  host tokenizer + IndexBuilder (C++, the reference tokenizer
-                                        src/adapters/analyzer/lexicon.rs:54-58)  -->  CSR  -->  oi_index_load_bm25
+    store  --posts, in doc_id order-->  oi_index_build_bm25_text: the reference tokenizer (src/adapters/analyzer/
+                                        lexicon.rs:54-58), vocabulary and CSR built on the device
            --embeddings (f32 BLOBs)-->  L2-normalise in f32 (SPEC §2)            -->  oi_index_load_embeddings
+
+lift_csr (host tokenizer + IndexBuilder, C++) builds the same vocabulary and CSR on the host: it is the reference the
+device build is tested against, and the sharded lift (lift_shard) uses it.
 
 Scoring happens in libopenintel_gpu.so only; nothing here computes a score.
 """
@@ -169,6 +172,25 @@ def lift_embeddings(conn, n_docs, dim, chunk=8192):
     return normalise_rows_f32(out)
 
 
+class Vocabulary:
+    """The vocabulary of an index built from text on the device: term id i = terms[i] (ascending byte order).
+    Maps query text to term ids with the rules of IndexBuilder.query_terms."""
+
+    def __init__(self, terms):
+        self.terms = terms
+        self.ids = {w: i for i, w in enumerate(terms)}
+
+    def term(self, term_id):
+        return self.terms[term_id]
+
+    def query_terms(self, text):
+        """term ids of the text's tokens: unknown tokens dropped, duplicates dropped in first-seen order (SPEC §3)"""
+        return _dedupe([self.ids[t] for t in hostlib.tokenize(text) if t in self.ids])
+
+    def close(self):
+        pass
+
+
 class StoreIndex:
     """A GPU hybrid index built from a post store: the drop-in search side of the path.
 
@@ -177,8 +199,14 @@ class StoreIndex:
 
     def __init__(self, conn, dtype=capi.DTYPE_F32, device=0, max_k=100, max_batch=16, k1=1.2, b=0.75):
         self.conn = conn
-        self.builder, csr, self.post_ids = lift_csr(conn)
-        self.n_docs, self.n_terms = csr["n_docs"], csr["n_terms"]
+        texts, self.post_ids = [], []
+        for rows in iter_posts(conn):
+            for doc_id, post_id, text in rows:
+                if doc_id != len(texts):
+                    raise ValueError("posts.doc_id must be dense 0..N-1 (gap at %d)" % len(texts))
+                texts.append(text)
+                self.post_ids.append(post_id)
+        self.n_docs = len(texts)
         self.dim = store_dim(conn)
         if self.dim is None:
             raise ValueError("store has no embeddings")
@@ -187,7 +215,8 @@ class StoreIndex:
         try:
             # a bf16 index stores the normalised rows rounded to nearest even (SPEC §2)
             self.ix.load_embeddings(to_bf16_rne(rows) if dtype == capi.DTYPE_BF16 else rows)
-            self.ix.load_bm25(csr["term_offsets"], csr["doc_ids"], csr["tfs"], csr["doc_len"])
+            self.builder = Vocabulary(self.ix.build_bm25_text(texts))
+            self.n_terms = self.ix.n_terms
             self.ix.bm25_finalize(k1=k1, b=b)
         except Exception:
             self.ix.close()
