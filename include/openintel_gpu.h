@@ -113,8 +113,19 @@ oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vocab, const 
  * without any token is OI_ERR_INVALID_ARG (an index needs a term).  Any failure leaves the index without a BM25 part. */
 oi_status oi_index_build_bm25_text(oi_index *h, const uint8_t *texts, const uint64_t *offsets, uint64_t n_posts,
                                    uint32_t *out_n_terms, uint64_t *out_vocab_bytes);
-/* the vocabulary of the last oi_index_build_bm25_text: term t = bytes[offsets[t] .. offsets[t+1]), offsets[n_terms+1].
- * OI_ERR_STATE when the BM25 part did not come from text. */
+/* document-sharded index (SPEC §5), after oi_index_build_bm25_text, before oi_index_bm25_finalize: entry i =
+ * terms[offsets[i] .. offsets[i+1]) (host memory), the concatenated vocabularies of all shards in any order, duplicates
+ * allowed (the host gathers them over any transport).  The vocabulary becomes the sorted distinct union of the entries
+ * (ascending byte order, a proper prefix first); this shard's CSR is re-indexed to it: term id = rank in the union,
+ * terms this shard does not hold get empty lists, doc_ids / tfs / doc_len unchanged.  out_n_terms / out_vocab_bytes
+ * size oi_index_read_vocabulary's buffers.  OI_ERR_STATE: the BM25 part was not built from text, or is finalized.
+ * OI_ERR_INVALID_ARG: NULL pointers, no entries or more than 2^32 - 2, decreasing offsets, an entry that is empty or
+ * holds a byte outside [0-9a-z] (tokens hold nothing else), a term of this shard missing from the entries.  A failed
+ * call leaves the BM25 part and its vocabulary as they were; calling again with the same entries changes nothing. */
+oi_status oi_index_bm25_union_vocabulary(oi_index *h, const uint8_t *terms, const uint64_t *offsets, uint64_t n_entries,
+                                         uint32_t *out_n_terms, uint64_t *out_vocab_bytes);
+/* the vocabulary of the BM25 part built from text (after oi_index_bm25_union_vocabulary: the union): term t =
+ * bytes[offsets[t] .. offsets[t+1]), offsets[n_terms+1].  OI_ERR_STATE when the BM25 part did not come from text. */
 oi_status oi_index_read_vocabulary(oi_index *h, uint8_t *bytes, uint64_t *offsets);
 /* this shard's df per term and sum of doc lengths, to be summed over shards by the host */
 oi_status oi_index_bm25_local_stats(oi_index *h, uint32_t *df_out, uint64_t *sum_doc_len,

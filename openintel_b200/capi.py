@@ -70,6 +70,7 @@ def load_library():
         "oi_index_load_bm25": (st, [H, _u64p, _u32p, _u32p, _u32p, C.c_uint32]),
         "oi_index_synth_bm25": (st, [H, C.c_uint64, C.c_uint32, _vp]),
         "oi_index_build_bm25_text": (st, [H, _vp, _u64p, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
+        "oi_index_bm25_union_vocabulary": (st, [H, _vp, _u64p, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
         "oi_index_read_vocabulary": (st, [H, _vp, _u64p]),
         "oi_index_bm25_local_stats": (st, [H, _u32p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "oi_index_bm25_finalize": (st, [H, C.POINTER(Bm25Params)]),
@@ -188,12 +189,30 @@ class GpuIndex:
         blob, offs = pack_texts(texts)
         nt, nb = C.c_uint32(), C.c_uint64()
         self._ck(self.L.oi_index_build_bm25_text(self.h, _addr(blob), _addr(offs), len(offs) - 1, C.byref(nt), C.byref(nb)))
-        self.n_terms = nt.value
-        vb = np.empty(max(nb.value, 1), dtype=np.uint8)
+        self.n_terms, self.vocab_bytes = nt.value, nb.value
+        return unpack_terms(*self.read_vocabulary_packed())
+
+    def bm25_union_vocabulary(self, blob, offsets):
+        """document-sharded index, after build_bm25_text and before bm25_finalize: (blob u8[], offsets u64[n + 1]) = the
+        concatenated vocabularies of all shards (any order, duplicates allowed; sharding.all_gather_packed).  The
+        vocabulary becomes their sorted union and this shard's lists are re-indexed to it, on the device
+        (oi_index_bm25_union_vocabulary).  Returns the global vocabulary: term id i = list[i]."""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8)
+        offs = np.ascontiguousarray(offsets, dtype=np.uint64)
+        if not len(blob):
+            blob = np.zeros(1, dtype=np.uint8)
+        nt, nb = C.c_uint32(), C.c_uint64()
+        self._ck(self.L.oi_index_bm25_union_vocabulary(self.h, _addr(blob), _addr(offs), len(offs) - 1, C.byref(nt), C.byref(nb)))
+        self.n_terms, self.vocab_bytes = nt.value, nb.value
+        return unpack_terms(*self.read_vocabulary_packed())
+
+    def read_vocabulary_packed(self):
+        """the vocabulary of a BM25 part built from text, undecoded: (bytes u8[], offsets u64[n_terms + 1]), term t =
+        bytes[offsets[t] .. offsets[t + 1])"""
+        vb = np.empty(max(getattr(self, "vocab_bytes", 0), 1), dtype=np.uint8)
         vo = np.empty(self.n_terms + 1, dtype=np.uint64)
         self._ck(self.L.oi_index_read_vocabulary(self.h, _addr(vb), _addr(vo)))
-        raw = vb.tobytes()
-        return [raw[vo[t]:vo[t + 1]].decode("ascii") for t in range(self.n_terms)]
+        return vb[:int(vo[-1])], vo
 
     def bm25_local_stats(self):
         df = np.empty(self.n_terms, dtype=np.uint32)
@@ -322,6 +341,13 @@ def pack_texts(texts):
     offs[1:] = np.cumsum([len(r) for r in raw])
     blob = np.frombuffer(b"".join(raw) or b"\0", dtype=np.uint8).copy()
     return blob, offs
+
+
+def unpack_terms(blob, offsets):
+    """(bytes, offsets) of a vocabulary or of gathered vocabularies -> list of str"""
+    raw = np.asarray(blob, dtype=np.uint8).tobytes()
+    offs = np.asarray(offsets, dtype=np.int64)
+    return [raw[offs[t]:offs[t + 1]].decode("ascii") for t in range(len(offs) - 1)]
 
 
 class GpuLexicon:

@@ -1058,6 +1058,16 @@ oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 
   return s;
 }
 
+const u64 *oi_bm25_term_offsets(const oi_index *h) { return h->bm25 ? h->bm25->d_term_off : nullptr; }
+bool oi_bm25_finalized(const oi_index *h) { return h->bm25 && h->bm25->finalized; }
+
+void oi_bm25_replace_terms(oi_index *h, uint32_t n_terms, u64 *d_term_off) {
+  OiBm25 *b = h->bm25;
+  cudaFree(b->d_term_off);
+  b->d_term_off = d_term_off;
+  b->n_terms = n_terms;
+}
+
 extern "C" oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vocab, const double *zipf_cdf) {
   if (!h) return OI_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lock(h->mu);

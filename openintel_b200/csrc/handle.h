@@ -108,6 +108,11 @@ void oi_bm25_free(oi_index *h);
 oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 *d_term_off, uint32_t *d_doc_ids,
                         uint32_t *d_tfs, uint32_t *d_doc_len);
 uint32_t oi_bm25_n_terms(const oi_index *h);  // 0 = no BM25 part
+const u64 *oi_bm25_term_offsets(const oi_index *h);  // device term_offsets[n_terms + 1]; NULL = no BM25 part
+bool oi_bm25_finalized(const oi_index *h);
+// re-indexes the BM25 part to n_terms terms over the same postings (text_index.cu's vocabulary union): d_term_off
+// [n_terms + 1] on the device becomes the index's, the old offsets are freed.  Before finalize only.
+void oi_bm25_replace_terms(oi_index *h, uint32_t n_terms, u64 *d_term_off);
 uint32_t *oi_bm25_stage_terms(oi_index *h);  // device staging for the host call's flat term array
 uint32_t *oi_bm25_stage_offs(oi_index *h);
 // prep -> blocked scoring -> merge: shard-local sorted key lists d_out_keys[nq][k] (global doc ids)

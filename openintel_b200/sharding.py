@@ -1,7 +1,8 @@
 """Host-side plumbing of the document-sharded index (docs/SPEC.md §5): one process per GPU,
 contiguous doc ranges, GLOBAL BM25 statistics, and the NCCL communicator the C library uses for
 the all-gather of local top-k lists.  torch.distributed is used only as the control plane
-(all-reduce of df / doc-length sums at build time, broadcast of the NCCL unique id); the
+(all-gather of the shards' vocabularies and all-reduce of df / doc-length sums at build time,
+broadcast of the NCCL unique id); the
 per-query exchange itself is libopenintel_gpu.so's ncclAllGather + device merge.
 
 The same functions run over gloo on CPU tensors (tests/test_sharding_gloo.py) and over NCCL.
@@ -39,6 +40,38 @@ def global_bm25_stats(dist, df_local, sum_doc_len_local, n_docs_local, device="c
     s, n = (int(x) for x in t_sc.cpu().tolist())
     avgdl = np.float32(np.float64(s) / np.float64(n)) if n else np.float32(1.0)
     return gdf.astype(np.uint32), avgdl, n
+
+
+def all_gather_packed(dist, blob, offsets, device="cpu"):
+    """Every rank's byte strings, packed as (blob u8[], offsets u64[n + 1]: string i = blob[offsets[i] .. offsets[i + 1]))
+    -> all ranks' strings concatenated in rank order, packed the same way (offsets from 0).  Used to gather the shards'
+    vocabularies for oi_index_bm25_union_vocabulary without decoding them to Python strings.  `dist` is
+    torch.distributed (initialised) or None for a single shard."""
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    offs = np.ascontiguousarray(offsets, dtype=np.int64)
+    mine, lens = blob[offs[0]:offs[-1]], np.diff(offs)
+    if dist is None or dist.get_world_size() == 1:
+        return mine.copy(), np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
+    import torch
+    world = dist.get_world_size()
+    size = torch.tensor([len(mine), len(lens)], dtype=torch.int64, device=device)
+    sizes = [torch.zeros_like(size) for _ in range(world)]
+    dist.all_gather(sizes, size)
+    sizes = [tuple(int(x) for x in t.cpu().tolist()) for t in sizes]
+    # padded to the largest rank's share, at least one element (a rank may hold nothing)
+    nb, nl = max(max(s[0] for s in sizes), 1), max(max(s[1] for s in sizes), 1)
+    t_blob = torch.zeros(nb, dtype=torch.uint8)
+    t_blob[:len(mine)] = torch.from_numpy(mine)
+    t_lens = torch.zeros(nl, dtype=torch.int64)
+    t_lens[:len(lens)] = torch.from_numpy(lens)
+    t_blob, t_lens = t_blob.to(device), t_lens.to(device)
+    g_blob = [torch.empty_like(t_blob) for _ in range(world)]
+    g_lens = [torch.empty_like(t_lens) for _ in range(world)]
+    dist.all_gather(g_blob, t_blob)
+    dist.all_gather(g_lens, t_lens)
+    out_blob = np.concatenate([g.cpu().numpy()[:s[0]] for g, s in zip(g_blob, sizes)])
+    out_lens = np.concatenate([g.cpu().numpy()[:s[1]] for g, s in zip(g_lens, sizes)])
+    return out_blob, np.concatenate([[0], np.cumsum(out_lens)]).astype(np.uint64)
 
 
 def broadcast_unique_id(dist, device="cpu"):

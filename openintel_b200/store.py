@@ -11,8 +11,12 @@ at most 10 000 chars: social_post.rs:7-23), `SourceKind {Reddit, Bluesky}` rende
                                         lexicon.rs:54-58), vocabulary and CSR built on the device
            --embeddings (f32 BLOBs)-->  L2-normalise in f32 (SPEC §2)            -->  oi_index_load_embeddings
 
-lift_csr (host tokenizer + IndexBuilder, C++) builds the same vocabulary and CSR on the host: it is the reference the
-device build is tested against, and the sharded lift (lift_shard) uses it.
+The document-sharded lift (lift_shard_gpu, ShardedStoreIndex) runs on the device too: every rank builds its doc range
+with oi_index_build_bm25_text, the ranks all-gather their packed vocabularies, and oi_index_bm25_union_vocabulary forms
+the sorted union and re-indexes the shard's lists to the global term ids.
+
+lift_csr and lift_shard (host tokenizer + IndexBuilder, C++) build the same vocabularies and CSRs on the host: they are
+the references the device builds are tested against.
 
 Scoring happens in libopenintel_gpu.so only; nothing here computes a score.
 """
@@ -308,37 +312,95 @@ def lift_shard(conn, dist, rank=None, world=None, device="cpu"):
                 post_ids=ids)
 
 
+def lift_shard_gpu(conn, dist, device="cpu", device_index=0, max_k=100, max_batch=16):
+    """lift_shard on the device: the same shard, built into an open GpuIndex on `device_index` --
+      * the rank's contiguous doc range is tokenised and indexed by oi_index_build_bm25_text,
+      * the packed vocabularies are all-gathered (sharding.all_gather_packed) and oi_index_bm25_union_vocabulary
+        forms their sorted union and re-indexes the shard's CSR to it (global term ids, absent terms = empty lists),
+      * df / doc-length sums are all-reduced (sharding.global_bm25_stats).
+    A shard whose posts hold no token contributes no vocabulary; it forms the union on the host from the gathered
+    entries and loads an all-empty CSR over it.
+
+    `dist` = torch.distributed (initialised, gloo or nccl) or None; `device` = where its collectives run.  The index is
+    not finalized: load the embeddings, then bm25_finalize with global_df / avgdl / n_docs_global.  -> dict(index,
+    doc_base, n_local, n_docs_global, vocab, global_df, avgdl, post_ids (this shard's))"""
+    from . import sharding
+    n_total = conn.execute("SELECT COUNT(*) FROM posts").fetchone()[0]
+    if dist is not None and dist.get_world_size() > 1:
+        rank, world = dist.get_rank(), dist.get_world_size()
+    else:
+        dist, rank, world = None, 0, 1
+    base, n_local = sharding.shard_range(n_total, world, rank)
+    texts, ids = [], []
+    cur = conn.execute("SELECT doc_id, id, text FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id", (base, base + n_local))
+    for doc_id, post_id, text in cur:
+        if doc_id != base + len(texts):
+            raise ValueError("posts.doc_id must be dense 0..N-1 (gap at %d)" % (base + len(texts)))
+        texts.append(text)
+        ids.append(post_id)
+    if len(texts) != n_local:
+        raise ValueError("posts.doc_id must be dense 0..N-1 (gap at %d)" % (base + len(texts)))
+    dim = store_dim(conn)
+    if dim is None:
+        raise ValueError("store has no embeddings")
+    ix = capi.GpuIndex(n_docs=n_local, dim=dim, device=device_index, doc_base=base, max_k=max_k, max_batch=max_batch)
+    try:
+        no_token = None
+        try:
+            ix.build_bm25_text(texts)
+            blob, offs = ix.read_vocabulary_packed()
+        except capi.OiError as e:
+            if e.status != 1 or "no token" not in e.message:
+                raise
+            no_token, blob, offs = e, np.zeros(0, np.uint8), np.zeros(1, np.uint64)
+        blob, offs = sharding.all_gather_packed(dist, blob, offs, device=device)
+        if no_token is not None:
+            vocab = sorted(set(capi.unpack_terms(blob, offs)))
+            if not vocab:  # no rank holds a token: the store cannot be indexed, sharded or not
+                raise no_token
+            ix.load_bm25(np.zeros(len(vocab) + 1, np.uint64), np.zeros(0, np.uint32), np.zeros(0, np.uint32),
+                         np.zeros(n_local, np.uint32))
+        else:
+            vocab = ix.bm25_union_vocabulary(blob, offs)
+        df, sum_dl, _ = ix.bm25_local_stats()
+        gdf, avgdl, n = sharding.global_bm25_stats(dist, df, sum_dl, n_local, device=device)
+        if n != n_total:
+            raise ValueError("the ranks see %d posts in total, the store holds %d" % (n, n_total))
+    except Exception:
+        ix.close()
+        raise
+    return dict(index=ix, doc_base=base, n_local=n_local, n_docs_global=n_total, vocab=vocab, global_df=gdf,
+                avgdl=float(avgdl), post_ids=ids)
+
+
 class ShardedStoreIndex:
-    """StoreIndex over the GPUs of one box: every rank lifts its doc range (lift_shard), loads it into its GPU with
-    GLOBAL BM25 statistics and joins the NCCL communicator; search() returns the same global lists on every rank."""
+    """StoreIndex over the GPUs of one box: every rank lifts its doc range on its GPU (lift_shard_gpu), loads its
+    embeddings, finalizes with GLOBAL BM25 statistics and joins the NCCL communicator; search() returns the same global
+    lists on every rank."""
 
     def __init__(self, conn, dist, device_index=0, max_k=100, max_batch=16, k1=1.2, b=0.75):
         from . import sharding
         self.dist = dist if (dist is not None and dist.get_world_size() > 1) else None
         dev = "cuda:%d" % device_index
-        sh = lift_shard(conn, self.dist, device=dev if self.dist else "cpu")
+        sh = lift_shard_gpu(conn, self.dist, device=dev if self.dist else "cpu", device_index=device_index, max_k=max_k,
+                            max_batch=max_batch)
+        self.ix = sh["index"]
         self.vocab, self.doc_base, self.n_local, self.n_docs = sh["vocab"], sh["doc_base"], sh["n_local"], sh["n_docs_global"]
         self.term_id = {w: i for i, w in enumerate(self.vocab)}
         self.dim = store_dim(conn)
-        if self.dim is None:
-            raise ValueError("store has no embeddings")
-        rows = np.empty((self.n_local, self.dim), dtype=np.float32)
-        cur = conn.execute("SELECT doc_id, vec FROM embeddings WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
-                           (self.doc_base, self.doc_base + self.n_local))
-        got = 0
-        for doc_id, blob in cur:
-            if doc_id != self.doc_base + got:
-                raise ValueError("embedding missing for doc %d" % (self.doc_base + got))
-            rows[got] = np.frombuffer(blob, dtype="<f4")
-            got += 1
-        if got != self.n_local:
-            raise ValueError("embedding missing for doc %d" % (self.doc_base + got))
-        rows = normalise_rows_f32(rows)
-        self.ix = capi.GpuIndex(n_docs=self.n_local, dim=self.dim, device=device_index, doc_base=self.doc_base, max_k=max_k, max_batch=max_batch)
         try:
-            self.ix.load_embeddings(rows)
-            c = sh["csr"]
-            self.ix.load_bm25(c["term_offsets"], c["doc_ids"], c["tfs"], c["doc_len"])
+            rows = np.empty((self.n_local, self.dim), dtype=np.float32)
+            cur = conn.execute("SELECT doc_id, vec FROM embeddings WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
+                               (self.doc_base, self.doc_base + self.n_local))
+            got = 0
+            for doc_id, blob in cur:
+                if doc_id != self.doc_base + got:
+                    raise ValueError("embedding missing for doc %d" % (self.doc_base + got))
+                rows[got] = np.frombuffer(blob, dtype="<f4")
+                got += 1
+            if got != self.n_local:
+                raise ValueError("embedding missing for doc %d" % (self.doc_base + got))
+            self.ix.load_embeddings(normalise_rows_f32(rows))
             self.ix.bm25_finalize(k1=k1, b=b, avgdl=sh["avgdl"], n_docs_global=self.n_docs, global_df=sh["global_df"])
             if self.dist:
                 self.ix.comm_init(self.dist.get_rank(), self.dist.get_world_size(), sharding.broadcast_unique_id(self.dist, device=dev))

@@ -79,6 +79,8 @@ extern "C" {
     pub fn oi_index_synth_bm25(h: *mut oi_index, seed: u64, vocab: u32, zipf_cdf: *const f64) -> oi_status;
     pub fn oi_index_build_bm25_text(h: *mut oi_index, texts: *const u8, offsets: *const u64, n_posts: u64,
                                     out_n_terms: *mut u32, out_vocab_bytes: *mut u64) -> oi_status;
+    pub fn oi_index_bm25_union_vocabulary(h: *mut oi_index, terms: *const u8, offsets: *const u64, n_entries: u64,
+                                          out_n_terms: *mut u32, out_vocab_bytes: *mut u64) -> oi_status;
     pub fn oi_index_read_vocabulary(h: *mut oi_index, bytes: *mut u8, offsets: *mut u64) -> oi_status;
     pub fn oi_index_bm25_local_stats(h: *mut oi_index, df_out: *mut u32, sum_doc_len: *mut u64, n_postings: *mut u64) -> oi_status;
     pub fn oi_index_bm25_finalize(h: *mut oi_index, params: *const oi_bm25_params) -> oi_status;
