@@ -205,6 +205,42 @@ oi_status oi_lexicon_analyze(int32_t device, const uint8_t *texts, const uint64_
                              uint64_t n_posts, double *out_polarity, uint8_t *out_speculative,
                              uint32_t *out_bull_hits, uint32_t *out_bear_hits);
 
+/* ---- per-term social summaries over the BM25 posting lists (docs/SPEC.md §8a) ---------------
+ * A post mentions term t iff one of its tokens equals t, so the posts that mention t are t's posting list, in doc
+ * order.  With per-post lexicon signals loaded next to the BM25 part, one call returns the social summary of
+ * oi_lexicon_run (same counts, same sequential f64 mean, same clamps) over each requested term's list.
+ *
+ * Document-sharded index: the mean is a SEQUENTIAL sum in doc order, so the shards run as a relay in rank order -- rank 0
+ * calls with carry_in = NULL, rank r > 0 continues from the out_state of rank r - 1 -- and the last rank's out_summary is
+ * bit-identical to the unsharded one.  (An all-reduce of per-shard partial sums would round differently.) */
+#define OI_N_SOURCES 2 /* post sources in store-schema order: 0 = reddit, 1 = bluesky */
+
+/* the running state of one term's summary after some prefix of the doc order */
+typedef struct {
+  uint64_t total, bullish, bearish, neutral, speculative; /* posts counted, by the bull/bear threshold, speculative */
+  uint64_t by_source[OI_N_SOURCES];                       /* posts counted per source code */
+  double sum; /* sequential f64 sum of the polarities so far, doc order (SPEC §8a) */
+} oi_mention_state;
+
+/* per-post lexicon signals of THIS shard, n = n_docs, host memory: polarity f64 (finite, in [-1, 1]; -0.0 is stored as
+ * +0.0, which changes no sum), speculative 0/1, source < OI_N_SOURCES.  Checked before anything is replaced: a refused
+ * call (OI_ERR_INVALID_ARG naming the first bad post) keeps the previous signals.  Independent of the BM25 part (a
+ * rebuilt BM25 part keeps them). */
+oi_status oi_index_load_post_signals(oi_index *h, const double *polarity, const uint8_t *speculative,
+                                     const uint8_t *source);
+
+/* for each of terms[0 .. n_terms): the social summary of the posts of this shard that mention the term
+ * (its posting list), continued from carry_in[i] (NULL = nothing before this shard).  source: -1 = all
+ * posts, else only that source's.  out_state[i] = the running state after this shard (may be NULL);
+ * out_summary[i] = the summary of every post counted in out_state[i].  On the last shard of a relay,
+ * that is the global summary.  Duplicate term ids are allowed (each gets its own output).
+ * OI_ERR_STATE: no BM25 part, or no signals loaded.  OI_ERR_INVALID_ARG: NULL terms / out_summary, a term id >= the
+ * BM25 part's n_terms, source outside -1 .. OI_N_SOURCES - 1.  Blocking; reads the posting lists only, so it works
+ * before and after oi_index_bm25_finalize and changes neither. */
+oi_status oi_index_mention_summary(oi_index *h, const uint32_t *terms, uint32_t n_terms, int32_t source,
+                                   double bull_bear_threshold, const oi_mention_state *carry_in,
+                                   oi_mention_state *out_state, oi_social_summary *out_summary);
+
 /* ---- tuning / introspection (bench + tests) ------------------------------------------------ */
 /* number of kernels this handle has launched since creation (bench "gpu_launches") */
 uint64_t oi_index_launch_count(const oi_index *h);

@@ -41,22 +41,23 @@ def select_posts(conn, source=None, mention=None, limit=None):
     return [r[0] for r in rows], [r[1] for r in rows], [r[2] for r in rows]
 
 
-def analyze_posts(lexicon, sources, texts, market=None, cfg=fusion.EngineConfig()):
-    """SpeculationEngine::aggregate (src/domain/engine/speculation_engine.rs:21-66) with the signals and the social
-    summary coming from ONE GPU call.  market: fusion.MarketSummary or None."""
-    if len(sources) != len(texts):
-        raise ValueError("analyzer mismatch: %d sources for %d posts" % (len(sources), len(texts)))
-    if not texts and market is None:
+def empty_summary():
+    """the social summary of no posts (SpeculationEngine::social_summary over an empty slice; -1 = no bearish post)"""
+    return dict(total=0, bullish=0, bearish=0, neutral=0, net_sentiment=0.0, speculation_index=0.0, bull_bear_ratio=-1.0)
+
+
+def build_report(sm, mentions_by_source, market=None, cfg=fusion.EngineConfig()):
+    """The rest of SpeculationEngine::aggregate (src/domain/engine/speculation_engine.rs:21-66) once the social summary
+    is known: the fusion signals and a report shaped like the reference's SpeculationReport.  sm: a summary dict shaped
+    like GpuLexicon's; mentions_by_source: {source name: post count}; market: fusion.MarketSummary or None.  Raises
+    NoData when there is neither a post nor a market snapshot."""
+    if sm["total"] == 0 and market is None:
         raise NoData("no posts and no market snapshot")
     notes = []
-    if texts:
-        pol, spec, _, _, sm = lexicon.analyze(texts, summary=True, threshold=cfg.bull_bear_threshold)
-    else:
-        pol, spec = [], []
-        sm = dict(total=0, bullish=0, bearish=0, neutral=0, net_sentiment=0.0, speculation_index=0.0, bull_bear_ratio=-1.0)
     by_source = OrderedDict()
-    for s in sorted(set(sources)):  # the reference keeps a BTreeMap: sorted keys
-        by_source[s] = sources.count(s)
+    for s in sorted(mentions_by_source):  # the reference keeps a BTreeMap: sorted keys
+        if mentions_by_source[s]:
+            by_source[s] = int(mentions_by_source[s])
     if market is None:
         notes.append("social-only, no price reference")
     social = {"total_mentions": int(sm["total"]), "mentions_by_source": by_source, "net_sentiment": sm["net_sentiment"],
@@ -67,10 +68,22 @@ def analyze_posts(lexicon, sources, texts, market=None, cfg=fusion.EngineConfig(
     class _S:
         total, net_sentiment, speculation_index = social["total_mentions"], social["net_sentiment"], social["speculation_index"]
     fz = fusion.fuse(_S, market, cfg)
-    report = {"social": social,
-              "market": None if market is None else {"pct_change": market.pct_change, "rvol": market.rvol, "iv_rank": market.iv_rank},
-              "fusion": {"alignment": fz["alignment"], "crowding": fz["crowding"], "notes": notes},
-              "social_confidence": fz["social_confidence"], "disclaimer": DISCLAIMER}
+    return {"social": social,
+            "market": None if market is None else {"pct_change": market.pct_change, "rvol": market.rvol, "iv_rank": market.iv_rank},
+            "fusion": {"alignment": fz["alignment"], "crowding": fz["crowding"], "notes": notes},
+            "social_confidence": fz["social_confidence"], "disclaimer": DISCLAIMER}
+
+
+def analyze_posts(lexicon, sources, texts, market=None, cfg=fusion.EngineConfig()):
+    """SpeculationEngine::aggregate (src/domain/engine/speculation_engine.rs:21-66) with the signals and the social
+    summary coming from ONE GPU call.  market: fusion.MarketSummary or None."""
+    if len(sources) != len(texts):
+        raise ValueError("analyzer mismatch: %d sources for %d posts" % (len(sources), len(texts)))
+    if texts:
+        pol, spec, _, _, sm = lexicon.analyze(texts, summary=True, threshold=cfg.bull_bear_threshold)
+    else:
+        pol, spec, sm = [], [], empty_summary()
+    report = build_report(sm, {s: sources.count(s) for s in set(sources)}, market, cfg)
     return report, pol, spec
 
 

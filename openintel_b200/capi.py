@@ -39,6 +39,17 @@ class SocialSummary(C.Structure):
                 ("net_sentiment", C.c_double), ("speculation_index", C.c_double), ("bull_bear_ratio", C.c_double)]
 
 
+N_SOURCES = 2  # OI_N_SOURCES: post sources in store-schema order (store.SOURCES)
+
+
+# oi_mention_state as a numpy structured type: the running state of one term's summary after a prefix of the doc order
+# (SPEC §8a)
+MENTION_STATE_DTYPE = np.dtype([("total", "<u8"), ("bullish", "<u8"), ("bearish", "<u8"), ("neutral", "<u8"),
+                                ("speculative", "<u8"), ("by_source", "<u8", (N_SOURCES,)), ("sum", "<f8")])
+# ... and of oi_social_summary
+SOCIAL_SUMMARY_DTYPE = np.dtype([(f, "<u8" if t is C.c_uint64 else "<f8") for f, t in SocialSummary._fields_])
+
+
 def lib_path():
     # OI_GPU_LIB: A/B experiments against another build of the same C ABI (tools/ only); the product loads the in-tree .so
     return os.environ.get("OI_GPU_LIB") or os.path.join(_HERE, "libopenintel_gpu.so")
@@ -91,6 +102,8 @@ def load_library():
         "oi_lexicon_destroy": (None, [H]),
         "oi_lexicon_run": (st, [H, _vp, _u64p, C.c_uint64, _vp, _vp, _u32p, _u32p, C.c_double, C.POINTER(SocialSummary)]),
         "oi_lexicon_launch_count": (C.c_uint64, [H]),
+        "oi_index_load_post_signals": (st, [H, _vp, _vp, _vp]),
+        "oi_index_mention_summary": (st, [H, _u32p, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
         "oi_index_launch_count": (C.c_uint64, [H]),
         "oi_index_set_option": (st, [H, C.c_char_p, C.c_int64]),
         "oi_debug_cosine_gemm_scores": (st, [H, _f32p, C.c_uint32, _f32p]),
@@ -235,6 +248,34 @@ class GpuIndex:
         self._ck(self.L.oi_index_read_bm25(self.h, _addr(to), _addr(di), _addr(tf), _addr(dl), _addr(w)))
         return dict(term_offsets=to, doc_ids=di, tfs=tf, doc_len=dl, weights=w)
 
+    # -- per-term social summaries over the posting lists (SPEC §8a)
+    def load_post_signals(self, polarity, speculative, source):
+        """per-post lexicon signals of this shard, in doc order: polarity f64 in [-1, 1], speculative 0/1, source code
+        (index into store.SOURCES).  A refused call keeps the previous signals."""
+        pol = np.ascontiguousarray(polarity, dtype=np.float64)
+        spec = np.ascontiguousarray(speculative, dtype=np.uint8)
+        src = np.ascontiguousarray(source, dtype=np.uint8)
+        if not len(pol) == len(spec) == len(src) == self.n_docs:
+            raise ValueError("need %d signals of each kind, got %d / %d / %d" % (self.n_docs, len(pol), len(spec), len(src)))
+        self._ck(self.L.oi_index_load_post_signals(self.h, _addr(pol), _addr(spec), _addr(src)))
+
+    def mention_summary(self, term_ids, source=None, threshold=0.2, carry=None):
+        """the social summary of each term's posting list on this shard (oi_index_mention_summary), continued from
+        `carry` (the states of the previous shard, or None).  source: None = all posts, else a source code.
+        -> (states: MENTION_STATE_DTYPE array, summaries: list of dicts shaped like GpuLexicon's summary)"""
+        terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
+        n = len(terms)
+        states = np.zeros(n, dtype=MENTION_STATE_DTYPE)
+        sums = np.zeros(n, dtype=SOCIAL_SUMMARY_DTYPE)
+        cin = None
+        if carry is not None:
+            cin = np.ascontiguousarray(carry, dtype=MENTION_STATE_DTYPE)
+            if len(cin) != n:
+                raise ValueError("%d carried states for %d terms" % (len(cin), n))
+        self._ck(self.L.oi_index_mention_summary(self.h, _addr(terms), n, -1 if source is None else int(source), threshold,
+                                                  _addr(cin), _addr(states), _addr(sums)))
+        return states, summaries_from_array(sums)
+
     # -- multi-GPU
     @staticmethod
     def comm_unique_id():
@@ -332,6 +373,20 @@ class GpuIndex:
 
     def set_option(self, name, value):
         self._ck(self.L.oi_index_set_option(self.h, name.encode(), int(value)))
+
+
+def summaries_from_array(a):
+    """SOCIAL_SUMMARY_DTYPE array -> list of summary dicts shaped like GpuLexicon's"""
+    return [{f: (int(r[f]) if t is C.c_uint64 else float(r[f])) for f, t in SocialSummary._fields_} for r in a]
+
+
+def summaries_to_array(summaries):
+    """list of summary dicts -> SOCIAL_SUMMARY_DTYPE array (the layout of oi_social_summary)"""
+    out = np.zeros(len(summaries), dtype=SOCIAL_SUMMARY_DTYPE)
+    for i, sm in enumerate(summaries):
+        for f, _ in SocialSummary._fields_:
+            out[i][f] = sm[f]
+    return out
 
 
 def pack_texts(texts):

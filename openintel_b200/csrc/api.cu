@@ -62,50 +62,16 @@ static bool stream_is_capturing(cudaStream_t st) {
   if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); return false; }
   return cs != cudaStreamCaptureStatusNone;
 }
-static cudaError_t call_begin(oi_index *h, cudaStream_t st) {
+cudaError_t call_begin(oi_index *h, cudaStream_t st) {
   if (!h->has_last || st == h->last_stream || stream_is_capturing(st)) return cudaSuccess;
   return cudaStreamWaitEvent(st, h->ev_last, 0);
 }
-static cudaError_t call_end(oi_index *h, cudaStream_t st) {
+cudaError_t call_end(oi_index *h, cudaStream_t st) {
   if (stream_is_capturing(st)) return cudaSuccess;
   cudaError_t e = cudaEventRecord(h->ev_last, st);
   if (e == cudaSuccess) { h->has_last = true; h->last_stream = st; }
   return e;
 }
-
-// A staging slot for one small host-buffer call.  Taken under the handle's lock (waiting, lock released, while all are
-// busy); given back by the guard after the caller has copied its results out -- or on any early return.
-struct SlotLease {
-  oi_index *h;
-  std::unique_lock<std::mutex> &lock;
-  oi_index::Slot *sl;
-  SlotLease(oi_index *h_, std::unique_lock<std::mutex> &lock_) : h(h_), lock(lock_), sl(nullptr) {
-    for (;;) {
-      for (oi_index::Slot &c : h->slots)
-        if (!c.busy) { sl = &c; break; }
-      if (sl) break;
-      h->slot_cv.wait(lock);
-    }
-    sl->busy = true;
-  }
-  ~SlotLease() {
-    if (!lock.owns_lock()) lock.lock();
-    sl->busy = false;
-    h->slot_cv.notify_one();
-  }
-  // the enqueue is complete: record the slot's event, let the next caller in, wait for this call's results
-  oi_status finish(cudaStream_t st) {
-    cudaError_t e = cudaEventRecord(sl->done, st);
-    if (e == cudaSuccess) e = call_end(h, st);
-    if (e == cudaSuccess) {
-      lock.unlock();
-      e = cudaEventSynchronize(sl->done);
-      if (e != cudaSuccess) lock.lock();
-    }
-    if (e != cudaSuccess) return h->fail(OI_ERR_CUDA, "host-buffer call failed: %s", cudaGetErrorString(e));
-    return OI_OK;
-  }
-};
 
 extern "C" oi_status oi_index_create(const oi_index_desc *desc, oi_index **out) {
   if (!out) return create_fail(OI_ERR_INVALID_ARG, "out is NULL");
@@ -187,6 +153,7 @@ extern "C" void oi_index_destroy(oi_index *h) {
   oi_comm_destroy(h);
   oi_bm25_free(h);
   oi_gemm_free(h);
+  oi_mention_free(h);
   cudaFree(h->d_emb);
   cudaFree(h->cws.cand);
   cudaFree(h->cws.gthr);

@@ -1059,6 +1059,7 @@ oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 
 }
 
 const u64 *oi_bm25_term_offsets(const oi_index *h) { return h->bm25 ? h->bm25->d_term_off : nullptr; }
+const uint32_t *oi_bm25_doc_ids(const oi_index *h) { return h->bm25 ? h->bm25->d_doc_ids : nullptr; }
 bool oi_bm25_finalized(const oi_index *h) { return h->bm25 && h->bm25->finalized; }
 
 void oi_bm25_replace_terms(oi_index *h, uint32_t n_terms, u64 *d_term_off) {

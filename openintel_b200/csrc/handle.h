@@ -91,6 +91,14 @@ struct oi_index {
   u64 *d_vocab_off = nullptr;
   uint64_t vocab_bytes = 0;
 
+  // per-post lexicon signals (mention.cu), independent of the BM25 part: polarity f64 and speculative | source << 1
+  // per post, [n_docs] each.  d_mention_io: grow-on-demand buffers of the calls too large for a pinned slot.
+  double *d_sig_pol = nullptr;
+  uint8_t *d_sig_flags = nullptr;
+  bool has_signals = false;
+  unsigned char *d_mention_io = nullptr;
+  size_t mention_io_bytes = 0;
+
   // multi-GPU
   OiComm *comm = nullptr;
   int rank = 0, world = 1;
@@ -101,6 +109,46 @@ struct oi_index {
   oi_status fail(oi_status code, const char *fmt, ...) __attribute__((format(printf, 3, 4)));
 };
 
+// api.cu: device-side ordering of the calls of one handle (see ev_last)
+cudaError_t call_begin(oi_index *h, cudaStream_t st);
+cudaError_t call_end(oi_index *h, cudaStream_t st);
+
+// A staging slot for one small host-buffer call.  Taken under the handle's lock (waiting, lock released, while all are
+// busy); given back by the guard after the caller has copied its results out -- or on any early return.
+struct SlotLease {
+  oi_index *h;
+  std::unique_lock<std::mutex> &lock;
+  oi_index::Slot *sl;
+  SlotLease(oi_index *h_, std::unique_lock<std::mutex> &lock_) : h(h_), lock(lock_), sl(nullptr) {
+    for (;;) {
+      for (oi_index::Slot &c : h->slots)
+        if (!c.busy) { sl = &c; break; }
+      if (sl) break;
+      h->slot_cv.wait(lock);
+    }
+    sl->busy = true;
+  }
+  ~SlotLease() {
+    if (!lock.owns_lock()) lock.lock();
+    sl->busy = false;
+    h->slot_cv.notify_one();
+  }
+  // the enqueue is complete: record the slot's event, let the next caller in, wait for this call's results
+  oi_status finish(cudaStream_t st) {
+    cudaError_t e = cudaEventRecord(sl->done, st);
+    if (e == cudaSuccess) e = call_end(h, st);
+    if (e == cudaSuccess) {
+      lock.unlock();
+      e = cudaEventSynchronize(sl->done);
+      if (e != cudaSuccess) lock.lock();
+    }
+    if (e != cudaSuccess) return h->fail(OI_ERR_CUDA, "host-buffer call failed: %s", cudaGetErrorString(e));
+    return OI_OK;
+  }
+};
+
+// mention.cu
+void oi_mention_free(oi_index *h);
 // bm25.cu
 void oi_bm25_free(oi_index *h);
 // installs a CSR that already lives on the device (text_index.cu) as the BM25 part, as oi_index_load_bm25 leaves it;
@@ -109,6 +157,7 @@ oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 
                         uint32_t *d_tfs, uint32_t *d_doc_len);
 uint32_t oi_bm25_n_terms(const oi_index *h);  // 0 = no BM25 part
 const u64 *oi_bm25_term_offsets(const oi_index *h);  // device term_offsets[n_terms + 1]; NULL = no BM25 part
+const uint32_t *oi_bm25_doc_ids(const oi_index *h);  // device doc_ids[n_postings] (kept after finalize); NULL = no BM25 part
 bool oi_bm25_finalized(const oi_index *h);
 // re-indexes the BM25 part to n_terms terms over the same postings (text_index.cu's vocabulary union): d_term_off
 // [n_terms + 1] on the device becomes the index's, the old offsets are freed.  Before finalize only.

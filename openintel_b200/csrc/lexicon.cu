@@ -24,6 +24,7 @@
 #include <string>
 
 #include "internal.h"
+#include "oi_summary.cuh"
 #include "oi_tokenize.cuh"
 
 namespace {
@@ -213,77 +214,11 @@ __global__ void __launch_bounds__(256) lexicon_kernel(const uint8_t *texts, cons
 
 void oi_set_thread_error(const std::string &msg);  // api.cu
 
-// The reference's social summary over the batch's signals (src/domain/engine/speculation_engine.rs:76-84).  The mean is
-// a SEQUENTIAL f64 sum there, so it is one here: every partial sum is rounded as the reference rounds it and the result
-// is bit-identical.  One CTA: all threads stream the signals tile by tile into a double-buffered shared-memory ring
-// (coalesced) and count the classes (order-free, integer); thread 0 runs the add chain over the tile loaded one step
-// earlier, so the chain never waits for memory -- its price is the dependent DADD latency (~19 cycles measured) per
-// post with a non-zero polarity, nothing else.
-constexpr int kSumTile = 2048;
+// The reference's social summary over the batch's signals (src/domain/engine/speculation_engine.rs:76-84): one CTA, the
+// shared summary body (oi_summary.cuh) over the identity order.
 __global__ void __launch_bounds__(128) social_summary_kernel(const double *polarity, const uint8_t *speculative, unsigned long long n, double thr,
                                                              oi_social_summary *out) {
-  __shared__ double s_v[2][kSumTile];   // the tile's NON-ZERO polarities, in post order
-  __shared__ int s_m[2];                // how many
-  __shared__ int s_wsum[4];
-  __shared__ unsigned long long s_cnt[4];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid < 4) s_cnt[tid] = 0ull;
-  unsigned long long bullish = 0, bearish = 0, neutral = 0, spec = 0;
-  double sum = 0.0;
-  const unsigned long long n_tiles = (n + kSumTile - 1) / kSumTile;
-  for (unsigned long long t = 0; t <= n_tiles; ++t) {
-    if (t < n_tiles) {  // stage tile t: thread i owns posts 16 i .. 16 i + 15 of the tile (one 128-byte line)
-      const unsigned long long base = t * kSumTile + 16ull * tid;
-      double v[16];
-      int c = 0;
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const unsigned long long g = base + j;
-        v[j] = 0.0;
-        if (g < n) {
-          v[j] = polarity[g];
-          if (v[j] > thr) ++bullish;
-          else if (v[j] < -thr) ++bearish;
-          else ++neutral;
-          spec += speculative[g] != 0;
-        }
-        c += v[j] != 0.0;  // s + 0.0 == s exactly (there are no -0.0 inputs): posts without a hit stay out of the chain
-      }
-      int x = c;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xFFFFFFFFu, x, o);
-        if (lane >= o) x += y;
-      }
-      if (lane == 31) s_wsum[warp] = x;
-      __syncthreads();
-      int off = x - c;
-      for (int w = 0; w < warp; ++w) off += s_wsum[w];
-      double *dst = s_v[t & 1];
-#pragma unroll
-      for (int j = 0; j < 16; ++j)
-        if (v[j] != 0.0) dst[off++] = v[j];
-      if (tid == 127) s_m[t & 1] = off;
-    }
-    if (tid == 0 && t > 0) {  // the add chain over tile t - 1, in post order
-      const int m = s_m[(t - 1) & 1];
-      const double *v = s_v[(t - 1) & 1];
-#pragma unroll 8
-      for (int i = 0; i < m; ++i) sum += v[i];
-    }
-    __syncthreads();
-  }
-  atomicAdd(&s_cnt[0], bullish); atomicAdd(&s_cnt[1], bearish); atomicAdd(&s_cnt[2], neutral); atomicAdd(&s_cnt[3], spec);
-  __syncthreads();
-  if (tid != 0) return;
-  bullish = s_cnt[0]; bearish = s_cnt[1]; neutral = s_cnt[2]; spec = s_cnt[3];
-  double net = n == 0 ? 0.0 : sum / (double)n;
-  double si = n == 0 ? 0.0 : (double)spec / (double)n;
-  net = net > 1.0 ? 1.0 : (net < -1.0 ? -1.0 : net);
-  si = si > 1.0 ? 1.0 : (si < 0.0 ? 0.0 : si);
-  out->total = n; out->bullish = bullish; out->bearish = bearish; out->neutral = neutral;
-  out->net_sentiment = net; out->speculation_index = si;
-  out->bull_bear_ratio = bearish == 0 ? -1.0 : (double)bullish / (double)bearish;
+  oi_social_summary_cta<false>(polarity, speculative, nullptr, 0ull, n, -1, thr, nullptr, nullptr, out);
 }
 
 struct oi_lexicon {

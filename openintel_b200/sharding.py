@@ -74,6 +74,39 @@ def all_gather_packed(dist, blob, offsets, device="cpu"):
     return out_blob, np.concatenate([[0], np.cumsum(out_lens)]).astype(np.uint64)
 
 
+def relay_mention_summary(dist, ix, term_ids, source=None, threshold=0.2, device="cpu"):
+    """The social summaries of `term_ids` over the posting lists of a document-sharded index (SPEC §8a), the same on
+    every rank: rank 0 summarises its shard and sends its running states to rank 1; every later rank receives them,
+    continues each term's chain over its own shard (GpuIndex.mention_summary with carry) and sends on; the last rank
+    broadcasts the final states and summaries.
+
+    The relay is sequential over the ranks by design: the reference's mean is a sequential f64 sum in doc order and the
+    shards hold contiguous doc ranges in rank order, so only carrying the running sum from shard to shard reproduces it
+    bit for bit -- an all-reduce of per-shard partial sums would round differently.  `dist` = torch.distributed
+    (initialised) or None for a single shard; every rank passes the same term ids.  -> (states, summaries) as
+    GpuIndex.mention_summary returns them."""
+    if dist is None or dist.get_world_size() == 1 or len(term_ids) == 0:
+        return ix.mention_summary(term_ids, source, threshold)
+    import torch
+    rank, world = dist.get_rank(), dist.get_world_size()
+    n = len(term_ids)
+    carry = None
+    if rank > 0:
+        buf = torch.empty(n * capi.MENTION_STATE_DTYPE.itemsize, dtype=torch.uint8, device=device)
+        dist.recv(buf, src=rank - 1)
+        carry = buf.cpu().numpy().view(capi.MENTION_STATE_DTYPE)
+    states, sums = ix.mention_summary(term_ids, source, threshold, carry)
+    if rank < world - 1:
+        dist.send(torch.from_numpy(states.view(np.uint8).copy()).to(device), dst=rank + 1)
+    # the last rank's states and summaries, as bytes, to everybody
+    raw = capi.summaries_to_array(sums) if rank == world - 1 else np.zeros(n, dtype=capi.SOCIAL_SUMMARY_DTYPE)
+    out = torch.from_numpy(np.concatenate([states.view(np.uint8), raw.view(np.uint8)])).to(device)
+    dist.broadcast(out, world - 1)
+    out = out.cpu().numpy()
+    cut = n * capi.MENTION_STATE_DTYPE.itemsize
+    return out[:cut].copy().view(capi.MENTION_STATE_DTYPE), capi.summaries_from_array(out[cut:].copy().view(capi.SOCIAL_SUMMARY_DTYPE))
+
+
 def broadcast_unique_id(dist, device="cpu"):
     """rank 0 creates the NCCL unique id (C ABI), everybody receives it."""
     import torch

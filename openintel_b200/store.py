@@ -24,7 +24,7 @@ import sqlite3
 
 import numpy as np
 
-from . import capi, hostlib
+from . import capi, fusion, hostlib
 
 MAX_POST_LEN = 10_000  # chars, not bytes (social_post.rs:7, :19)
 SOURCES = ("reddit", "bluesky")
@@ -312,7 +312,7 @@ def lift_shard(conn, dist, rank=None, world=None, device="cpu"):
                 post_ids=ids)
 
 
-def lift_shard_gpu(conn, dist, device="cpu", device_index=0, max_k=100, max_batch=16):
+def lift_shard_gpu(conn, dist, device="cpu", device_index=0, max_k=100, max_batch=16, with_embeddings=True):
     """lift_shard on the device: the same shard, built into an open GpuIndex on `device_index` --
       * the rank's contiguous doc range is tokenised and indexed by oi_index_build_bm25_text,
       * the packed vocabularies are all-gathered (sharding.all_gather_packed) and oi_index_bm25_union_vocabulary
@@ -322,8 +322,10 @@ def lift_shard_gpu(conn, dist, device="cpu", device_index=0, max_k=100, max_batc
     entries and loads an all-empty CSR over it.
 
     `dist` = torch.distributed (initialised, gloo or nccl) or None; `device` = where its collectives run.  The index is
-    not finalized: load the embeddings, then bm25_finalize with global_df / avgdl / n_docs_global.  -> dict(index,
-    doc_base, n_local, n_docs_global, vocab, global_df, avgdl, post_ids (this shard's))"""
+    not finalized: load the embeddings, then bm25_finalize with global_df / avgdl / n_docs_global.  with_embeddings=False:
+    an index for the BM25 part alone (mention summaries, SPEC §8a) -- the store needs no embeddings and the index holds
+    the smallest row it takes (4 f32), never loaded.  -> dict(index, doc_base, n_local, n_docs_global, vocab, global_df,
+    avgdl, post_ids (this shard's))"""
     from . import sharding
     n_total = conn.execute("SELECT COUNT(*) FROM posts").fetchone()[0]
     if dist is not None and dist.get_world_size() > 1:
@@ -340,7 +342,7 @@ def lift_shard_gpu(conn, dist, device="cpu", device_index=0, max_k=100, max_batc
         ids.append(post_id)
     if len(texts) != n_local:
         raise ValueError("posts.doc_id must be dense 0..N-1 (gap at %d)" % (base + len(texts)))
-    dim = store_dim(conn)
+    dim = store_dim(conn) if with_embeddings else 4
     if dim is None:
         raise ValueError("store has no embeddings")
     ix = capi.GpuIndex(n_docs=n_local, dim=dim, device=device_index, doc_base=base, max_k=max_k, max_batch=max_batch)
@@ -414,6 +416,71 @@ class ShardedStoreIndex:
     def search(self, texts, vectors, k, rrf_k=60):
         q = normalise_rows_f32(np.asarray(vectors, dtype=np.float32).reshape(len(texts), self.dim))
         return self.ix.search_hybrid(q, self.query_terms(texts), k, rrf_k)
+
+    def close(self):
+        self.ix.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+
+class MentionIndex:
+    """Per-ticker social reports from the index (SPEC §8a): the posts that mention a ticker are its posting list, so
+    the reference's `analyze --mention` report of many tickers takes one device call (one relay over the ranks of a
+    document-sharded index) instead of a pass over the store per ticker.
+
+    Every rank lifts its doc range through lift_shard_gpu (unsharded when `dist` is None; the store needs no
+    embeddings), scores its posts with the GPU PostAnalyzer and loads the signals and source codes next to the BM25
+    part.  reports() returns on every rank exactly what analyze.analyze_posts returns for select_posts(source,
+    mention=ticker)."""
+
+    def __init__(self, conn, dist=None, device_index=0):
+        self.dist = dist if (dist is not None and dist.get_world_size() > 1) else None
+        # the relay's control plane: CPU tensors over gloo, the rank's GPU over NCCL
+        self.device = "cpu" if self.dist is None or self.dist.get_backend() == "gloo" else "cuda:%d" % device_index
+        sh = lift_shard_gpu(conn, self.dist, device=self.device, device_index=device_index, max_k=1, max_batch=1,
+                            with_embeddings=False)
+        self.ix = sh["index"]
+        self.term_id = {w: i for i, w in enumerate(sh["vocab"])}
+        self.doc_base, self.n_local = sh["doc_base"], sh["n_local"]
+        try:
+            rows = conn.execute("SELECT source, text FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
+                                (self.doc_base, self.doc_base + self.n_local)).fetchall()
+            with capi.GpuLexicon(device_index) as lx:
+                pol, spec, _, _ = lx.analyze([r[1] for r in rows])
+            self.ix.load_post_signals(pol, spec, [SOURCES.index(r[0]) for r in rows])
+        except Exception:
+            self.ix.close()
+            raise
+
+    def reports(self, tickers, source=None, markets=None, cfg=fusion.EngineConfig()):
+        """one report per ticker, in the order given: analyze.build_report of the ticker's posts (of `source` only, when
+        given).  A ticker is normalised like select_posts' mention (leading '$' dropped, lower case); `markets` maps
+        tickers, normalised the same way, to fusion.MarketSummary.  A ticker with no post and no market snapshot -- what
+        analyze refuses with NoData -- gives None."""
+        from . import analyze, sharding
+        keys = [t.lstrip("$").lower() for t in tickers]
+        mk = {k.lstrip("$").lower(): v for k, v in (markets or {}).items()}
+        known = [k for k in dict.fromkeys(keys) if k in self.term_id]  # a ticker outside the vocabulary has no post
+        states, sums = sharding.relay_mention_summary(
+            self.dist, self.ix, np.array([self.term_id[k] for k in known], dtype=np.uint32),
+            None if source is None else SOURCES.index(source), cfg.bull_bear_threshold, device=self.device)
+        found = {k: (st, sm) for k, st, sm in zip(known, states, sums)}
+        out = []
+        for k in keys:
+            if k in found:
+                st, sm = found[k]
+                by_source = {SOURCES[s]: int(st["by_source"][s]) for s in range(len(SOURCES))}
+            else:
+                sm, by_source = analyze.empty_summary(), {}
+            try:
+                out.append(analyze.build_report(sm, by_source, mk.get(k), cfg))
+            except analyze.NoData:
+                out.append(None)
+        return out
 
     def close(self):
         self.ix.close()

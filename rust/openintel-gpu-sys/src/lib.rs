@@ -18,6 +18,8 @@ pub const OI_UNIQUE_ID_BYTES: usize = 128;
 pub const OI_P2P_HANDLE_BYTES: usize = 64;
 pub const OI_DTYPE_F32: u32 = 0;
 pub const OI_DTYPE_BF16: u32 = 1;
+/// post sources in store-schema order: 0 = reddit, 1 = bluesky
+pub const OI_N_SOURCES: usize = 2;
 
 #[repr(C)]
 pub struct oi_index {
@@ -40,6 +42,20 @@ pub struct oi_social_summary {
     pub net_sentiment: f64,
     pub speculation_index: f64,
     pub bull_bear_ratio: f64,
+}
+
+/// the running state of one term's summary after a prefix of the doc order (docs/SPEC.md §8a)
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct oi_mention_state {
+    pub total: u64,
+    pub bullish: u64,
+    pub bearish: u64,
+    pub neutral: u64,
+    pub speculative: u64,
+    pub by_source: [u64; OI_N_SOURCES],
+    /// sequential f64 sum of the polarities so far, doc order
+    pub sum: f64,
 }
 
 #[repr(C)]
@@ -116,6 +132,11 @@ extern "C" {
                           out_speculative: *mut u8, out_bull_hits: *mut u32, out_bear_hits: *mut u32, bull_bear_threshold: f64,
                           out_summary: *mut oi_social_summary) -> oi_status;
     pub fn oi_lexicon_launch_count(lx: *const oi_lexicon) -> u64;
+
+    pub fn oi_index_load_post_signals(h: *mut oi_index, polarity: *const f64, speculative: *const u8, source: *const u8) -> oi_status;
+    pub fn oi_index_mention_summary(h: *mut oi_index, terms: *const u32, n_terms: u32, source: i32, bull_bear_threshold: f64,
+                                    carry_in: *const oi_mention_state, out_state: *mut oi_mention_state,
+                                    out_summary: *mut oi_social_summary) -> oi_status;
 
     pub fn oi_index_launch_count(h: *const oi_index) -> u64;
     pub fn oi_index_set_option(h: *mut oi_index, name: *const c_char, value: i64) -> oi_status;
