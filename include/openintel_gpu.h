@@ -241,6 +241,30 @@ oi_status oi_index_mention_summary(oi_index *h, const uint32_t *terms, uint32_t 
                                    double bull_bear_threshold, const oi_mention_state *carry_in,
                                    oi_mention_state *out_state, oi_social_summary *out_summary);
 
+/* ---- per-term timelines: the summaries above split by creation time (docs/SPEC.md §8b) ------
+ * Bucket b of edges[0 .. n_buckets] is [edges[b], edges[b+1]) in seconds since the Unix epoch; a post outside
+ * [edges[0], edges[n_buckets]) is in no bucket.  The summary of (term, bucket) is the §8a summary of the posts that
+ * mention the term and fall in the bucket, in doc order, so with one bucket around all posts it equals
+ * oi_index_mention_summary bit for bit.  A document-sharded index relays each (term, bucket) state in rank order
+ * exactly as oi_index_mention_summary does. */
+
+/* per-post creation times of THIS shard, n = n_docs, host memory, seconds since the Unix epoch (SPEC §8b).
+ * Independent of the BM25 part and of the signals; a rebuilt BM25 part keeps them. */
+oi_status oi_index_load_post_times(oi_index *h, const int64_t *created_at);
+
+/* for term i of terms[0..n_terms) and bucket b of edges[0..n_buckets]: the social summary of this shard's posts that
+ * mention the term and were created in [edges[b], edges[b+1]), doc order, continued from carry_in[i * n_buckets + b]
+ * (NULL = nothing before this shard).  out_state (may be NULL) / out_summary: [n_terms][n_buckets], term-major.
+ * source and duplicate term ids as in oi_index_mention_summary.  n_terms == 0 is a no-op.
+ * OI_ERR_STATE: no BM25 part, no signals or no times loaded.  OI_ERR_INVALID_ARG: NULL terms / edges / out_summary,
+ * n_buckets == 0, n_terms x n_buckets > 2^32 - 1 (the (term, bucket) keys are 32-bit), edges not strictly increasing,
+ * a term id >= the BM25 part's n_terms, source outside -1 .. OI_N_SOURCES - 1.  A refused call changes nothing.
+ * Blocking; reads the posting lists only, so it works before and after oi_index_bm25_finalize. */
+oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *terms, uint32_t n_terms, const int64_t *edges,
+                                    uint32_t n_buckets, int32_t source, double bull_bear_threshold,
+                                    const oi_mention_state *carry_in, oi_mention_state *out_state,
+                                    oi_social_summary *out_summary);
+
 /* ---- tuning / introspection (bench + tests) ------------------------------------------------ */
 /* number of kernels this handle has launched since creation (bench "gpu_launches") */
 uint64_t oi_index_launch_count(const oi_index *h);

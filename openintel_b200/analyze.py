@@ -23,15 +23,28 @@ class NoData(ValueError):
     """DomainError::NoData (src/application/analyze.rs:58-60): neither posts nor a market snapshot"""
 
 
-def select_posts(conn, source=None, mention=None, limit=None):
+def select_posts(conn, source=None, mention=None, limit=None, since=None, until=None):
     """(ids, sources, texts) of the stored posts in doc order; `mention`: keep posts one of whose tokens equals it
-    (case-insensitive, a leading '$' ignored: the reference's tokenizer drops it too)"""
-    sql, args = "SELECT id, source, text FROM posts", []
+    (case-insensitive, a leading '$' ignored: the reference's tokenizer drops it too); `since` / `until`: keep posts
+    created in [since, until), seconds since the Unix epoch (store.parse_created_at; SPEC §8b), before `limit`"""
+    window = since is not None or until is not None
+    sql, args = "SELECT id, source, text%s FROM posts" % (", doc_id, created_at" if window else ""), []
     if source:
         sql += " WHERE source = ?"
         args.append(source)
     sql += " ORDER BY doc_id"
     rows = conn.execute(sql, args).fetchall()
+    if window:
+        from .store import parse_created_at
+        kept = []
+        for r in rows:
+            try:
+                t = parse_created_at(r[4])
+            except ValueError as e:
+                raise ValueError("post doc_id %d: %s" % (r[3], e)) from None
+            if (since is None or t >= since) and (until is None or t < until):
+                kept.append(r)
+        rows = kept
     if mention:
         from . import hostlib
         want = mention.lstrip("$").lower()
@@ -46,6 +59,19 @@ def empty_summary():
     return dict(total=0, bullish=0, bearish=0, neutral=0, net_sentiment=0.0, speculation_index=0.0, bull_bear_ratio=-1.0)
 
 
+def social_block(sm, mentions_by_source):
+    """the "social" block of a report (the reference's SocialSummary as SpeculationReport shows it): sm: a summary dict
+    shaped like GpuLexicon's; mentions_by_source: {source name: post count}"""
+    by_source = OrderedDict()
+    for s in sorted(mentions_by_source):  # the reference keeps a BTreeMap: sorted keys
+        if mentions_by_source[s]:
+            by_source[s] = int(mentions_by_source[s])
+    return {"total_mentions": int(sm["total"]), "mentions_by_source": by_source, "net_sentiment": sm["net_sentiment"],
+            "bullish": int(sm["bullish"]), "bearish": int(sm["bearish"]), "neutral": int(sm["neutral"]),
+            "bull_bear_ratio": None if sm["bull_bear_ratio"] < 0 else sm["bull_bear_ratio"],
+            "speculation_index": sm["speculation_index"]}
+
+
 def build_report(sm, mentions_by_source, market=None, cfg=fusion.EngineConfig()):
     """The rest of SpeculationEngine::aggregate (src/domain/engine/speculation_engine.rs:21-66) once the social summary
     is known: the fusion signals and a report shaped like the reference's SpeculationReport.  sm: a summary dict shaped
@@ -54,16 +80,9 @@ def build_report(sm, mentions_by_source, market=None, cfg=fusion.EngineConfig())
     if sm["total"] == 0 and market is None:
         raise NoData("no posts and no market snapshot")
     notes = []
-    by_source = OrderedDict()
-    for s in sorted(mentions_by_source):  # the reference keeps a BTreeMap: sorted keys
-        if mentions_by_source[s]:
-            by_source[s] = int(mentions_by_source[s])
     if market is None:
         notes.append("social-only, no price reference")
-    social = {"total_mentions": int(sm["total"]), "mentions_by_source": by_source, "net_sentiment": sm["net_sentiment"],
-              "bullish": int(sm["bullish"]), "bearish": int(sm["bearish"]), "neutral": int(sm["neutral"]),
-              "bull_bear_ratio": None if sm["bull_bear_ratio"] < 0 else sm["bull_bear_ratio"],
-              "speculation_index": sm["speculation_index"]}
+    social = social_block(sm, mentions_by_source)
 
     class _S:
         total, net_sentiment, speculation_index = social["total_mentions"], social["net_sentiment"], social["speculation_index"]
@@ -92,6 +111,8 @@ def main(argv=None):
     ap.add_argument("--store", required=True, help="SQLite post store (openintel_b200.store schema)")
     ap.add_argument("--source", choices=["reddit", "bluesky"], help="only this source's posts")
     ap.add_argument("--mention", help="only posts that mention this cashtag / word (e.g. GME)")
+    ap.add_argument("--since", help="only posts created at or after this RFC 3339 time (e.g. 2024-01-01T00:00:00Z)")
+    ap.add_argument("--until", help="only posts created before this RFC 3339 time")
     ap.add_argument("--limit", type=int, help="at most this many posts")
     ap.add_argument("--market", help="last_price,previous_close,volume,avg_volume[,iv_rank]")
     ap.add_argument("--device", type=int, default=0)
@@ -103,8 +124,20 @@ def main(argv=None):
         if len(f) not in (4, 5):
             ap.error("--market takes last_price,previous_close,volume,avg_volume[,iv_rank]")
         market = fusion.MarketSummary.from_snapshot(float(f[0]), float(f[1]), int(f[2]), int(f[3]), float(f[4]) if len(f) == 5 else None)
+    since = until = None
+    try:
+        if args.since is not None:
+            since = store.parse_created_at(args.since)
+        if args.until is not None:
+            until = store.parse_created_at(args.until)
+    except ValueError as e:
+        ap.error("--since / --until: %s" % e)
     conn = store.open_store(args.store)
-    _, sources, texts = select_posts(conn, args.source, args.mention, args.limit)
+    try:
+        _, sources, texts = select_posts(conn, args.source, args.mention, args.limit, since, until)
+    except ValueError as e:  # a stored created_at that is not RFC 3339 with an offset
+        sys.stderr.write("error: %s\n" % e)
+        return 1
     with capi.GpuLexicon(args.device) as lx:
         try:
             report, _, _ = analyze_posts(lx, sources, texts, market)

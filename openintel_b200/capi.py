@@ -104,6 +104,8 @@ def load_library():
         "oi_lexicon_launch_count": (C.c_uint64, [H]),
         "oi_index_load_post_signals": (st, [H, _vp, _vp, _vp]),
         "oi_index_mention_summary": (st, [H, _u32p, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
+        "oi_index_load_post_times": (st, [H, _vp]),
+        "oi_index_mention_timeline": (st, [H, _u32p, C.c_uint32, _vp, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
         "oi_index_launch_count": (C.c_uint64, [H]),
         "oi_index_set_option": (st, [H, C.c_char_p, C.c_int64]),
         "oi_debug_cosine_gemm_scores": (st, [H, _f32p, C.c_uint32, _f32p]),
@@ -275,6 +277,32 @@ class GpuIndex:
         self._ck(self.L.oi_index_mention_summary(self.h, _addr(terms), n, -1 if source is None else int(source), threshold,
                                                   _addr(cin), _addr(states), _addr(sums)))
         return states, summaries_from_array(sums)
+
+    # -- per-term timelines (SPEC §8b)
+    def load_post_times(self, seconds):
+        """per-post creation times of this shard, in doc order: int64 seconds since the Unix epoch"""
+        t = np.ascontiguousarray(seconds, dtype=np.int64)
+        if t.ndim != 1 or len(t) != self.n_docs:
+            raise ValueError("need %d post times, got %d" % (self.n_docs, t.size))
+        self._ck(self.L.oi_index_load_post_times(self.h, _addr(t)))
+
+    def mention_timeline(self, term_ids, edges, source=None, threshold=0.2, carry=None):
+        """the social summary of each term's posts in each bucket [edges[b], edges[b + 1]) on this shard
+        (oi_index_mention_timeline), continued from `carry` ([n][B] states of the previous shard, or None).
+        -> (states: MENTION_STATE_DTYPE [n][B], summaries: n lists of B dicts shaped like GpuLexicon's summary)"""
+        terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
+        e = np.ascontiguousarray(edges, dtype=np.int64).reshape(-1)
+        n, nb = len(terms), max(len(e) - 1, 0)
+        states = np.zeros((n, nb), dtype=MENTION_STATE_DTYPE)
+        sums = np.zeros((n, nb), dtype=SOCIAL_SUMMARY_DTYPE)
+        cin = None
+        if carry is not None:
+            cin = np.ascontiguousarray(carry, dtype=MENTION_STATE_DTYPE)
+            if cin.size != n * nb:
+                raise ValueError("%d carried states for %d terms x %d buckets" % (cin.size, n, nb))
+        self._ck(self.L.oi_index_mention_timeline(self.h, _addr(terms), n, _addr(e), nb, -1 if source is None else int(source),
+                                                   threshold, _addr(cin), _addr(states), _addr(sums)))
+        return states, [summaries_from_array(row) for row in sums]
 
     # -- multi-GPU
     @staticmethod

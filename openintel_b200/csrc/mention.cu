@@ -7,6 +7,15 @@
 // its longest list's chain (one dependent DADD per mentioning post with a non-zero polarity); the gather hides behind the
 // chain in the tile ring.  The running state in and out lets the shards of a document-sharded index continue one
 // another's sequential sum in rank order (a relay), which keeps the mean bit-identical to the unsharded one.
+//
+// Timelines (SPEC §8b): with a creation time per post, a time bucket splits a posting list into doc-order subsequences.
+// One thread per requested posting keys it by (term, bucket); one stable radix sort groups the keys, which keeps every
+// (term, bucket) segment in doc order because the input is in (term, doc) order; a binary search in the sorted keys gives
+// the segment offsets, and the same summary body runs once per segment.  The chains of all segments run side by side,
+// so a call costs about its largest segment's chain, plus a fixed cost per segment that dominates when there are
+// millions of tiny ones (DESIGN §4.4).
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cstring>
 #include <vector>
 
@@ -26,7 +35,92 @@ __global__ void __launch_bounds__(128) mention_summary_kernel(const double *pola
   }
 }
 
+// ---- timelines (SPEC §8b)
+constexpr int kEdgesInSmem = 4096;  // edges[0 .. n_buckets] staged in shared memory (32 KB) when they fit
+
+// len[i] = the length of term i's list, len[n] = 0: the exclusive scan in place makes len the lists' starts in the
+// concatenation of the requested lists and len[n] their total
+__global__ void timeline_lengths_kernel(const u64 *term_off, const uint32_t *terms, uint32_t n, u64 *len) {
+  for (u64 i = blockIdx.x * (u64)blockDim.x + threadIdx.x; i <= n; i += (u64)gridDim.x * blockDim.x)
+    len[i] = i < n ? term_off[terms[i] + 1] - term_off[terms[i]] : 0;
+}
+
+// posting p of the concatenation -> key i * nb + b (term i, bucket b) or the sentinel n * nb when the post's time is
+// outside [edges[0], edges[nb]); value = the doc id.  start[0 .. n]: the lists' starts, start[n] = total.
+__global__ void __launch_bounds__(256) timeline_keys_kernel(const u64 *term_off, const uint32_t *doc_ids, const int64_t *times,
+                                                            const uint32_t *terms, const u64 *start, uint32_t n, u64 total,
+                                                            const int64_t *edges, uint32_t nb, uint32_t *keys, uint32_t *vals) {
+  __shared__ int64_t s_edges[kEdgesInSmem];
+  const bool staged = nb < kEdgesInSmem;
+  if (staged)
+    for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_edges[k] = edges[k];
+  __syncthreads();
+  const int64_t *E = staged ? s_edges : edges;
+  const int64_t t_lo = E[0], t_hi = E[nb];
+  for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
+    uint32_t a = 0, b = n;  // the term: start[a] <= p < start[b] (an empty list shares its start with the next one)
+    while (b - a > 1) {
+      const uint32_t m = (a + b) >> 1;
+      if (start[m] <= p) a = m; else b = m;
+    }
+    const uint32_t doc = doc_ids[term_off[terms[a]] + (p - start[a])];
+    const int64_t t = times[doc];
+    u64 key = (u64)n * nb;
+    if (t >= t_lo && t < t_hi) {
+      uint32_t lo = 0, hi = nb;  // the bucket: E[lo] <= t < E[hi]
+      while (hi - lo > 1) {
+        const uint32_t m = (lo + hi) >> 1;
+        if (E[m] <= t) lo = m; else hi = m;
+      }
+      key = (u64)a * nb + lo;
+    }
+    keys[p] = (uint32_t)key;
+    vals[p] = doc;
+  }
+}
+
+// seg_off[j] = the first place of the sorted keys holding a key >= j, j = 0 .. n_seg: segment j is
+// [seg_off[j], seg_off[j + 1]), and the sentinel's postings follow seg_off[n_seg]
+__global__ void timeline_segments_kernel(const uint32_t *keys, u64 total, u64 n_seg, u64 *seg_off) {
+  for (u64 j = blockIdx.x * (u64)blockDim.x + threadIdx.x; j <= n_seg; j += (u64)gridDim.x * blockDim.x) {
+    u64 lo = 0, hi = total;
+    while (lo < hi) {
+      const u64 m = (lo + hi) >> 1;
+      if (keys[m] < j) lo = m + 1; else hi = m;
+    }
+    seg_off[j] = lo;
+  }
+}
+
+// the summary body, unchanged, once per (term, bucket) segment of the sorted doc ids
+__global__ void __launch_bounds__(128) mention_timeline_kernel(const double *polarity, const uint8_t *flags, const uint32_t *docs,
+                                                               const u64 *seg_off, u64 n_seg, int source, double thr,
+                                                               const oi_mention_state *carry, oi_mention_state *out_state,
+                                                               oi_social_summary *out) {
+  for (u64 j = blockIdx.x; j < n_seg; j += gridDim.x)
+    oi_social_summary_cta<true>(polarity, flags, docs, seg_off[j], seg_off[j + 1] - seg_off[j], source, thr,
+                                carry ? carry + j : nullptr, out_state + j, out + j);
+}
+
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+unsigned grid_for(u64 n, int num_sms) {
+  const u64 b = (n + 255) / 256, cap = (u64)num_sms * 16;
+  return (unsigned)(b == 0 ? 1 : (b < cap ? b : cap));
+}
+
+// a grow-on-demand device buffer of the handle: at least `want` bytes, with 25 % headroom when it grows
+cudaError_t grow(unsigned char *&buf, size_t &cap, size_t want, cudaStream_t st) {
+  if (want <= cap) return cudaSuccess;
+  cudaError_t e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return e;
+  cudaFree(buf);
+  buf = nullptr;
+  cap = 0;
+  e = cudaMalloc(&buf, want + want / 4);
+  if (e == cudaSuccess) cap = want + want / 4;
+  return e;
+}
 
 }  // namespace
 
@@ -42,11 +136,17 @@ void oi_mention_free(oi_index *h) {
   cudaFree(h->d_sig_pol);
   cudaFree(h->d_sig_flags);
   cudaFree(h->d_mention_io);
+  cudaFree(h->d_times);
+  cudaFree(h->d_timeline_ws);
   h->d_sig_pol = nullptr;
   h->d_sig_flags = nullptr;
   h->d_mention_io = nullptr;
   h->mention_io_bytes = 0;
   h->has_signals = false;
+  h->d_times = nullptr;
+  h->has_times = false;
+  h->d_timeline_ws = nullptr;
+  h->timeline_ws_bytes = 0;
 }
 
 extern "C" oi_status oi_index_load_post_signals(oi_index *h, const double *polarity, const uint8_t *speculative,
@@ -142,21 +242,140 @@ extern "C" oi_status oi_index_mention_summary(oi_index *h, const uint32_t *terms
   }
   // a large call: the handle's own device buffers, direct copies from / to the caller's memory
   const size_t o_out = align16(in_bytes);
-  if (o_out + out_bytes > h->mention_io_bytes) {
-    MN_CK(cudaStreamSynchronize(st));
-    cudaFree(h->d_mention_io);
-    h->d_mention_io = nullptr;
-    h->mention_io_bytes = 0;
-    const size_t want = (o_out + out_bytes) + (o_out + out_bytes) / 4;
-    MN_CK(cudaMalloc(&h->d_mention_io, want));
-    h->mention_io_bytes = want;
-  }
+  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_out + out_bytes, st));
   unsigned char *d_in = h->d_mention_io, *d_out = h->d_mention_io + o_out;
   MN_CK(cudaMemcpyAsync(d_in, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
   if (carry_in) MN_CK(cudaMemcpyAsync(d_in + o_carry, carry_in, n * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
   MN_CK(launch(d_in, d_out));
   if (out_state) MN_CK(cudaMemcpyAsync(out_state, d_out, n * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
   MN_CK(cudaMemcpyAsync(out_summary, d_out + o_sum, n * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
+  MN_CK(call_end(h, st));
+  MN_CK(cudaStreamSynchronize(st));
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_load_post_times(oi_index *h, const int64_t *created_at) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  if (!created_at) return h->fail(OI_ERR_INVALID_ARG, "NULL created_at");
+  const u64 n = h->desc.n_docs;
+  MN_CK(cudaSetDevice(h->desc.device));
+  if (!h->d_times) {
+    const cudaError_t e = cudaMalloc(&h->d_times, (n ? n : 1) * sizeof(int64_t));
+    if (e != cudaSuccess) {
+      h->d_times = nullptr;
+      return h->fail(e == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA, "allocating the post times failed: %s",
+                     cudaGetErrorString(e));
+    }
+  }
+  MN_CK(call_begin(h, h->stream));
+  h->has_times = false;  // until the copy has landed
+  if (n) MN_CK(cudaMemcpyAsync(h->d_times, created_at, n * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+  MN_CK(call_end(h, h->stream));
+  MN_CK(cudaStreamSynchronize(h->stream));
+  h->has_times = true;
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *terms, uint32_t n_terms, const int64_t *edges,
+                                               uint32_t n_buckets, int32_t source, double bull_bear_threshold,
+                                               const oi_mention_state *carry_in, oi_mention_state *out_state,
+                                               oi_social_summary *out_summary) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  const u64 *term_off = oi_bm25_term_offsets(h);
+  if (!term_off) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
+  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
+  if (!h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
+  if (n_terms == 0) return OI_OK;
+  if (!terms || !edges || !out_summary) return h->fail(OI_ERR_INVALID_ARG, "NULL terms / edges / out_summary");
+  if (n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "n_buckets = 0: a timeline needs a bucket");
+  const u64 n_seg = (u64)n_terms * n_buckets;
+  if (n_seg > 0xFFFFFFFFull)  // the keys are u32 and the sentinel is n_seg itself
+    return h->fail(OI_ERR_INVALID_ARG, "n_terms x n_buckets = %llu: at most 2^32 - 1", (unsigned long long)n_seg);
+  for (uint32_t b = 0; b < n_buckets; ++b)
+    if (!(edges[b] < edges[b + 1]))
+      return h->fail(OI_ERR_INVALID_ARG, "edges[%u] = %lld, edges[%u] = %lld: the edges must increase strictly", b,
+                     (long long)edges[b], b + 1, (long long)edges[b + 1]);
+  if (source < -1 || source >= OI_N_SOURCES)
+    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
+  const uint32_t V = oi_bm25_n_terms(h);
+  for (uint32_t i = 0; i < n_terms; ++i)
+    if (terms[i] >= V) return h->fail(OI_ERR_INVALID_ARG, "terms[%u] = %u: the BM25 part has %u terms", i, terms[i], V);
+  MN_CK(cudaSetDevice(h->desc.device));
+  cudaStream_t st = h->stream;
+  MN_CK(call_begin(h, st));
+
+  // d_mention_io: terms u32 [n] | edges i64 [B + 1] | starts u64 [n + 1] | carries [n B] (when given) | states [n B] |
+  // summaries [n B] | scan temporaries
+  const size_t n = n_terms, nb = n_buckets;
+  size_t scan_tmp = 0;
+  MN_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)n + 1, st));
+  const size_t o_edges = align16(n * sizeof(uint32_t)), o_start = align16(o_edges + (nb + 1) * sizeof(int64_t));
+  const size_t o_carry = align16(o_start + (n + 1) * sizeof(u64));
+  const size_t o_state = align16(o_carry + (carry_in ? n_seg * sizeof(oi_mention_state) : 0));
+  const size_t o_sum = align16(o_state + n_seg * sizeof(oi_mention_state));
+  const size_t o_tmp = align16(o_sum + n_seg * sizeof(oi_social_summary));
+  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
+  unsigned char *io = h->d_mention_io;
+  uint32_t *d_terms = reinterpret_cast<uint32_t *>(io);
+  int64_t *d_edges = reinterpret_cast<int64_t *>(io + o_edges);
+  u64 *d_start = reinterpret_cast<u64 *>(io + o_start);
+  oi_mention_state *d_carry = carry_in ? reinterpret_cast<oi_mention_state *>(io + o_carry) : nullptr;
+  oi_mention_state *d_state = reinterpret_cast<oi_mention_state *>(io + o_state);
+  oi_social_summary *d_sum = reinterpret_cast<oi_social_summary *>(io + o_sum);
+  MN_CK(cudaMemcpyAsync(d_terms, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  MN_CK(cudaMemcpyAsync(d_edges, edges, (nb + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  if (carry_in) MN_CK(cudaMemcpyAsync(d_carry, carry_in, n_seg * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
+  timeline_lengths_kernel<<<grid_for(n + 1, h->num_sms), 256, 0, st>>>(term_off, d_terms, n_terms, d_start);
+  ++h->launches;
+  MN_CK(cudaGetLastError());
+  MN_CK(cub::DeviceScan::ExclusiveSum(io + o_tmp, scan_tmp, d_start, d_start, (int64_t)n + 1, st));
+  h->launches += 2;
+  u64 total = 0;
+  MN_CK(cudaMemcpyAsync(&total, d_start + n, sizeof(u64), cudaMemcpyDeviceToHost, st));
+  MN_CK(cudaStreamSynchronize(st));
+
+  // d_timeline_ws: keys u32 [P] x 2 | doc ids u32 [P] x 2 | segment offsets u64 [n B + 1] | sort temporaries
+  int end_bit = 0;
+  while (end_bit < 32 && (n_seg >> end_bit)) ++end_bit;  // the bits of the largest key, the sentinel n B
+  size_t sort_tmp = 0;
+  if (total) {
+    cub::DoubleBuffer<uint32_t> kb(nullptr, nullptr), vb(nullptr, nullptr);
+    MN_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+  }
+  const size_t o_seg = align16(4 * total * sizeof(uint32_t)), o_stmp = align16(o_seg + (n_seg + 1) * sizeof(u64));
+  MN_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, o_stmp + sort_tmp, st));
+  unsigned char *ws = h->d_timeline_ws;
+  uint32_t *d_keys = reinterpret_cast<uint32_t *>(ws);
+  u64 *d_seg = reinterpret_cast<u64 *>(ws + o_seg);
+  const uint32_t *sorted_keys = d_keys, *sorted_docs = nullptr;
+  if (total) {
+    timeline_keys_kernel<<<grid_for(total, h->num_sms), 256, 0, st>>>(term_off, oi_bm25_doc_ids(h), h->d_times, d_terms, d_start,
+                                                                      n_terms, total, d_edges, n_buckets, d_keys,
+                                                                      d_keys + 2 * total);
+    ++h->launches;
+    MN_CK(cudaGetLastError());
+    // stable: the input is in (term, doc) order, so every (term, bucket) segment stays in doc order
+    cub::DoubleBuffer<uint32_t> kb(d_keys, d_keys + total), vb(d_keys + 2 * total, d_keys + 3 * total);
+    MN_CK(cub::DeviceRadixSort::SortPairs(ws + o_stmp, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+    h->launches += 1 + (end_bit + 7) / 8;  // histogram + one pass per 8 bits
+    sorted_keys = kb.Current();
+    sorted_docs = vb.Current();
+  }
+  timeline_segments_kernel<<<grid_for(n_seg + 1, h->num_sms), 256, 0, st>>>(sorted_keys, total, n_seg, d_seg);
+  ++h->launches;
+  MN_CK(cudaGetLastError());
+  // a grid that stays resident walks the segments: most are tiny, so no CTA is launched for a single one of them
+  int per_sm = 0;
+  MN_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_timeline_kernel, 128, 0));
+  const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
+  mention_timeline_kernel<<<(unsigned)(n_seg < resident ? n_seg : resident), 128, 0, st>>>(
+      h->d_sig_pol, h->d_sig_flags, sorted_docs, d_seg, n_seg, source, bull_bear_threshold, d_carry, d_state, d_sum);
+  ++h->launches;
+  MN_CK(cudaGetLastError());
+  if (out_state) MN_CK(cudaMemcpyAsync(out_state, d_state, n_seg * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
+  MN_CK(cudaMemcpyAsync(out_summary, d_sum, n_seg * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
   MN_CK(call_end(h, st));
   MN_CK(cudaStreamSynchronize(st));
   return OI_OK;

@@ -74,6 +74,31 @@ def all_gather_packed(dist, blob, offsets, device="cpu"):
     return out_blob, np.concatenate([[0], np.cumsum(out_lens)]).astype(np.uint64)
 
 
+def _relay_states(dist, n, run, device="cpu"):
+    """The relay of n running states over the ranks in rank order (SPEC §8a): rank 0 runs `run(None)`, every later rank
+    receives the states of rank - 1 and runs `run(carry)`, and sends its states on; the last rank broadcasts its states
+    and summaries.  run(carry) -> (states: MENTION_STATE_DTYPE [n], summaries: SOCIAL_SUMMARY_DTYPE [n]).
+    -> the last rank's (states, summaries) on every rank."""
+    import torch
+    rank, world = dist.get_rank(), dist.get_world_size()
+    carry = None
+    if rank > 0:
+        buf = torch.empty(n * capi.MENTION_STATE_DTYPE.itemsize, dtype=torch.uint8, device=device)
+        dist.recv(buf, src=rank - 1)
+        carry = buf.cpu().numpy().view(capi.MENTION_STATE_DTYPE)
+    states, raw = run(carry)
+    states = np.ascontiguousarray(states).reshape(-1)
+    if rank < world - 1:
+        dist.send(torch.from_numpy(states.view(np.uint8).copy()).to(device), dst=rank + 1)
+    # the last rank's states and summaries, as bytes, to everybody
+    raw = np.ascontiguousarray(raw).reshape(-1) if rank == world - 1 else np.zeros(n, dtype=capi.SOCIAL_SUMMARY_DTYPE)
+    out = torch.from_numpy(np.concatenate([states.view(np.uint8), raw.view(np.uint8)])).to(device)
+    dist.broadcast(out, world - 1)
+    out = out.cpu().numpy()
+    cut = n * capi.MENTION_STATE_DTYPE.itemsize
+    return out[:cut].copy().view(capi.MENTION_STATE_DTYPE), out[cut:].copy().view(capi.SOCIAL_SUMMARY_DTYPE)
+
+
 def relay_mention_summary(dist, ix, term_ids, source=None, threshold=0.2, device="cpu"):
     """The social summaries of `term_ids` over the posting lists of a document-sharded index (SPEC §8a), the same on
     every rank: rank 0 summarises its shard and sends its running states to rank 1; every later rank receives them,
@@ -87,24 +112,29 @@ def relay_mention_summary(dist, ix, term_ids, source=None, threshold=0.2, device
     GpuIndex.mention_summary returns them."""
     if dist is None or dist.get_world_size() == 1 or len(term_ids) == 0:
         return ix.mention_summary(term_ids, source, threshold)
-    import torch
-    rank, world = dist.get_rank(), dist.get_world_size()
-    n = len(term_ids)
-    carry = None
-    if rank > 0:
-        buf = torch.empty(n * capi.MENTION_STATE_DTYPE.itemsize, dtype=torch.uint8, device=device)
-        dist.recv(buf, src=rank - 1)
-        carry = buf.cpu().numpy().view(capi.MENTION_STATE_DTYPE)
-    states, sums = ix.mention_summary(term_ids, source, threshold, carry)
-    if rank < world - 1:
-        dist.send(torch.from_numpy(states.view(np.uint8).copy()).to(device), dst=rank + 1)
-    # the last rank's states and summaries, as bytes, to everybody
-    raw = capi.summaries_to_array(sums) if rank == world - 1 else np.zeros(n, dtype=capi.SOCIAL_SUMMARY_DTYPE)
-    out = torch.from_numpy(np.concatenate([states.view(np.uint8), raw.view(np.uint8)])).to(device)
-    dist.broadcast(out, world - 1)
-    out = out.cpu().numpy()
-    cut = n * capi.MENTION_STATE_DTYPE.itemsize
-    return out[:cut].copy().view(capi.MENTION_STATE_DTYPE), capi.summaries_from_array(out[cut:].copy().view(capi.SOCIAL_SUMMARY_DTYPE))
+
+    def run(carry):
+        states, sums = ix.mention_summary(term_ids, source, threshold, carry)
+        return states, capi.summaries_to_array(sums)
+    states, raw = _relay_states(dist, len(term_ids), run, device)
+    return states, capi.summaries_from_array(raw)
+
+
+def relay_mention_timeline(dist, ix, term_ids, edges, source=None, threshold=0.2, device="cpu"):
+    """The per-(term, bucket) summaries of a document-sharded index (SPEC §8b), the same on every rank: the relay of
+    relay_mention_summary over the n x B running states of GpuIndex.mention_timeline.  Every rank passes the same term
+    ids and edges.  -> (states [n][B], summaries: n lists of B dicts) as GpuIndex.mention_timeline returns them."""
+    if dist is None or dist.get_world_size() == 1 or len(term_ids) == 0:
+        return ix.mention_timeline(term_ids, edges, source, threshold)
+    n, nb = len(term_ids), len(edges) - 1
+
+    def run(carry):
+        states, sums = ix.mention_timeline(term_ids, edges, source, threshold,
+                                           None if carry is None else carry.reshape(n, nb))
+        return states, capi.summaries_to_array([sm for row in sums for sm in row])
+    states, raw = _relay_states(dist, n * nb, run, device)
+    sums = capi.summaries_from_array(raw)
+    return states.reshape(n, nb), [sums[i * nb:(i + 1) * nb] for i in range(n)]
 
 
 def broadcast_unique_id(dist, device="cpu"):

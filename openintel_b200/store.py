@@ -20,6 +20,7 @@ the references the device builds are tested against.
 
 Scoring happens in libopenintel_gpu.so only; nothing here computes a score.
 """
+import datetime
 import sqlite3
 
 import numpy as np
@@ -68,6 +69,19 @@ def parse_post_text(raw):
     if len(t) > MAX_POST_LEN:
         raise InvalidPostText("exceeds max length")
     return t
+
+
+_EPOCH = datetime.datetime(1970, 1, 1, tzinfo=datetime.timezone.utc)
+
+
+def parse_created_at(text):
+    """A post's creation time (SPEC §8b): RFC 3339 with a UTC offset ('Z' or +-HH:MM) -> whole seconds since the Unix
+    epoch, fractional seconds floored.  A value without an offset is refused (ValueError): its instant is unknown."""
+    dt = datetime.datetime.fromisoformat(text)
+    if dt.utcoffset() is None:
+        raise ValueError("created_at %r has no UTC offset" % (text,))
+    d = dt - _EPOCH  # a timedelta keeps 0 <= seconds < 86400 and 0 <= microseconds: this is the floor
+    return d.days * 86400 + d.seconds
 
 
 def open_store(path=":memory:", dim=None):
@@ -435,7 +449,8 @@ class MentionIndex:
     Every rank lifts its doc range through lift_shard_gpu (unsharded when `dist` is None; the store needs no
     embeddings), scores its posts with the GPU PostAnalyzer and loads the signals and source codes next to the BM25
     part.  reports() returns on every rank exactly what analyze.analyze_posts returns for select_posts(source,
-    mention=ticker)."""
+    mention=ticker).  timeline() splits the same summaries by creation time (SPEC §8b); it reads the post times from
+    `conn` on its first call, so `conn` stays open while the index is used."""
 
     def __init__(self, conn, dist=None, device_index=0):
         self.dist = dist if (dist is not None and dist.get_world_size() > 1) else None
@@ -446,6 +461,7 @@ class MentionIndex:
         self.ix = sh["index"]
         self.term_id = {w: i for i, w in enumerate(sh["vocab"])}
         self.doc_base, self.n_local = sh["doc_base"], sh["n_local"]
+        self.conn, self.times_loaded = conn, False
         try:
             rows = conn.execute("SELECT source, text FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
                                 (self.doc_base, self.doc_base + self.n_local)).fetchall()
@@ -480,6 +496,59 @@ class MentionIndex:
                 out.append(analyze.build_report(sm, by_source, mk.get(k), cfg))
             except analyze.NoData:
                 out.append(None)
+        return out
+
+    def _load_times(self):
+        """parses this shard's created_at and loads it next to the BM25 part.  Sharded, the ranks agree first on whether
+        every rank parsed its rows, so a bad row on one rank raises on all of them instead of leaving the others waiting
+        in the relay."""
+        rows = self.conn.execute("SELECT doc_id, created_at FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
+                                 (self.doc_base, self.doc_base + self.n_local)).fetchall()
+        err, times = None, np.zeros(len(rows), dtype=np.int64)
+        for i, (doc_id, text) in enumerate(rows):
+            try:
+                times[i] = parse_created_at(text)
+            except ValueError as e:
+                err = "post doc_id %d: %s" % (doc_id, e)
+                break
+        if self.dist is not None:
+            import torch
+            bad = torch.tensor([0 if err is None else 1], dtype=torch.int64, device=self.device)
+            self.dist.all_reduce(bad, op=self.dist.ReduceOp.SUM)
+            if err is None and int(bad.item()):
+                err = "created_at of another shard's post is not RFC 3339 with a UTC offset"
+        if err is not None:
+            raise ValueError(err)
+        self.ix.load_post_times(times)
+        self.times_loaded = True
+
+    def timeline(self, tickers, edges, source=None, cfg=fusion.EngineConfig()):
+        """per ticker, in the order given, a list of len(edges) - 1 "social" blocks (analyze.social_block): block b
+        summarises the ticker's posts (of `source` only, when given) created in [edges[b], edges[b + 1]), seconds since
+        the Unix epoch -- what analyze_posts(select_posts(source, mention=ticker, since=edges[b], until=edges[b + 1]))
+        reports as "social".  Tickers are normalised like reports(); one outside the vocabulary gets empty blocks.  The
+        post times are read from the store and loaded on the first call; sharded, every rank calls with the same
+        arguments."""
+        from . import analyze, sharding
+        edges = [int(e) for e in edges]
+        if len(edges) < 2 or any(a >= b for a, b in zip(edges, edges[1:])):
+            raise ValueError("edges must be at least two strictly increasing times")
+        if not self.times_loaded:
+            self._load_times()
+        keys = [t.lstrip("$").lower() for t in tickers]
+        known = [k for k in dict.fromkeys(keys) if k in self.term_id]
+        states, sums = sharding.relay_mention_timeline(
+            self.dist, self.ix, np.array([self.term_id[k] for k in known], dtype=np.uint32), edges,
+            None if source is None else SOURCES.index(source), cfg.bull_bear_threshold, device=self.device)
+        found = {k: (st, sm) for k, st, sm in zip(known, states, sums)}
+        out = []
+        for k in keys:
+            if k not in found:
+                out.append([analyze.social_block(analyze.empty_summary(), {}) for _ in range(len(edges) - 1)])
+                continue
+            st, sm = found[k]
+            out.append([analyze.social_block(sm[b], {SOURCES[s]: int(st[b]["by_source"][s]) for s in range(len(SOURCES))})
+                        for b in range(len(edges) - 1)])
         return out
 
     def close(self):

@@ -137,6 +137,12 @@ extern "C" {
     pub fn oi_index_mention_summary(h: *mut oi_index, terms: *const u32, n_terms: u32, source: i32, bull_bear_threshold: f64,
                                     carry_in: *const oi_mention_state, out_state: *mut oi_mention_state,
                                     out_summary: *mut oi_social_summary) -> oi_status;
+    /// per-post creation times of this shard, seconds since the Unix epoch (docs/SPEC.md §8b)
+    pub fn oi_index_load_post_times(h: *mut oi_index, created_at: *const i64) -> oi_status;
+    /// per-(term, bucket) summaries, [n_terms][n_buckets] term-major; edges has n_buckets + 1 entries
+    pub fn oi_index_mention_timeline(h: *mut oi_index, terms: *const u32, n_terms: u32, edges: *const i64, n_buckets: u32,
+                                     source: i32, bull_bear_threshold: f64, carry_in: *const oi_mention_state,
+                                     out_state: *mut oi_mention_state, out_summary: *mut oi_social_summary) -> oi_status;
 
     pub fn oi_index_launch_count(h: *const oi_index) -> u64;
     pub fn oi_index_set_option(h: *mut oi_index, name: *const c_char, value: i64) -> oi_status;
