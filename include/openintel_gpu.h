@@ -265,6 +265,19 @@ oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *terms, uint32_t
                                     const oi_mention_state *carry_in, oi_mention_state *out_state,
                                     oi_social_summary *out_summary);
 
+/* ---- per-term mention counts by time bucket, over the whole vocabulary (docs/SPEC.md §8c) ---
+ * out_counts[t * n_buckets + b] = the number of this shard's posts that mention term t and were created in
+ * [edges[b], edges[b+1]), for every term t of the BM25 part (n_terms as oi_index_read_bm25 reports it), term-major, host
+ * memory.  A post that repeats the term counts once; source: -1 = all posts, else only that source's.  It equals the
+ * `total` of oi_index_mention_timeline's state for (t, b), without the sort and the summaries.  A document-sharded
+ * index sums the shards' counts (integers: the sum is exact in any order); a shard without a posting returns zeros.
+ * OI_ERR_STATE: no BM25 part, no signals or no times loaded.  OI_ERR_INVALID_ARG: NULL edges / out_counts,
+ * n_buckets == 0, edges not strictly increasing, source outside -1 .. OI_N_SOURCES - 1.  A refused call changes nothing.
+ * OI_ERR_OUT_OF_MEMORY: no room for the counts on the device.  Blocking; reads the posting lists only, so it works
+ * before and after oi_index_bm25_finalize. */
+oi_status oi_index_mention_counts(oi_index *h, const int64_t *edges, uint32_t n_buckets, int32_t source,
+                                  uint32_t *out_counts);
+
 /* ---- tuning / introspection (bench + tests) ------------------------------------------------ */
 /* number of kernels this handle has launched since creation (bench "gpu_launches") */
 uint64_t oi_index_launch_count(const oi_index *h);

@@ -106,6 +106,7 @@ def load_library():
         "oi_index_mention_summary": (st, [H, _u32p, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
         "oi_index_load_post_times": (st, [H, _vp]),
         "oi_index_mention_timeline": (st, [H, _u32p, C.c_uint32, _vp, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
+        "oi_index_mention_counts": (st, [H, _vp, C.c_uint32, C.c_int32, _u32p]),
         "oi_index_launch_count": (C.c_uint64, [H]),
         "oi_index_set_option": (st, [H, C.c_char_p, C.c_int64]),
         "oi_debug_cosine_gemm_scores": (st, [H, _f32p, C.c_uint32, _f32p]),
@@ -303,6 +304,16 @@ class GpuIndex:
         self._ck(self.L.oi_index_mention_timeline(self.h, _addr(terms), n, _addr(e), nb, -1 if source is None else int(source),
                                                    threshold, _addr(cin), _addr(states), _addr(sums)))
         return states, [summaries_from_array(row) for row in sums]
+
+    # -- per-term mention counts over the whole vocabulary (SPEC §8c)
+    def mention_counts(self, edges, source=None):
+        """the number of this shard's posts that mention each term of the BM25 part and were created in each bucket
+        [edges[b], edges[b + 1]) (oi_index_mention_counts).  -> uint32 [n_terms][B]"""
+        e = np.ascontiguousarray(edges, dtype=np.int64).reshape(-1)
+        nb = max(len(e) - 1, 0)
+        out = np.zeros((getattr(self, "n_terms", 0), nb), dtype=np.uint32)  # no BM25 part: the call refuses
+        self._ck(self.L.oi_index_mention_counts(self.h, _addr(e), nb, -1 if source is None else int(source), _addr(out)))
+        return out
 
     # -- multi-GPU
     @staticmethod

@@ -40,6 +40,7 @@
 #include "../../include/oi_synth_tables.h"
 #include "handle.h"
 #include "oi_common.cuh"
+#include "oi_postings.cuh"
 #include "oi_synth.cuh"
 
 #define OI_BM25_MAX_QTERMS 64
@@ -759,28 +760,7 @@ __global__ void __launch_bounds__(128) bm25_prep_queries_kernel(const uint32_t *
   if (lane == 0) out_nt[q] = n_kept;
 }
 
-// Term of posting p = the last t with term_off[t] <= p, searched inside [lo, hi) (invariant: term_off[lo] <= p <
-// term_off[hi]).  The per-posting kernels below walk the postings in warp tiles of 256: two full searches per tile (its
-// first and last posting) bound every other search to the few terms the tile spans -- none at all in the long lists.
-__device__ __forceinline__ uint32_t bm25_term_of(const u64 *__restrict__ term_off, uint32_t lo, uint32_t hi, u64 p) {
-  while (hi - lo > 1) {
-    const uint32_t mid = lo + ((hi - lo) >> 1);
-    if (__ldg(term_off + mid) <= p) lo = mid; else hi = mid;
-  }
-  return lo;
-}
-#define OI_BM25_TILE 256u
-struct TileTerms { uint32_t lo, hi; };
-__device__ __forceinline__ TileTerms bm25_tile_terms(const u64 *__restrict__ term_off, uint32_t n_terms, u64 tile, u64 n_postings, int lane) {
-  const u64 last = min(tile + OI_BM25_TILE - 1, n_postings - 1);
-  uint32_t b = 0;
-  if (lane == 0) b = bm25_term_of(term_off, 0, n_terms, tile);
-  if (lane == 31) b = bm25_term_of(term_off, 0, n_terms, last);
-  TileTerms t;
-  t.lo = __shfl_sync(0xFFFFFFFFu, b, 0);
-  t.hi = __shfl_sync(0xFFFFFFFFu, b, 31) + 1;
-  return t;
-}
+// the term of each posting: the warp-tile walk of oi_postings.cuh (bm25_tile_terms / bm25_term_of)
 
 // per-posting folded weight, SPEC §3 association, one IEEE op per line (file built with -fmad=false)
 __global__ void __launch_bounds__(256) bm25_weights_kernel(const u64 *term_off, const uint32_t *doc_ids, const uint32_t *tfs,
@@ -1059,6 +1039,7 @@ oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 
 }
 
 const u64 *oi_bm25_term_offsets(const oi_index *h) { return h->bm25 ? h->bm25->d_term_off : nullptr; }
+uint64_t oi_bm25_n_postings(const oi_index *h) { return h->bm25 ? h->bm25->n_postings : 0; }
 const uint32_t *oi_bm25_doc_ids(const oi_index *h) { return h->bm25 ? h->bm25->d_doc_ids : nullptr; }
 bool oi_bm25_finalized(const oi_index *h) { return h->bm25 && h->bm25->finalized; }
 

@@ -164,6 +164,7 @@ oi_status oi_bm25_adopt(oi_index *h, uint32_t n_terms, uint64_t n_postings, u64 
 uint32_t oi_bm25_n_terms(const oi_index *h);  // 0 = no BM25 part
 const u64 *oi_bm25_term_offsets(const oi_index *h);  // device term_offsets[n_terms + 1]; NULL = no BM25 part
 const uint32_t *oi_bm25_doc_ids(const oi_index *h);  // device doc_ids[n_postings] (kept after finalize); NULL = no BM25 part
+uint64_t oi_bm25_n_postings(const oi_index *h);  // 0 = no BM25 part or no posting
 bool oi_bm25_finalized(const oi_index *h);
 // re-indexes the BM25 part to n_terms terms over the same postings (text_index.cu's vocabulary union): d_term_off
 // [n_terms + 1] on the device becomes the index's, the old offsets are freed.  Before finalize only.

@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "handle.h"
+#include "oi_postings.cuh"
 #include "oi_summary.cuh"
 
 namespace {
@@ -56,7 +57,6 @@ __global__ void __launch_bounds__(256) timeline_keys_kernel(const u64 *term_off,
     for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_edges[k] = edges[k];
   __syncthreads();
   const int64_t *E = staged ? s_edges : edges;
-  const int64_t t_lo = E[0], t_hi = E[nb];
   for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
     uint32_t a = 0, b = n;  // the term: start[a] <= p < start[b] (an empty list shares its start with the next one)
     while (b - a > 1) {
@@ -64,17 +64,8 @@ __global__ void __launch_bounds__(256) timeline_keys_kernel(const u64 *term_off,
       if (start[m] <= p) a = m; else b = m;
     }
     const uint32_t doc = doc_ids[term_off[terms[a]] + (p - start[a])];
-    const int64_t t = times[doc];
-    u64 key = (u64)n * nb;
-    if (t >= t_lo && t < t_hi) {
-      uint32_t lo = 0, hi = nb;  // the bucket: E[lo] <= t < E[hi]
-      while (hi - lo > 1) {
-        const uint32_t m = (lo + hi) >> 1;
-        if (E[m] <= t) lo = m; else hi = m;
-      }
-      key = (u64)a * nb + lo;
-    }
-    keys[p] = (uint32_t)key;
+    const uint32_t bk = oi_time_bucket(E, nb, times[doc]);
+    keys[p] = (uint32_t)(bk < nb ? (u64)a * nb + bk : (u64)n * nb);
     vals[p] = doc;
   }
 }
@@ -100,6 +91,46 @@ __global__ void __launch_bounds__(128) mention_timeline_kernel(const double *pol
   for (u64 j = blockIdx.x; j < n_seg; j += gridDim.x)
     oi_social_summary_cta<true>(polarity, flags, docs, seg_off[j], seg_off[j + 1] - seg_off[j], source, thr,
                                 carry ? carry + j : nullptr, out_state + j, out + j);
+}
+
+// ---- mention counts (SPEC §8c)
+// One pass over all postings of the shard, load-balanced over the postings: each warp walks tiles of 256 postings
+// (oi_postings.cuh), finds each posting's term and its post's bucket, and counts it in counts[term * nb + bucket].  The
+// lanes of a warp that hit the same slot -- the common case inside a long list -- add their popcount with one atomic,
+// so a head term does not serialise on its few counters.  The doc ids are streamed; the times (and the flags with a
+// source filter) are gathered.  Integer counts: any schedule gives the same result.  The edges are staged in dynamic
+// shared memory when nb < kEdgesInSmem (the launch sizes it), else read from global memory.
+__global__ void __launch_bounds__(256) mention_counts_kernel(const u64 *__restrict__ term_off, const uint32_t *__restrict__ doc_ids,
+                                                             const int64_t *__restrict__ times, const uint8_t *__restrict__ flags,
+                                                             uint32_t n_terms, u64 n_postings, const int64_t *edges, uint32_t nb,
+                                                             int source, uint32_t *counts) {
+  extern __shared__ int64_t s_dyn_edges[];
+  const bool staged = nb < kEdgesInSmem;
+  if (staged)
+    for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_dyn_edges[k] = edges[k];
+  __syncthreads();
+  const int64_t *E = staged ? s_dyn_edges : edges;
+  const int lane = threadIdx.x & 31;
+  const u64 warp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((u64)gridDim.x * blockDim.x) >> 5;
+  for (u64 tile = warp * OI_BM25_TILE; tile < n_postings; tile += n_warps * OI_BM25_TILE) {
+    const TileTerms tt = bm25_tile_terms(term_off, n_terms, tile, n_postings, lane);
+    uint32_t lo = tt.lo;
+    for (uint32_t u = 0; u < OI_BM25_TILE / 32; ++u) {
+      if (tile + 32u * u >= n_postings) break;  // warp-uniform: the whole warp stays in for the match below
+      const u64 p = tile + 32u * u + (uint32_t)lane;
+      u64 slot = ~0ull;  // no slot: past the end, another source, or outside the edges
+      if (p < n_postings) {
+        lo = bm25_term_of(term_off, lo, tt.hi, p);
+        const uint32_t doc = __ldcs(doc_ids + p);
+        if (source < 0 || (flags[doc] >> 1) == source) {
+          const uint32_t bk = oi_time_bucket(E, nb, times[doc]);
+          if (bk < nb) slot = (u64)lo * nb + bk;
+        }
+      }
+      const uint32_t peers = __match_any_sync(0xFFFFFFFFu, slot);
+      if (slot != ~0ull && lane == __ffs(peers) - 1) atomicAdd(counts + slot, (uint32_t)__popc(peers));
+    }
+  }
 }
 
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
@@ -376,6 +407,55 @@ extern "C" oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *term
   MN_CK(cudaGetLastError());
   if (out_state) MN_CK(cudaMemcpyAsync(out_state, d_state, n_seg * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
   MN_CK(cudaMemcpyAsync(out_summary, d_sum, n_seg * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
+  MN_CK(call_end(h, st));
+  MN_CK(cudaStreamSynchronize(st));
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_mention_counts(oi_index *h, const int64_t *edges, uint32_t n_buckets, int32_t source,
+                                             uint32_t *out_counts) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  const u64 *term_off = oi_bm25_term_offsets(h);
+  if (!term_off) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
+  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
+  if (!h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
+  if (!edges || !out_counts) return h->fail(OI_ERR_INVALID_ARG, "NULL edges / out_counts");
+  if (n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "n_buckets = 0: counts need a bucket");
+  for (uint32_t b = 0; b < n_buckets; ++b)
+    if (!(edges[b] < edges[b + 1]))
+      return h->fail(OI_ERR_INVALID_ARG, "edges[%u] = %lld, edges[%u] = %lld: the edges must increase strictly", b,
+                     (long long)edges[b], b + 1, (long long)edges[b + 1]);
+  if (source < -1 || source >= OI_N_SOURCES)
+    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
+  const uint32_t V = oi_bm25_n_terms(h);
+  const u64 n_seg = (u64)V * n_buckets, nb1 = (u64)n_buckets + 1;
+  if (n_seg == 0) return OI_OK;
+  // d_mention_io: edges i64 [B + 1] | counts u32 [V B]; the byte count cannot wrap below 2^64
+  if (n_seg > (~(u64)0 - 64 - nb1 * sizeof(int64_t)) / sizeof(uint32_t))
+    return h->fail(OI_ERR_OUT_OF_MEMORY, "%u terms x %u buckets of counts do not fit the address space", V, n_buckets);
+  MN_CK(cudaSetDevice(h->desc.device));
+  cudaStream_t st = h->stream;
+  MN_CK(call_begin(h, st));
+  const size_t o_counts = align16(nb1 * sizeof(int64_t)), bytes = n_seg * sizeof(uint32_t);
+  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_counts + bytes, st));
+  int64_t *d_edges = reinterpret_cast<int64_t *>(h->d_mention_io);
+  uint32_t *d_counts = reinterpret_cast<uint32_t *>(h->d_mention_io + o_counts);
+  MN_CK(cudaMemsetAsync(d_counts, 0, bytes, st));
+  const u64 P = oi_bm25_n_postings(h);
+  if (P) {  // a shard without a posting (the token-free shard of a sharded lift) counts nothing
+    MN_CK(cudaMemcpyAsync(d_edges, edges, nb1 * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    const size_t smem = n_buckets < kEdgesInSmem ? nb1 * sizeof(int64_t) : 0;
+    int per_sm = 0;
+    MN_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_counts_kernel, 256, smem));
+    const u64 tiles = (P + OI_BM25_TILE - 1) / OI_BM25_TILE, want = (tiles + 7) / 8;  // 8 warps per CTA
+    const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
+    mention_counts_kernel<<<(unsigned)(want < resident ? want : resident), 256, smem, st>>>(
+        term_off, oi_bm25_doc_ids(h), h->d_times, h->d_sig_flags, V, P, d_edges, n_buckets, source, d_counts);
+    ++h->launches;
+    MN_CK(cudaGetLastError());
+  }
+  MN_CK(cudaMemcpyAsync(out_counts, d_counts, bytes, cudaMemcpyDeviceToHost, st));
   MN_CK(call_end(h, st));
   MN_CK(cudaStreamSynchronize(st));
   return OI_OK;

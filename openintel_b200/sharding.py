@@ -137,6 +137,20 @@ def relay_mention_timeline(dist, ix, term_ids, edges, source=None, threshold=0.2
     return states.reshape(n, nb), [sums[i * nb:(i + 1) * nb] for i in range(n)]
 
 
+def all_reduce_counts(dist, counts, device="cpu"):
+    """The global mention counts of a document-sharded index (SPEC §8c): the sum of the shards' counts, the same on
+    every rank.  Integers, so an all-reduce is exact in any order and no relay is needed; the shards' arrays line up
+    because the vocabulary is the global union (SPEC §5).  `dist` = torch.distributed (initialised) or None for a single
+    shard.  -> int64 array shaped like `counts`"""
+    out = np.asarray(counts).astype(np.int64)
+    if dist is None or dist.get_world_size() == 1:
+        return out
+    import torch
+    t = torch.from_numpy(out).to(device)
+    dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    return t.cpu().numpy()
+
+
 def broadcast_unique_id(dist, device="cpu"):
     """rank 0 creates the NCCL unique id (C ABI), everybody receives it."""
     import torch

@@ -449,8 +449,9 @@ class MentionIndex:
     Every rank lifts its doc range through lift_shard_gpu (unsharded when `dist` is None; the store needs no
     embeddings), scores its posts with the GPU PostAnalyzer and loads the signals and source codes next to the BM25
     part.  reports() returns on every rank exactly what analyze.analyze_posts returns for select_posts(source,
-    mention=ticker).  timeline() splits the same summaries by creation time (SPEC §8b); it reads the post times from
-    `conn` on its first call, so `conn` stays open while the index is used."""
+    mention=ticker).  timeline() splits the same summaries by creation time (SPEC §8b); mention_counts() counts every
+    term's mentions by creation time and trending() ranks the terms by the surge of their counts (SPEC §8c).  These read
+    the post times from `conn` on their first call, so `conn` stays open while the index is used."""
 
     def __init__(self, conn, dist=None, device_index=0):
         self.dist = dist if (dist is not None and dist.get_world_size() > 1) else None
@@ -459,7 +460,8 @@ class MentionIndex:
         sh = lift_shard_gpu(conn, self.dist, device=self.device, device_index=device_index, max_k=1, max_batch=1,
                             with_embeddings=False)
         self.ix = sh["index"]
-        self.term_id = {w: i for i, w in enumerate(sh["vocab"])}
+        self.vocab = sh["vocab"]
+        self.term_id = {w: i for i, w in enumerate(self.vocab)}
         self.doc_base, self.n_local = sh["doc_base"], sh["n_local"]
         self.conn, self.times_loaded = conn, False
         try:
@@ -549,6 +551,52 @@ class MentionIndex:
             st, sm = found[k]
             out.append([analyze.social_block(sm[b], {SOURCES[s]: int(st[b]["by_source"][s]) for s in range(len(SOURCES))})
                         for b in range(len(edges) - 1)])
+        return out
+
+    def mention_counts(self, edges, source=None):
+        """count[t][b] = the number of posts (of `source` only, when given) that mention term t of the vocabulary and
+        were created in [edges[b], edges[b + 1]), seconds since the Unix epoch (SPEC §8c): one device call per shard over
+        all terms, and an all-reduce of the shards' counts.  The post times are read from the store and loaded on the
+        first call; sharded, every rank calls with the same arguments.  -> int64 [len(vocab)][len(edges) - 1], the same
+        on every rank"""
+        from . import sharding
+        edges = [int(e) for e in edges]
+        if len(edges) < 2 or any(a >= b for a, b in zip(edges, edges[1:])):
+            raise ValueError("edges must be at least two strictly increasing times")
+        if not self.times_loaded:
+            self._load_times()
+        counts = self.ix.mention_counts(edges, None if source is None else SOURCES.index(source))
+        return sharding.all_reduce_counts(self.dist, counts, device=self.device)
+
+    def trending(self, since, until, baseline_since, k, min_mentions=1, source=None, universe=None, cfg=fusion.EngineConfig()):
+        """the terms whose mentions in the window [since, until) rise most above what the baseline [baseline_since, since)
+        predicts, ranked by SPEC §8c (trending.rank): at most k entries {ticker, mentions, baseline_mentions, expected,
+        surge, social: {baseline, window}}, where the social blocks are those of timeline() over the two windows.  Only
+        terms with at least min_mentions mentions in the window are ranked; `universe` (tickers, normalised like
+        reports()) restricts the ranking to its entries, and one outside the vocabulary is never ranked.  Times are
+        seconds since the Unix epoch; sharded, every rank calls with the same arguments and gets the same list."""
+        from . import analyze, sharding, trending
+        t0, t1, t2 = int(baseline_since), int(since), int(until)
+        if not t0 < t1 < t2:
+            raise ValueError("the times must satisfy baseline_since < since < until")
+        if int(k) < 1 or int(min_mentions) < 1:
+            raise ValueError("k and min_mentions must be at least 1")
+        counts = self.mention_counts([t0, t1, t2], source)
+        mask = None
+        if universe is not None:
+            mask = np.zeros(len(self.vocab), dtype=bool)
+            mask[[self.term_id[w] for w in (u.lstrip("$").lower() for u in universe) if w in self.term_id]] = True
+        ids, expected, surge = trending.rank(counts[:, 1], counts[:, 0], t0, t1, t2, k, min_mentions, mask)
+        states, sums = sharding.relay_mention_timeline(self.dist, self.ix, ids.astype(np.uint32), [t0, t1, t2],
+                                                       None if source is None else SOURCES.index(source),
+                                                       cfg.bull_bear_threshold, device=self.device)
+        out = []
+        for i, t in enumerate(ids):
+            blocks = [analyze.social_block(sums[i][b], {SOURCES[s]: int(states[i][b]["by_source"][s]) for s in range(len(SOURCES))})
+                      for b in range(2)]
+            out.append({"ticker": self.vocab[t], "mentions": int(counts[t, 1]), "baseline_mentions": int(counts[t, 0]),
+                        "expected": float(expected[i]), "surge": float(surge[i]),
+                        "social": {"baseline": blocks[0], "window": blocks[1]}})
         return out
 
     def close(self):

@@ -143,6 +143,10 @@ extern "C" {
     pub fn oi_index_mention_timeline(h: *mut oi_index, terms: *const u32, n_terms: u32, edges: *const i64, n_buckets: u32,
                                      source: i32, bull_bear_threshold: f64, carry_in: *const oi_mention_state,
                                      out_state: *mut oi_mention_state, out_summary: *mut oi_social_summary) -> oi_status;
+    /// per-(term, bucket) mention counts over every term of the BM25 part, [n_terms][n_buckets] term-major
+    /// (docs/SPEC.md §8c); edges has n_buckets + 1 entries
+    pub fn oi_index_mention_counts(h: *mut oi_index, edges: *const i64, n_buckets: u32, source: i32,
+                                   out_counts: *mut u32) -> oi_status;
 
     pub fn oi_index_launch_count(h: *const oi_index) -> u64;
     pub fn oi_index_set_option(h: *mut oi_index, name: *const c_char, value: i64) -> oi_status;
