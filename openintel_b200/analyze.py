@@ -23,9 +23,15 @@ class NoData(ValueError):
     """DomainError::NoData (src/application/analyze.rs:58-60): neither posts nor a market snapshot"""
 
 
+def ticker_key(text):
+    """a ticker or mention word as the index holds it: the leading '$' dropped (the reference's tokenizer drops it
+    too), lower case"""
+    return text.lstrip("$").lower()
+
+
 def select_posts(conn, source=None, mention=None, limit=None, since=None, until=None):
     """(ids, sources, texts) of the stored posts in doc order; `mention`: keep posts one of whose tokens equals it
-    (case-insensitive, a leading '$' ignored: the reference's tokenizer drops it too); `since` / `until`: keep posts
+    (normalised by ticker_key); `since` / `until`: keep posts
     created in [since, until), seconds since the Unix epoch (store.parse_created_at; SPEC §8b), before `limit`"""
     window = since is not None or until is not None
     sql, args = "SELECT id, source, text%s FROM posts" % (", doc_id, created_at" if window else ""), []
@@ -47,7 +53,7 @@ def select_posts(conn, source=None, mention=None, limit=None, since=None, until=
         rows = kept
     if mention:
         from . import hostlib
-        want = mention.lstrip("$").lower()
+        want = ticker_key(mention)
         rows = [r for r in rows if want in hostlib.tokenize(r[2])]
     if limit is not None:
         rows = rows[:limit]

@@ -42,6 +42,11 @@ class SocialSummary(C.Structure):
 N_SOURCES = 2  # OI_N_SOURCES: post sources in store-schema order (store.SOURCES)
 
 
+def _source_code(source):
+    """a mention call's source argument: -1 for all posts (None), else the source code"""
+    return -1 if source is None else int(source)
+
+
 # oi_mention_state as a numpy structured type: the running state of one term's summary after a prefix of the doc order
 # (SPEC §8a)
 MENTION_STATE_DTYPE = np.dtype([("total", "<u8"), ("bullish", "<u8"), ("bearish", "<u8"), ("neutral", "<u8"),
@@ -267,17 +272,24 @@ class GpuIndex:
         `carry` (the states of the previous shard, or None).  source: None = all posts, else a source code.
         -> (states: MENTION_STATE_DTYPE array, summaries: list of dicts shaped like GpuLexicon's summary)"""
         terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
-        n = len(terms)
-        states = np.zeros(n, dtype=MENTION_STATE_DTYPE)
-        sums = np.zeros(n, dtype=SOCIAL_SUMMARY_DTYPE)
+        states, sums, cin = self._mention_outputs((len(terms),), carry)
+        self._ck(self.L.oi_index_mention_summary(self.h, _addr(terms), len(terms), _source_code(source), threshold,
+                                                  _addr(cin), _addr(states), _addr(sums)))
+        return states, summaries_from_array(sums)
+
+    @staticmethod
+    def _mention_outputs(shape, carry):
+        """zeroed states and summaries of a mention call, shaped (terms,) or (terms, buckets), and the carried states
+        checked against that shape (None when not given)"""
+        states = np.zeros(shape, dtype=MENTION_STATE_DTYPE)
+        sums = np.zeros(shape, dtype=SOCIAL_SUMMARY_DTYPE)
         cin = None
         if carry is not None:
             cin = np.ascontiguousarray(carry, dtype=MENTION_STATE_DTYPE)
-            if len(cin) != n:
-                raise ValueError("%d carried states for %d terms" % (len(cin), n))
-        self._ck(self.L.oi_index_mention_summary(self.h, _addr(terms), n, -1 if source is None else int(source), threshold,
-                                                  _addr(cin), _addr(states), _addr(sums)))
-        return states, summaries_from_array(sums)
+            if cin.size != states.size:
+                what = ("%d terms x %d buckets" if len(shape) == 2 else "%d terms") % shape
+                raise ValueError("%d carried states for %s" % (cin.size, what))
+        return states, sums, cin
 
     # -- per-term timelines (SPEC §8b)
     def load_post_times(self, seconds):
@@ -294,15 +306,9 @@ class GpuIndex:
         terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
         e = np.ascontiguousarray(edges, dtype=np.int64).reshape(-1)
         n, nb = len(terms), max(len(e) - 1, 0)
-        states = np.zeros((n, nb), dtype=MENTION_STATE_DTYPE)
-        sums = np.zeros((n, nb), dtype=SOCIAL_SUMMARY_DTYPE)
-        cin = None
-        if carry is not None:
-            cin = np.ascontiguousarray(carry, dtype=MENTION_STATE_DTYPE)
-            if cin.size != n * nb:
-                raise ValueError("%d carried states for %d terms x %d buckets" % (cin.size, n, nb))
-        self._ck(self.L.oi_index_mention_timeline(self.h, _addr(terms), n, _addr(e), nb, -1 if source is None else int(source),
-                                                   threshold, _addr(cin), _addr(states), _addr(sums)))
+        states, sums, cin = self._mention_outputs((n, nb), carry)
+        self._ck(self.L.oi_index_mention_timeline(self.h, _addr(terms), n, _addr(e), nb, _source_code(source), threshold,
+                                                   _addr(cin), _addr(states), _addr(sums)))
         return states, [summaries_from_array(row) for row in sums]
 
     # -- per-term mention counts over the whole vocabulary (SPEC §8c)
@@ -312,7 +318,7 @@ class GpuIndex:
         e = np.ascontiguousarray(edges, dtype=np.int64).reshape(-1)
         nb = max(len(e) - 1, 0)
         out = np.zeros((getattr(self, "n_terms", 0), nb), dtype=np.uint32)  # no BM25 part: the call refuses
-        self._ck(self.L.oi_index_mention_counts(self.h, _addr(e), nb, -1 if source is None else int(source), _addr(out)))
+        self._ck(self.L.oi_index_mention_counts(self.h, _addr(e), nb, _source_code(source), _addr(out)))
         return out
 
     # -- multi-GPU

@@ -21,14 +21,6 @@ oi_status oi_index::fail(oi_status code, const char *fmt, ...) {
   return code;
 }
 
-#define OI_CK(call)                                                                              \
-  do {                                                                                           \
-    cudaError_t e_ = (call);                                                                     \
-    if (e_ != cudaSuccess)                                                                       \
-      return h->fail(e_ == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA,       \
-                     "%s failed: %s", #call, cudaGetErrorString(e_));                            \
-  } while (0)
-
 #define OI_REQUIRE(cond, ...)                                   \
   do {                                                          \
     if (!(cond)) return h->fail(OI_ERR_INVALID_ARG, __VA_ARGS__); \

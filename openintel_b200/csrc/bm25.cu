@@ -910,22 +910,7 @@ __global__ void csr_from_sorted_kernel(const u64 *keys, u64 n, uint32_t n_terms,
   }
 }
 
-unsigned grid_for(u64 n, int threads, int num_sms) {
-  u64 b = (n + threads - 1) / threads;
-  const u64 cap = (u64)num_sms * 16;
-  if (b > cap) b = cap;
-  return (unsigned)(b ? b : 1);
-}
-
 }  // namespace
-
-#define BM_CK(call)                                                                              \
-  do {                                                                                           \
-    cudaError_t e_ = (call);                                                                     \
-    if (e_ != cudaSuccess)                                                                       \
-      return h->fail(e_ == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA,       \
-                     "%s failed: %s", #call, cudaGetErrorString(e_));                            \
-  } while (0)
 
 void oi_bm25_free(oi_index *h) {
   cudaFree(h->d_vocab); cudaFree(h->d_vocab_off);
@@ -950,16 +935,16 @@ static size_t bm25_lists_cap(const oi_index *h) {
 
 static oi_status bm25_alloc_workspace(oi_index *h, OiBm25 *b) {
   const size_t B = h->desc.max_batch;
-  BM_CK(cudaMalloc(&b->d_qterms, B * OI_BM25_MAX_QTERMS * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_qnt, B * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_gthr, B * sizeof(u64)));
-  BM_CK(cudaMalloc(&b->d_counter, sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_qterms, B * OI_BM25_MAX_QTERMS * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_qnt, B * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_gthr, B * sizeof(u64)));
+  OI_CK(cudaMalloc(&b->d_counter, sizeof(uint32_t)));
   b->lists_cap = bm25_lists_cap(h);
-  BM_CK(cudaMalloc(&b->d_lists, b->lists_cap * sizeof(u64)));
-  BM_CK(cudaMalloc(&b->d_best, B * (size_t)h->desc.max_k * sizeof(u64)));
-  BM_CK(cudaMalloc(&b->d_qlock, B * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_in_terms, B * OI_BM25_MAX_QTERMS * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_in_offs, (B + 1) * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_lists, b->lists_cap * sizeof(u64)));
+  OI_CK(cudaMalloc(&b->d_best, B * (size_t)h->desc.max_k * sizeof(u64)));
+  OI_CK(cudaMalloc(&b->d_qlock, B * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_in_terms, B * OI_BM25_MAX_QTERMS * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_in_offs, (B + 1) * sizeof(uint32_t)));
   return OI_OK;
 }
 
@@ -973,41 +958,41 @@ extern "C" oi_status oi_index_load_bm25(oi_index *h, const uint64_t *term_offset
   if (term_offsets[0] != 0) return h->fail(OI_ERR_INVALID_ARG, "term_offsets[0] must be 0");
   for (uint32_t t = 0; t < n_terms; ++t)
     if (term_offsets[t + 1] < term_offsets[t]) return h->fail(OI_ERR_INVALID_ARG, "term_offsets not monotone at term %u", t);
-  BM_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   oi_bm25_free(h);
   OiBm25 *b = new OiBm25();
   h->bm25 = b;
   b->n_terms = n_terms;
   b->n_postings = P;
   const size_t Pa = P ? P : 1;
-  BM_CK(cudaMalloc(&b->d_term_off, ((size_t)n_terms + 1) * sizeof(u64)));
-  BM_CK(cudaMalloc(&b->d_doc_ids, Pa * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_tfs, Pa * sizeof(uint32_t)));
-  BM_CK(cudaMalloc(&b->d_w, Pa * sizeof(float)));
-  BM_CK(cudaMalloc(&b->d_doc_len, (h->desc.n_docs ? h->desc.n_docs : 1) * sizeof(uint32_t)));
-  BM_CK(cudaMemcpyAsync(b->d_term_off, term_offsets, ((size_t)n_terms + 1) * sizeof(u64), cudaMemcpyHostToDevice, h->stream));
+  OI_CK(cudaMalloc(&b->d_term_off, ((size_t)n_terms + 1) * sizeof(u64)));
+  OI_CK(cudaMalloc(&b->d_doc_ids, Pa * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_tfs, Pa * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&b->d_w, Pa * sizeof(float)));
+  OI_CK(cudaMalloc(&b->d_doc_len, (h->desc.n_docs ? h->desc.n_docs : 1) * sizeof(uint32_t)));
+  OI_CK(cudaMemcpyAsync(b->d_term_off, term_offsets, ((size_t)n_terms + 1) * sizeof(u64), cudaMemcpyHostToDevice, h->stream));
   if (P) {
-    BM_CK(cudaMemcpyAsync(b->d_doc_ids, doc_ids, P * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
-    BM_CK(cudaMemcpyAsync(b->d_tfs, tfs, P * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    OI_CK(cudaMemcpyAsync(b->d_doc_ids, doc_ids, P * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    OI_CK(cudaMemcpyAsync(b->d_tfs, tfs, P * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
   }
-  if (h->desc.n_docs) BM_CK(cudaMemcpyAsync(b->d_doc_len, doc_len, h->desc.n_docs * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  if (h->desc.n_docs) OI_CK(cudaMemcpyAsync(b->d_doc_len, doc_len, h->desc.n_docs * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
   // the postings are validated where they now are (one pass at HBM speed instead of an O(P) host loop)
   u64 bad = ~0ull;
   if (P) {
     u64 *d_err = nullptr;
-    BM_CK(cudaMalloc(&d_err, sizeof(u64)));
+    OI_CK(cudaMalloc(&d_err, sizeof(u64)));
     cudaError_t e = cudaMemsetAsync(d_err, 0xFF, sizeof(u64), h->stream);
     if (e == cudaSuccess) {
-      bm25_validate_kernel<<<grid_for(P / 8 + 1, 256, h->num_sms), 256, 0, h->stream>>>(b->d_term_off, b->d_doc_ids, n_terms, P, (uint32_t)h->desc.n_docs, d_err);
+      bm25_validate_kernel<<<oi_grid(P / 8 + 1, 256, h->num_sms), 256, 0, h->stream>>>(b->d_term_off, b->d_doc_ids, n_terms, P, (uint32_t)h->desc.n_docs, d_err);
       ++h->launches;
       e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(&bad, d_err, sizeof(u64), cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     cudaFree(d_err);
-    BM_CK(e);
+    OI_CK(e);
   } else {
-    BM_CK(cudaStreamSynchronize(h->stream));
+    OI_CK(cudaStreamSynchronize(h->stream));
   }
   if (bad != ~0ull) {
     const uint64_t pb = bad >> 1;
@@ -1054,7 +1039,7 @@ extern "C" oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vo
   if (!h) return OI_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lock(h->mu);
   if (!zipf_cdf || vocab == 0) return h->fail(OI_ERR_INVALID_ARG, "zipf_cdf is NULL or vocab == 0");
-  BM_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   oi_bm25_free(h);
   OiBm25 *b = new OiBm25();
   h->bm25 = b;
@@ -1081,8 +1066,8 @@ extern "C" oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vo
   SY_CK(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(u64), st));
   u64 h_cnt[2] = {0, 0};
   if (n) {
-    synth_doc_len_kernel<<<grid_for(n, 256, h->num_sms), 256, 0, st>>>(seed, h->desc.doc_base, n, b->d_doc_len);
-    sum_u32_kernel<<<grid_for(n, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, n, d_cnt);
+    synth_doc_len_kernel<<<oi_grid(n, 256, h->num_sms), 256, 0, st>>>(seed, h->desc.doc_base, n, b->d_doc_len);
+    sum_u32_kernel<<<oi_grid(n, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, n, d_cnt);
     h->launches += 2;
     SY_CK(cudaGetLastError());
     SY_CK(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(u64), cudaMemcpyDeviceToHost, st));
@@ -1125,7 +1110,7 @@ extern "C" oi_status oi_index_synth_bm25(oi_index *h, uint64_t seed, uint32_t vo
   SY_CK(cudaMalloc(&b->d_doc_ids, Pa * sizeof(uint32_t)));
   SY_CK(cudaMalloc(&b->d_tfs, Pa * sizeof(uint32_t)));
   SY_CK(cudaMalloc(&b->d_w, Pa * sizeof(float)));
-  csr_from_sorted_kernel<<<grid_for(P + 1, 256, h->num_sms), 256, 0, st>>>(sorted_keys, P, vocab, b->d_term_off, b->d_doc_ids);
+  csr_from_sorted_kernel<<<oi_grid(P + 1, 256, h->num_sms), 256, 0, st>>>(sorted_keys, P, vocab, b->d_term_off, b->d_doc_ids);
   ++h->launches;
   SY_CK(cudaGetLastError());
   if (P) SY_CK(cudaMemcpyAsync(b->d_tfs, sorted_vals, P * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
@@ -1140,32 +1125,32 @@ extern "C" oi_status oi_index_bm25_local_stats(oi_index *h, uint32_t *df_out, ui
   std::lock_guard<std::mutex> lock(h->mu);
   OiBm25 *b = h->bm25;
   if (!b) return h->fail(OI_ERR_STATE, "no BM25 index loaded");
-  BM_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
   if (n_postings) *n_postings = b->n_postings;
   if (df_out) {
     uint32_t *d_df = nullptr;
-    BM_CK(cudaMalloc(&d_df, (size_t)b->n_terms * sizeof(uint32_t)));
+    OI_CK(cudaMalloc(&d_df, (size_t)b->n_terms * sizeof(uint32_t)));
     df_from_offsets_kernel<<<(b->n_terms + 255) / 256, 256, 0, st>>>(b->d_term_off, b->n_terms, d_df);
     ++h->launches;
     cudaError_t e = cudaMemcpyAsync(df_out, d_df, (size_t)b->n_terms * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     cudaFree(d_df);
-    BM_CK(e);
+    OI_CK(e);
   }
   if (sum_doc_len) {
     u64 *d_s = nullptr;
-    BM_CK(cudaMalloc(&d_s, sizeof(u64)));
+    OI_CK(cudaMalloc(&d_s, sizeof(u64)));
     cudaError_t e = cudaMemsetAsync(d_s, 0, sizeof(u64), st);
     if (e == cudaSuccess && h->desc.n_docs) {
-      sum_u32_kernel<<<grid_for(h->desc.n_docs, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, h->desc.n_docs, d_s);
+      sum_u32_kernel<<<oi_grid(h->desc.n_docs, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, h->desc.n_docs, d_s);
       ++h->launches;
       e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(sum_doc_len, d_s, sizeof(u64), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     cudaFree(d_s);
-    BM_CK(e);
+    OI_CK(e);
   }
   return OI_OK;
 }
@@ -1177,15 +1162,15 @@ extern "C" oi_status oi_index_bm25_finalize(oi_index *h, const oi_bm25_params *p
   if (!b) return h->fail(OI_ERR_STATE, "no BM25 index loaded");
   if (!params || params->struct_size != sizeof(oi_bm25_params)) return h->fail(OI_ERR_INVALID_ARG, "bad oi_bm25_params (struct_size mismatch)");
   if (!(params->k1 >= 0.0f) || !(params->b >= 0.0f && params->b <= 1.0f)) return h->fail(OI_ERR_INVALID_ARG, "k1 must be >= 0 and b in [0, 1]");
-  BM_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
   // df: global if given, else this shard's list lengths
   std::vector<uint32_t> df(b->n_terms);
   // one copy of the offsets (8 B per term) serves both the local df and the choice of the dense columns; the O(P)
   // work -- weights, interleaved postings, dense columns, column maxima -- stays on the device
   std::vector<u64> off((size_t)b->n_terms + 1);
-  BM_CK(cudaMemcpyAsync(off.data(), b->d_term_off, off.size() * sizeof(u64), cudaMemcpyDeviceToHost, st));
-  BM_CK(cudaStreamSynchronize(st));
+  OI_CK(cudaMemcpyAsync(off.data(), b->d_term_off, off.size() * sizeof(u64), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
   if (params->global_df) {
     std::copy(params->global_df, params->global_df + b->n_terms, df.begin());
   } else {
@@ -1195,17 +1180,17 @@ extern "C" oi_status oi_index_bm25_finalize(oi_index *h, const oi_bm25_params *p
   float avgdl = params->avgdl;
   if (!(avgdl > 0.0f)) {
     u64 *d_s = nullptr, sum = 0;
-    BM_CK(cudaMalloc(&d_s, sizeof(u64)));
+    OI_CK(cudaMalloc(&d_s, sizeof(u64)));
     cudaError_t e = cudaMemsetAsync(d_s, 0, sizeof(u64), st);
     if (e == cudaSuccess && h->desc.n_docs) {
-      sum_u32_kernel<<<grid_for(h->desc.n_docs, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, h->desc.n_docs, d_s);
+      sum_u32_kernel<<<oi_grid(h->desc.n_docs, 256, h->num_sms), 256, 0, st>>>(b->d_doc_len, h->desc.n_docs, d_s);
       ++h->launches;
       e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(&sum, d_s, sizeof(u64), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     cudaFree(d_s);
-    BM_CK(e);
+    OI_CK(e);
     avgdl = h->desc.n_docs ? (float)((double)sum / (double)h->desc.n_docs) : 1.0f;
   }
   // idf: double on the host, rounded once (SPEC §3)
@@ -1234,19 +1219,19 @@ extern "C" oi_status oi_index_bm25_finalize(oi_index *h, const oi_bm25_params *p
   cudaFree(b->d_post); cudaFree(b->d_dense); cudaFree(b->d_dense_slot); cudaFree(b->d_dense_max);
   b->d_post = nullptr; b->d_dense = nullptr; b->d_dense_slot = nullptr; b->d_dense_max = nullptr;
   const size_t dense_elems = (size_t)std::max<uint32_t>(b->n_dense, 1) * b->dense_stride;
-  BM_CK(cudaMalloc(&b->d_post, ((size_t)b->n_postings + OI_BM25_POST_PAD) * sizeof(uint2)));
-  BM_CK(cudaMalloc(&b->d_dense, std::max<size_t>(dense_elems, 4) * sizeof(float)));
-  BM_CK(cudaMalloc(&b->d_dense_slot, (size_t)b->n_terms * sizeof(int)));
-  BM_CK(cudaMemsetAsync(b->d_post, 0xFF, ((size_t)b->n_postings + OI_BM25_POST_PAD) * sizeof(uint2), st));
-  BM_CK(cudaMemsetAsync(b->d_dense, 0, std::max<size_t>(dense_elems, 4) * sizeof(float), st));
-  BM_CK(cudaMemcpyAsync(b->d_dense_slot, slot.data(), slot.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-  BM_CK(cudaMalloc(&b->d_dense_max, OI_BM25_MAX_DENSE * sizeof(float)));
-  BM_CK(cudaMemsetAsync(b->d_dense_max, 0, OI_BM25_MAX_DENSE * sizeof(float), st));
+  OI_CK(cudaMalloc(&b->d_post, ((size_t)b->n_postings + OI_BM25_POST_PAD) * sizeof(uint2)));
+  OI_CK(cudaMalloc(&b->d_dense, std::max<size_t>(dense_elems, 4) * sizeof(float)));
+  OI_CK(cudaMalloc(&b->d_dense_slot, (size_t)b->n_terms * sizeof(int)));
+  OI_CK(cudaMemsetAsync(b->d_post, 0xFF, ((size_t)b->n_postings + OI_BM25_POST_PAD) * sizeof(uint2), st));
+  OI_CK(cudaMemsetAsync(b->d_dense, 0, std::max<size_t>(dense_elems, 4) * sizeof(float), st));
+  OI_CK(cudaMemcpyAsync(b->d_dense_slot, slot.data(), slot.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  OI_CK(cudaMalloc(&b->d_dense_max, OI_BM25_MAX_DENSE * sizeof(float)));
+  OI_CK(cudaMemsetAsync(b->d_dense_max, 0, OI_BM25_MAX_DENSE * sizeof(float), st));
   float *d_idf = nullptr;
-  BM_CK(cudaMalloc(&d_idf, (size_t)b->n_terms * sizeof(float)));
+  OI_CK(cudaMalloc(&d_idf, (size_t)b->n_terms * sizeof(float)));
   cudaError_t e = cudaMemcpyAsync(d_idf, idf.data(), idf.size() * sizeof(float), cudaMemcpyHostToDevice, st);
   if (e == cudaSuccess && b->n_postings) {
-    bm25_weights_kernel<<<grid_for(b->n_postings, 256, h->num_sms), 256, 0, st>>>(b->d_term_off, b->d_doc_ids, b->d_tfs, b->d_doc_len, d_idf,
+    bm25_weights_kernel<<<oi_grid(b->n_postings, 256, h->num_sms), 256, 0, st>>>(b->d_term_off, b->d_doc_ids, b->d_tfs, b->d_doc_len, d_idf,
                                                                                   b->n_terms, b->n_postings, params->k1, params->b, avgdl, b->d_w,
                                                                                   b->d_post, b->d_dense_slot, b->d_dense, b->dense_stride);
     ++h->launches;
@@ -1260,7 +1245,7 @@ extern "C" oi_status oi_index_bm25_finalize(oi_index *h, const oi_bm25_params *p
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   cudaFree(d_idf);
-  BM_CK(e);
+  OI_CK(e);
   b->finalized = true;
   return OI_OK;
 }
@@ -1272,15 +1257,15 @@ extern "C" oi_status oi_index_read_bm25(oi_index *h, uint64_t *term_offsets, uin
   OiBm25 *b = h->bm25;
   if (!b) return h->fail(OI_ERR_STATE, "no BM25 index loaded");
   if (weights && !b->finalized) return h->fail(OI_ERR_STATE, "weights requested before oi_index_bm25_finalize");
-  BM_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
   const size_t P = b->n_postings;
-  if (term_offsets) BM_CK(cudaMemcpyAsync(term_offsets, b->d_term_off, ((size_t)b->n_terms + 1) * sizeof(u64), cudaMemcpyDeviceToHost, st));
-  if (doc_ids && P) BM_CK(cudaMemcpyAsync(doc_ids, b->d_doc_ids, P * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-  if (tfs && P) BM_CK(cudaMemcpyAsync(tfs, b->d_tfs, P * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-  if (doc_len && h->desc.n_docs) BM_CK(cudaMemcpyAsync(doc_len, b->d_doc_len, h->desc.n_docs * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-  if (weights && P) BM_CK(cudaMemcpyAsync(weights, b->d_w, P * sizeof(float), cudaMemcpyDeviceToHost, st));
-  BM_CK(cudaStreamSynchronize(st));
+  if (term_offsets) OI_CK(cudaMemcpyAsync(term_offsets, b->d_term_off, ((size_t)b->n_terms + 1) * sizeof(u64), cudaMemcpyDeviceToHost, st));
+  if (doc_ids && P) OI_CK(cudaMemcpyAsync(doc_ids, b->d_doc_ids, P * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  if (tfs && P) OI_CK(cudaMemcpyAsync(tfs, b->d_tfs, P * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  if (doc_len && h->desc.n_docs) OI_CK(cudaMemcpyAsync(doc_len, b->d_doc_len, h->desc.n_docs * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  if (weights && P) OI_CK(cudaMemcpyAsync(weights, b->d_w, P * sizeof(float), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
   return OI_OK;
 }
 
@@ -1299,7 +1284,7 @@ oi_status oi_bm25_local_keys(oi_index *h, const uint32_t *d_q_terms, const uint3
   bm25_prep_queries_kernel<<<(nq + 3) / 4, 128, 0, st>>>(d_q_terms, d_q_offs, nq, b->d_term_off, b->n_terms,
                                                              b->d_qterms, b->d_qnt, b->d_gthr, b->d_counter, b->d_best, k, b->d_qlock);
   ++h->launches;
-  BM_CK(cudaGetLastError());
+  OI_CK(cudaGetLastError());
 
   Bm25Params p;
   p.term_off = b->d_term_off; p.doc_ids = b->d_doc_ids; p.post = b->d_post;
@@ -1367,11 +1352,11 @@ oi_status oi_bm25_local_keys(oi_index *h, const uint32_t *d_q_terms, const uint3
   if ((size_t)p.S * nq * k > b->lists_cap) return h->fail(OI_ERR_CUDA, "internal: BM25 list workspace too small (%u x %u)", p.S, nq);
   const size_t smem = smem_for(ng, p.R, nslot);
   if (!b->attr_set) {  // once per index (the attribute is per function and device)
-    BM_CK(cudaFuncSetAttribute(bm25_blocked_kernel<512, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    BM_CK(cudaFuncSetAttribute(bm25_blocked_kernel<512, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    BM_CK(cudaFuncSetAttribute(bm25_blocked_kernel<768, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    BM_CK(cudaFuncSetAttribute(bm25_blocked_kernel<576, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    BM_CK(cudaFuncSetAttribute(bm25_blocked_kernel<640, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    OI_CK(cudaFuncSetAttribute(bm25_blocked_kernel<512, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    OI_CK(cudaFuncSetAttribute(bm25_blocked_kernel<512, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    OI_CK(cudaFuncSetAttribute(bm25_blocked_kernel<768, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    OI_CK(cudaFuncSetAttribute(bm25_blocked_kernel<576, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    OI_CK(cudaFuncSetAttribute(bm25_blocked_kernel<640, 2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     b->attr_set = true;
   }
   // one CTA per SM; with fewer items than SMs x warps the items still spread over all SMs (each SM's first warps
@@ -1383,10 +1368,10 @@ oi_status oi_bm25_local_keys(oi_index *h, const uint32_t *d_q_terms, const uint3
   else if (p.R == 2048) bm25_blocked_kernel<512, 2048><<<grid, ng * 32, smem, st>>>(p);
   else bm25_blocked_kernel<512, 0><<<grid, ng * 32, smem, st>>>(p);
   ++h->launches;
-  BM_CK(cudaGetLastError());
+  OI_CK(cudaGetLastError());
 #ifdef OI_BM25_STATS
   bm25_stats_print_kernel<<<1, 1, 0, st>>>();
 #endif
-  BM_CK(oi_launch_merge_shards(b->d_lists, p.S, nq, k, d_out_keys, st, &h->launches, 0, b->d_gthr));
+  OI_CK(oi_launch_merge_shards(b->d_lists, p.S, nq, k, d_out_keys, st, &h->launches, 0, b->d_gthr));
   return OI_OK;
 }

@@ -621,14 +621,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
 
 }  // namespace
 
-#define GM_CK(call)                                                                              \
-  do {                                                                                           \
-    cudaError_t e_ = (call);                                                                     \
-    if (e_ != cudaSuccess)                                                                       \
-      return h->fail(e_ == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA,       \
-                     "%s failed: %s", #call, cudaGetErrorString(e_));                            \
-  } while (0)
-
 void oi_gemm_free(oi_index *h) {
   OiGemm *g = h->gemm;
   if (!g) return;
@@ -653,17 +645,17 @@ static oi_status gemm_prepare(oi_index *h) {
   const size_t n_qt_max = (B + 127) / 128;
   g->cap = kCapMax;
   g->max_lists = (size_t)std::max<size_t>((size_t)h->num_sms, n_qt_max) * 128;
-  GM_CK(cudaMalloc(&g->d_qb, n_qt_max * 128 * dim * sizeof(__nv_bfloat16)));
-  GM_CK(cudaMalloc(&g->d_cand, g->max_lists * g->cap * sizeof(u64)));
-  GM_CK(cudaMalloc(&g->d_cnt, g->max_lists * sizeof(uint32_t)));
-  GM_CK(cudaMalloc(&g->d_keys_a, B * K * sizeof(u64)));
-  GM_CK(cudaMalloc(&g->d_keys_b, B * K * sizeof(u64)));
-  GM_CK(cudaMalloc(&g->d_lvl_thr, B * kLevels * sizeof(float)));
-  GM_CK(cudaMalloc(&g->d_lvl_cnt, B * kLevels * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&g->d_qb, n_qt_max * 128 * dim * sizeof(__nv_bfloat16)));
+  OI_CK(cudaMalloc(&g->d_cand, g->max_lists * g->cap * sizeof(u64)));
+  OI_CK(cudaMalloc(&g->d_cnt, g->max_lists * sizeof(uint32_t)));
+  OI_CK(cudaMalloc(&g->d_keys_a, B * K * sizeof(u64)));
+  OI_CK(cudaMalloc(&g->d_keys_b, B * K * sizeof(u64)));
+  OI_CK(cudaMalloc(&g->d_lvl_thr, B * kLevels * sizeof(float)));
+  OI_CK(cudaMalloc(&g->d_lvl_cnt, B * kLevels * sizeof(uint32_t)));
 
   void *fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
-  GM_CK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+  OI_CK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
   if (!fn || qres != cudaDriverEntryPointSuccess) return h->fail(OI_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
   // 3-D view (64 elements, rows, k-blocks): one TMA op brings KBS consecutive 128 B column slabs of 64 rows,
   // each landing as its own swizzled 8 KB slab.  If the driver rejects the view, fall back to one 2-D box per slab.
@@ -697,7 +689,7 @@ static oi_status gemm_prepare(oi_index *h) {
     g->tma3d = false;
   }
   const int smem = (int)gemm_smem_bytes(24), smem_lite = (int)gemm_smem_bytes(12);
-#define OI_GEMM_ATTR(KERNEL, NKB, RING, BYTES) GM_CK(cudaFuncSetAttribute(KERNEL<NKB, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES))
+#define OI_GEMM_ATTR(KERNEL, NKB, RING, BYTES) OI_CK(cudaFuncSetAttribute(KERNEL<NKB, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES))
   OI_GEMM_ATTR(cosine_gemm_kernel, 1, 24, smem); OI_GEMM_ATTR(cosine_gemm_kernel, 2, 24, smem); OI_GEMM_ATTR(cosine_gemm_kernel, 3, 24, smem);
   OI_GEMM_ATTR(cosine_gemm_kernel, 4, 24, smem); OI_GEMM_ATTR(cosine_gemm_kernel, 6, 24, smem); OI_GEMM_ATTR(cosine_gemm_kernel, 8, 24, smem);
   OI_GEMM_ATTR(cosine_gemm_kernel, 12, 24, smem);
@@ -749,7 +741,7 @@ static oi_status gemm_launch(oi_index *h, uint32_t nq, uint32_t n_qt, uint32_t n
     }
 #undef OI_GEMM_PAIR
     ++h->launches;
-    GM_CK(cudaGetLastError());
+    OI_CK(cudaGetLastError());
     return OI_OK;
   }
   const size_t smem = gemm_smem_bytes(lite ? 12 : 24);
@@ -764,7 +756,7 @@ static oi_status gemm_launch(oi_index *h, uint32_t nq, uint32_t n_qt, uint32_t n
   }
 #undef OI_GEMM_GO
   ++h->launches;
-  GM_CK(cudaGetLastError());
+  OI_CK(cudaGetLastError());
   return OI_OK;
 }
 
@@ -792,7 +784,7 @@ oi_status oi_gemm_local_keys(oi_index *h, const float *d_queries, uint32_t nq, u
     unsigned blocks = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)h->num_sms * 8);
     gemm_prep_queries_kernel<<<blocks, 256, 0, st>>>(d_queries, nq, rows, h->desc.dim, reinterpret_cast<uint32_t *>(g->d_qb));
     ++h->launches;
-    GM_CK(cudaGetLastError());
+    OI_CK(cudaGetLastError());
   }
   // Two passes.  PROBE: every CTA scores `pt` tiles of a strided sample of the shard (about 1/256 of its tiles) and
   // keeps only the maxima of groups of 8 scores; the merge's k-th best of those is a score at least k documents
@@ -812,12 +804,12 @@ oi_status oi_gemm_local_keys(oi_index *h, const float *d_queries, uint32_t nq, u
     if ((s = gemm_launch(h, nq, n_qt, n_ranges, k, cap, 0, n_probe, stride, true, nullptr, nullptr, lite, pair, st))) return s;
     gemm_merge_kernel<<<nq, 256, 0, st>>>(g->d_cand, g->d_cnt, cap, n_ranges, n_qt, k, nullptr, g->d_keys_a, g->d_lvl_thr, g->d_lvl_cnt);
     ++h->launches;
-    GM_CK(cudaGetLastError());
+    OI_CK(cudaGetLastError());
     thr = g->d_lvl_thr;
   }
   if ((s = gemm_launch(h, nq, n_qt, n_ranges, k, cap, 0, n_tiles, 1, false, thr, d_dump, lite, pair, st))) return s;
   gemm_merge_kernel<<<nq, 256, 0, st>>>(g->d_cand, g->d_cnt, cap, n_ranges, n_qt, k, nullptr, d_out_keys, nullptr, nullptr);
   ++h->launches;
-  GM_CK(cudaGetLastError());
+  OI_CK(cudaGetLastError());
   return OI_OK;
 }

@@ -119,6 +119,23 @@ struct oi_index {
 cudaError_t call_begin(oi_index *h, cudaStream_t st);
 cudaError_t call_end(oi_index *h, cudaStream_t st);
 
+// a failed CUDA call fails the handle's call (`h` in scope): out of memory for a failed allocation, a CUDA error else
+#define OI_CK(call)                                                                              \
+  do {                                                                                           \
+    cudaError_t e_ = (call);                                                                     \
+    if (e_ != cudaSuccess)                                                                       \
+      return h->fail(e_ == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA,       \
+                     "%s failed: %s", #call, cudaGetErrorString(e_));                            \
+  } while (0)
+
+// blocks of `threads` for a grid-stride loop over n items: one per `threads` items, at most 16 per SM, at least 1
+inline unsigned oi_grid(u64 n, int threads, int num_sms) {
+  u64 b = (n + threads - 1) / threads;
+  const u64 cap = (u64)num_sms * 16;
+  if (b > cap) b = cap;
+  return (unsigned)(b ? b : 1);
+}
+
 // A staging slot for one small host-buffer call.  Taken under the handle's lock (waiting, lock released, while all are
 // busy); given back by the guard after the caller has copied its results out -- or on any early return.
 struct SlotLease {

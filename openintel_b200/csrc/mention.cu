@@ -37,8 +37,6 @@ __global__ void __launch_bounds__(128) mention_summary_kernel(const double *pola
 }
 
 // ---- timelines (SPEC §8b)
-constexpr int kEdgesInSmem = 4096;  // edges[0 .. n_buckets] staged in shared memory (32 KB) when they fit
-
 // len[i] = the length of term i's list, len[n] = 0: the exclusive scan in place makes len the lists' starts in the
 // concatenation of the requested lists and len[n] their total
 __global__ void timeline_lengths_kernel(const u64 *term_off, const uint32_t *terms, uint32_t n, u64 *len) {
@@ -47,16 +45,12 @@ __global__ void timeline_lengths_kernel(const u64 *term_off, const uint32_t *ter
 }
 
 // posting p of the concatenation -> key i * nb + b (term i, bucket b) or the sentinel n * nb when the post's time is
-// outside [edges[0], edges[nb]); value = the doc id.  start[0 .. n]: the lists' starts, start[n] = total.
+// outside [edges[0], edges[nb]); value = the doc id.  start[0 .. n]: the lists' starts, start[n] = total.  The edges
+// are staged in dynamic shared memory when they fit (oi_stage_edges; the launch sizes it).
 __global__ void __launch_bounds__(256) timeline_keys_kernel(const u64 *term_off, const uint32_t *doc_ids, const int64_t *times,
                                                             const uint32_t *terms, const u64 *start, uint32_t n, u64 total,
                                                             const int64_t *edges, uint32_t nb, uint32_t *keys, uint32_t *vals) {
-  __shared__ int64_t s_edges[kEdgesInSmem];
-  const bool staged = nb < kEdgesInSmem;
-  if (staged)
-    for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_edges[k] = edges[k];
-  __syncthreads();
-  const int64_t *E = staged ? s_edges : edges;
+  const int64_t *E = oi_stage_edges(edges, nb);
   for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
     uint32_t a = 0, b = n;  // the term: start[a] <= p < start[b] (an empty list shares its start with the next one)
     while (b - a > 1) {
@@ -98,18 +92,13 @@ __global__ void __launch_bounds__(128) mention_timeline_kernel(const double *pol
 // (oi_postings.cuh), finds each posting's term and its post's bucket, and counts it in counts[term * nb + bucket].  The
 // lanes of a warp that hit the same slot -- the common case inside a long list -- add their popcount with one atomic,
 // so a head term does not serialise on its few counters.  The doc ids are streamed; the times (and the flags with a
-// source filter) are gathered.  Integer counts: any schedule gives the same result.  The edges are staged in dynamic
-// shared memory when nb < kEdgesInSmem (the launch sizes it), else read from global memory.
+// source filter) are gathered.  Integer counts: any schedule gives the same result.  The edges are staged as in
+// timeline_keys_kernel.
 __global__ void __launch_bounds__(256) mention_counts_kernel(const u64 *__restrict__ term_off, const uint32_t *__restrict__ doc_ids,
                                                              const int64_t *__restrict__ times, const uint8_t *__restrict__ flags,
                                                              uint32_t n_terms, u64 n_postings, const int64_t *edges, uint32_t nb,
                                                              int source, uint32_t *counts) {
-  extern __shared__ int64_t s_dyn_edges[];
-  const bool staged = nb < kEdgesInSmem;
-  if (staged)
-    for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_dyn_edges[k] = edges[k];
-  __syncthreads();
-  const int64_t *E = staged ? s_dyn_edges : edges;
+  const int64_t *E = oi_stage_edges(edges, nb);
   const int lane = threadIdx.x & 31;
   const u64 warp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((u64)gridDim.x * blockDim.x) >> 5;
   for (u64 tile = warp * OI_BM25_TILE; tile < n_postings; tile += n_warps * OI_BM25_TILE) {
@@ -135,10 +124,8 @@ __global__ void __launch_bounds__(256) mention_counts_kernel(const u64 *__restri
 
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
-unsigned grid_for(u64 n, int num_sms) {
-  const u64 b = (n + 255) / 256, cap = (u64)num_sms * 16;
-  return (unsigned)(b == 0 ? 1 : (b < cap ? b : cap));
-}
+// the dynamic shared memory of a kernel that stages nb + 1 edges (oi_stage_edges)
+size_t edges_smem(uint32_t nb) { return nb < kEdgesInSmem ? ((size_t)nb + 1) * sizeof(int64_t) : 0; }
 
 // a grow-on-demand device buffer of the handle: at least `want` bytes, with 25 % headroom when it grows
 cudaError_t grow(unsigned char *&buf, size_t &cap, size_t want, cudaStream_t st) {
@@ -153,15 +140,45 @@ cudaError_t grow(unsigned char *&buf, size_t &cap, size_t want, cudaStream_t st)
   return e;
 }
 
-}  // namespace
+// What a mention call takes: term ids (summary, timeline), bucket edges and the post times (timeline, counts), and
+// the messages of its NULL-argument and no-bucket refusals.
+struct MentionCall {
+  bool terms, edges;
+  const char *null_args, *no_bucket;
+};
+constexpr MentionCall kSummary{true, false, "NULL terms / out_summary", nullptr};
+constexpr MentionCall kTimeline{true, true, "NULL terms / edges / out_summary", "n_buckets = 0: a timeline needs a bucket"};
+constexpr MentionCall kCounts{false, true, "NULL edges / out_counts", "n_buckets = 0: counts need a bucket"};
 
-#define MN_CK(call)                                                                              \
-  do {                                                                                           \
-    cudaError_t e_ = (call);                                                                     \
-    if (e_ != cudaSuccess)                                                                       \
-      return h->fail(e_ == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA,       \
-                     "%s failed: %s", #call, cudaGetErrorString(e_));                            \
-  } while (0)
+// The state and argument checks of the mention calls, in the order they find a fault: the BM25 part, the signals and
+// the times; no term (OI_OK, nothing to do -- with any pointers); a NULL argument, no bucket, more (term, bucket)
+// segments than 32-bit keys hold, edges that do not increase strictly, the source, the term ids.  Under the lock.
+oi_status mention_check(oi_index *h, const MentionCall &c, const uint32_t *terms, uint32_t n_terms, const int64_t *edges,
+                        uint32_t n_buckets, int32_t source, const void *out) {
+  if (!oi_bm25_term_offsets(h)) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
+  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
+  if (c.edges && !h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
+  if (c.terms && n_terms == 0) return OI_OK;
+  if ((c.terms && !terms) || (c.edges && !edges) || !out) return h->fail(OI_ERR_INVALID_ARG, "%s", c.null_args);
+  if (c.edges && n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "%s", c.no_bucket);
+  const u64 n_seg = (u64)n_terms * n_buckets;
+  if (c.terms && c.edges && n_seg > 0xFFFFFFFFull)  // the keys are u32 and the sentinel is n_seg itself
+    return h->fail(OI_ERR_INVALID_ARG, "n_terms x n_buckets = %llu: at most 2^32 - 1", (unsigned long long)n_seg);
+  if (c.edges)
+    for (uint32_t b = 0; b < n_buckets; ++b)
+      if (!(edges[b] < edges[b + 1]))
+        return h->fail(OI_ERR_INVALID_ARG, "edges[%u] = %lld, edges[%u] = %lld: the edges must increase strictly", b,
+                       (long long)edges[b], b + 1, (long long)edges[b + 1]);
+  if (source < -1 || source >= OI_N_SOURCES)
+    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
+  const uint32_t V = oi_bm25_n_terms(h);
+  if (c.terms)
+    for (uint32_t i = 0; i < n_terms; ++i)
+      if (terms[i] >= V) return h->fail(OI_ERR_INVALID_ARG, "terms[%u] = %u: the BM25 part has %u terms", i, terms[i], V);
+  return OI_OK;
+}
+
+}  // namespace
 
 void oi_mention_free(oi_index *h) {
   cudaFree(h->d_sig_pol);
@@ -201,7 +218,7 @@ extern "C" oi_status oi_index_load_post_signals(oi_index *h, const double *polar
     pol[i] = p == 0.0 ? 0.0 : p;  // -0.0 -> +0.0: the summary leaves zero polarities out of its add chain
     fl[i] = (uint8_t)(speculative[i] | source[i] << 1);
   }
-  MN_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   if (!h->d_sig_pol) {
     cudaError_t e = cudaMalloc(&h->d_sig_pol, pol.size() * sizeof(double));
     if (e == cudaSuccess) e = cudaMalloc(&h->d_sig_flags, fl.size());
@@ -213,14 +230,14 @@ extern "C" oi_status oi_index_load_post_signals(oi_index *h, const double *polar
                      cudaGetErrorString(e));
     }
   }
-  MN_CK(call_begin(h, h->stream));
+  OI_CK(call_begin(h, h->stream));
   h->has_signals = false;  // until the copies have landed
   if (n) {
-    MN_CK(cudaMemcpyAsync(h->d_sig_pol, pol.data(), n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    MN_CK(cudaMemcpyAsync(h->d_sig_flags, fl.data(), n, cudaMemcpyHostToDevice, h->stream));
+    OI_CK(cudaMemcpyAsync(h->d_sig_pol, pol.data(), n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    OI_CK(cudaMemcpyAsync(h->d_sig_flags, fl.data(), n, cudaMemcpyHostToDevice, h->stream));
   }
-  MN_CK(call_end(h, h->stream));
-  MN_CK(cudaStreamSynchronize(h->stream));
+  OI_CK(call_end(h, h->stream));
+  OI_CK(cudaStreamSynchronize(h->stream));
   h->has_signals = true;
   return OI_OK;
 }
@@ -230,19 +247,12 @@ extern "C" oi_status oi_index_mention_summary(oi_index *h, const uint32_t *terms
                                               oi_mention_state *out_state, oi_social_summary *out_summary) {
   if (!h) return OI_ERR_INVALID_ARG;
   std::unique_lock<std::mutex> lock(h->mu);
+  const oi_status s = mention_check(h, kSummary, terms, n_terms, nullptr, 0, source, out_summary);
+  if (s || n_terms == 0) return s;
   const u64 *term_off = oi_bm25_term_offsets(h);
-  if (!term_off) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
-  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
-  if (n_terms == 0) return OI_OK;
-  if (!terms || !out_summary) return h->fail(OI_ERR_INVALID_ARG, "NULL terms / out_summary");
-  if (source < -1 || source >= OI_N_SOURCES)
-    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
-  const uint32_t V = oi_bm25_n_terms(h);
-  for (uint32_t i = 0; i < n_terms; ++i)
-    if (terms[i] >= V) return h->fail(OI_ERR_INVALID_ARG, "terms[%u] = %u: the BM25 part has %u terms", i, terms[i], V);
-  MN_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
-  MN_CK(call_begin(h, st));
+  OI_CK(call_begin(h, st));
   // in: terms u32 [n] | carries [n] (when given); out: states [n] | summaries [n]
   const size_t n = n_terms, o_carry = align16(n * sizeof(uint32_t));
   const size_t in_bytes = o_carry + (carry_in ? n * sizeof(oi_mention_state) : 0);
@@ -262,26 +272,25 @@ extern "C" oi_status oi_index_mention_summary(oi_index *h, const uint32_t *terms
     oi_index::Slot *sl = lease.sl;
     memcpy(sl->h_in, terms, n * sizeof(uint32_t));
     if (carry_in) memcpy(sl->h_in + o_carry, carry_in, n * sizeof(oi_mention_state));
-    MN_CK(cudaMemcpyAsync(sl->d_in, sl->h_in, in_bytes, cudaMemcpyHostToDevice, st));
-    MN_CK(launch(sl->d_in, sl->d_out));
-    MN_CK(cudaMemcpyAsync(sl->h_out, sl->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
-    oi_status s = lease.finish(st);
-    if (s) return s;
+    OI_CK(cudaMemcpyAsync(sl->d_in, sl->h_in, in_bytes, cudaMemcpyHostToDevice, st));
+    OI_CK(launch(sl->d_in, sl->d_out));
+    OI_CK(cudaMemcpyAsync(sl->h_out, sl->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+    if (oi_status f = lease.finish(st)) return f;
     if (out_state) memcpy(out_state, sl->h_out, n * sizeof(oi_mention_state));
     memcpy(out_summary, sl->h_out + o_sum, n * sizeof(oi_social_summary));
     return OI_OK;
   }
   // a large call: the handle's own device buffers, direct copies from / to the caller's memory
   const size_t o_out = align16(in_bytes);
-  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_out + out_bytes, st));
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_out + out_bytes, st));
   unsigned char *d_in = h->d_mention_io, *d_out = h->d_mention_io + o_out;
-  MN_CK(cudaMemcpyAsync(d_in, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  if (carry_in) MN_CK(cudaMemcpyAsync(d_in + o_carry, carry_in, n * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
-  MN_CK(launch(d_in, d_out));
-  if (out_state) MN_CK(cudaMemcpyAsync(out_state, d_out, n * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
-  MN_CK(cudaMemcpyAsync(out_summary, d_out + o_sum, n * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
-  MN_CK(call_end(h, st));
-  MN_CK(cudaStreamSynchronize(st));
+  OI_CK(cudaMemcpyAsync(d_in, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  if (carry_in) OI_CK(cudaMemcpyAsync(d_in + o_carry, carry_in, n * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
+  OI_CK(launch(d_in, d_out));
+  if (out_state) OI_CK(cudaMemcpyAsync(out_state, d_out, n * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaMemcpyAsync(out_summary, d_out + o_sum, n * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
   return OI_OK;
 }
 
@@ -290,7 +299,7 @@ extern "C" oi_status oi_index_load_post_times(oi_index *h, const int64_t *create
   std::lock_guard<std::mutex> lock(h->mu);
   if (!created_at) return h->fail(OI_ERR_INVALID_ARG, "NULL created_at");
   const u64 n = h->desc.n_docs;
-  MN_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   if (!h->d_times) {
     const cudaError_t e = cudaMalloc(&h->d_times, (n ? n : 1) * sizeof(int64_t));
     if (e != cudaSuccess) {
@@ -299,11 +308,11 @@ extern "C" oi_status oi_index_load_post_times(oi_index *h, const int64_t *create
                      cudaGetErrorString(e));
     }
   }
-  MN_CK(call_begin(h, h->stream));
+  OI_CK(call_begin(h, h->stream));
   h->has_times = false;  // until the copy has landed
-  if (n) MN_CK(cudaMemcpyAsync(h->d_times, created_at, n * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
-  MN_CK(call_end(h, h->stream));
-  MN_CK(cudaStreamSynchronize(h->stream));
+  if (n) OI_CK(cudaMemcpyAsync(h->d_times, created_at, n * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+  OI_CK(call_end(h, h->stream));
+  OI_CK(cudaStreamSynchronize(h->stream));
   h->has_times = true;
   return OI_OK;
 }
@@ -314,40 +323,25 @@ extern "C" oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *term
                                                oi_social_summary *out_summary) {
   if (!h) return OI_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lock(h->mu);
+  const oi_status s = mention_check(h, kTimeline, terms, n_terms, edges, n_buckets, source, out_summary);
+  if (s || n_terms == 0) return s;
   const u64 *term_off = oi_bm25_term_offsets(h);
-  if (!term_off) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
-  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
-  if (!h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
-  if (n_terms == 0) return OI_OK;
-  if (!terms || !edges || !out_summary) return h->fail(OI_ERR_INVALID_ARG, "NULL terms / edges / out_summary");
-  if (n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "n_buckets = 0: a timeline needs a bucket");
   const u64 n_seg = (u64)n_terms * n_buckets;
-  if (n_seg > 0xFFFFFFFFull)  // the keys are u32 and the sentinel is n_seg itself
-    return h->fail(OI_ERR_INVALID_ARG, "n_terms x n_buckets = %llu: at most 2^32 - 1", (unsigned long long)n_seg);
-  for (uint32_t b = 0; b < n_buckets; ++b)
-    if (!(edges[b] < edges[b + 1]))
-      return h->fail(OI_ERR_INVALID_ARG, "edges[%u] = %lld, edges[%u] = %lld: the edges must increase strictly", b,
-                     (long long)edges[b], b + 1, (long long)edges[b + 1]);
-  if (source < -1 || source >= OI_N_SOURCES)
-    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
-  const uint32_t V = oi_bm25_n_terms(h);
-  for (uint32_t i = 0; i < n_terms; ++i)
-    if (terms[i] >= V) return h->fail(OI_ERR_INVALID_ARG, "terms[%u] = %u: the BM25 part has %u terms", i, terms[i], V);
-  MN_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
-  MN_CK(call_begin(h, st));
+  OI_CK(call_begin(h, st));
 
   // d_mention_io: terms u32 [n] | edges i64 [B + 1] | starts u64 [n + 1] | carries [n B] (when given) | states [n B] |
   // summaries [n B] | scan temporaries
   const size_t n = n_terms, nb = n_buckets;
   size_t scan_tmp = 0;
-  MN_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)n + 1, st));
+  OI_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)n + 1, st));
   const size_t o_edges = align16(n * sizeof(uint32_t)), o_start = align16(o_edges + (nb + 1) * sizeof(int64_t));
   const size_t o_carry = align16(o_start + (n + 1) * sizeof(u64));
   const size_t o_state = align16(o_carry + (carry_in ? n_seg * sizeof(oi_mention_state) : 0));
   const size_t o_sum = align16(o_state + n_seg * sizeof(oi_mention_state));
   const size_t o_tmp = align16(o_sum + n_seg * sizeof(oi_social_summary));
-  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
   unsigned char *io = h->d_mention_io;
   uint32_t *d_terms = reinterpret_cast<uint32_t *>(io);
   int64_t *d_edges = reinterpret_cast<int64_t *>(io + o_edges);
@@ -355,17 +349,17 @@ extern "C" oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *term
   oi_mention_state *d_carry = carry_in ? reinterpret_cast<oi_mention_state *>(io + o_carry) : nullptr;
   oi_mention_state *d_state = reinterpret_cast<oi_mention_state *>(io + o_state);
   oi_social_summary *d_sum = reinterpret_cast<oi_social_summary *>(io + o_sum);
-  MN_CK(cudaMemcpyAsync(d_terms, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  MN_CK(cudaMemcpyAsync(d_edges, edges, (nb + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-  if (carry_in) MN_CK(cudaMemcpyAsync(d_carry, carry_in, n_seg * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
-  timeline_lengths_kernel<<<grid_for(n + 1, h->num_sms), 256, 0, st>>>(term_off, d_terms, n_terms, d_start);
+  OI_CK(cudaMemcpyAsync(d_terms, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  OI_CK(cudaMemcpyAsync(d_edges, edges, (nb + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  if (carry_in) OI_CK(cudaMemcpyAsync(d_carry, carry_in, n_seg * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
+  timeline_lengths_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(term_off, d_terms, n_terms, d_start);
   ++h->launches;
-  MN_CK(cudaGetLastError());
-  MN_CK(cub::DeviceScan::ExclusiveSum(io + o_tmp, scan_tmp, d_start, d_start, (int64_t)n + 1, st));
+  OI_CK(cudaGetLastError());
+  OI_CK(cub::DeviceScan::ExclusiveSum(io + o_tmp, scan_tmp, d_start, d_start, (int64_t)n + 1, st));
   h->launches += 2;
   u64 total = 0;
-  MN_CK(cudaMemcpyAsync(&total, d_start + n, sizeof(u64), cudaMemcpyDeviceToHost, st));
-  MN_CK(cudaStreamSynchronize(st));
+  OI_CK(cudaMemcpyAsync(&total, d_start + n, sizeof(u64), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
 
   // d_timeline_ws: keys u32 [P] x 2 | doc ids u32 [P] x 2 | segment offsets u64 [n B + 1] | sort temporaries
   int end_bit = 0;
@@ -373,42 +367,41 @@ extern "C" oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *term
   size_t sort_tmp = 0;
   if (total) {
     cub::DoubleBuffer<uint32_t> kb(nullptr, nullptr), vb(nullptr, nullptr);
-    MN_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+    OI_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
   }
   const size_t o_seg = align16(4 * total * sizeof(uint32_t)), o_stmp = align16(o_seg + (n_seg + 1) * sizeof(u64));
-  MN_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, o_stmp + sort_tmp, st));
+  OI_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, o_stmp + sort_tmp, st));
   unsigned char *ws = h->d_timeline_ws;
   uint32_t *d_keys = reinterpret_cast<uint32_t *>(ws);
   u64 *d_seg = reinterpret_cast<u64 *>(ws + o_seg);
   const uint32_t *sorted_keys = d_keys, *sorted_docs = nullptr;
   if (total) {
-    timeline_keys_kernel<<<grid_for(total, h->num_sms), 256, 0, st>>>(term_off, oi_bm25_doc_ids(h), h->d_times, d_terms, d_start,
-                                                                      n_terms, total, d_edges, n_buckets, d_keys,
-                                                                      d_keys + 2 * total);
+    timeline_keys_kernel<<<oi_grid(total, 256, h->num_sms), 256, edges_smem(n_buckets), st>>>(
+        term_off, oi_bm25_doc_ids(h), h->d_times, d_terms, d_start, n_terms, total, d_edges, n_buckets, d_keys, d_keys + 2 * total);
     ++h->launches;
-    MN_CK(cudaGetLastError());
+    OI_CK(cudaGetLastError());
     // stable: the input is in (term, doc) order, so every (term, bucket) segment stays in doc order
     cub::DoubleBuffer<uint32_t> kb(d_keys, d_keys + total), vb(d_keys + 2 * total, d_keys + 3 * total);
-    MN_CK(cub::DeviceRadixSort::SortPairs(ws + o_stmp, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+    OI_CK(cub::DeviceRadixSort::SortPairs(ws + o_stmp, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
     h->launches += 1 + (end_bit + 7) / 8;  // histogram + one pass per 8 bits
     sorted_keys = kb.Current();
     sorted_docs = vb.Current();
   }
-  timeline_segments_kernel<<<grid_for(n_seg + 1, h->num_sms), 256, 0, st>>>(sorted_keys, total, n_seg, d_seg);
+  timeline_segments_kernel<<<oi_grid(n_seg + 1, 256, h->num_sms), 256, 0, st>>>(sorted_keys, total, n_seg, d_seg);
   ++h->launches;
-  MN_CK(cudaGetLastError());
+  OI_CK(cudaGetLastError());
   // a grid that stays resident walks the segments: most are tiny, so no CTA is launched for a single one of them
   int per_sm = 0;
-  MN_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_timeline_kernel, 128, 0));
+  OI_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_timeline_kernel, 128, 0));
   const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
   mention_timeline_kernel<<<(unsigned)(n_seg < resident ? n_seg : resident), 128, 0, st>>>(
       h->d_sig_pol, h->d_sig_flags, sorted_docs, d_seg, n_seg, source, bull_bear_threshold, d_carry, d_state, d_sum);
   ++h->launches;
-  MN_CK(cudaGetLastError());
-  if (out_state) MN_CK(cudaMemcpyAsync(out_state, d_state, n_seg * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
-  MN_CK(cudaMemcpyAsync(out_summary, d_sum, n_seg * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
-  MN_CK(call_end(h, st));
-  MN_CK(cudaStreamSynchronize(st));
+  OI_CK(cudaGetLastError());
+  if (out_state) OI_CK(cudaMemcpyAsync(out_state, d_state, n_seg * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaMemcpyAsync(out_summary, d_sum, n_seg * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
   return OI_OK;
 }
 
@@ -416,48 +409,38 @@ extern "C" oi_status oi_index_mention_counts(oi_index *h, const int64_t *edges, 
                                              uint32_t *out_counts) {
   if (!h) return OI_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lock(h->mu);
+  const oi_status s = mention_check(h, kCounts, nullptr, 0, edges, n_buckets, source, out_counts);
+  if (s) return s;
   const u64 *term_off = oi_bm25_term_offsets(h);
-  if (!term_off) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
-  if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
-  if (!h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
-  if (!edges || !out_counts) return h->fail(OI_ERR_INVALID_ARG, "NULL edges / out_counts");
-  if (n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "n_buckets = 0: counts need a bucket");
-  for (uint32_t b = 0; b < n_buckets; ++b)
-    if (!(edges[b] < edges[b + 1]))
-      return h->fail(OI_ERR_INVALID_ARG, "edges[%u] = %lld, edges[%u] = %lld: the edges must increase strictly", b,
-                     (long long)edges[b], b + 1, (long long)edges[b + 1]);
-  if (source < -1 || source >= OI_N_SOURCES)
-    return h->fail(OI_ERR_INVALID_ARG, "source = %d: -1 (all posts) or a source code below %d", source, OI_N_SOURCES);
   const uint32_t V = oi_bm25_n_terms(h);
   const u64 n_seg = (u64)V * n_buckets, nb1 = (u64)n_buckets + 1;
   if (n_seg == 0) return OI_OK;
   // d_mention_io: edges i64 [B + 1] | counts u32 [V B]; the byte count cannot wrap below 2^64
   if (n_seg > (~(u64)0 - 64 - nb1 * sizeof(int64_t)) / sizeof(uint32_t))
     return h->fail(OI_ERR_OUT_OF_MEMORY, "%u terms x %u buckets of counts do not fit the address space", V, n_buckets);
-  MN_CK(cudaSetDevice(h->desc.device));
+  OI_CK(cudaSetDevice(h->desc.device));
   cudaStream_t st = h->stream;
-  MN_CK(call_begin(h, st));
+  OI_CK(call_begin(h, st));
   const size_t o_counts = align16(nb1 * sizeof(int64_t)), bytes = n_seg * sizeof(uint32_t);
-  MN_CK(grow(h->d_mention_io, h->mention_io_bytes, o_counts + bytes, st));
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_counts + bytes, st));
   int64_t *d_edges = reinterpret_cast<int64_t *>(h->d_mention_io);
   uint32_t *d_counts = reinterpret_cast<uint32_t *>(h->d_mention_io + o_counts);
-  MN_CK(cudaMemsetAsync(d_counts, 0, bytes, st));
+  OI_CK(cudaMemsetAsync(d_counts, 0, bytes, st));
   const u64 P = oi_bm25_n_postings(h);
   if (P) {  // a shard without a posting (the token-free shard of a sharded lift) counts nothing
-    MN_CK(cudaMemcpyAsync(d_edges, edges, nb1 * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    const size_t smem = n_buckets < kEdgesInSmem ? nb1 * sizeof(int64_t) : 0;
+    OI_CK(cudaMemcpyAsync(d_edges, edges, nb1 * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    const size_t smem = edges_smem(n_buckets);
     int per_sm = 0;
-    MN_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_counts_kernel, 256, smem));
+    OI_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_counts_kernel, 256, smem));
     const u64 tiles = (P + OI_BM25_TILE - 1) / OI_BM25_TILE, want = (tiles + 7) / 8;  // 8 warps per CTA
     const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
     mention_counts_kernel<<<(unsigned)(want < resident ? want : resident), 256, smem, st>>>(
         term_off, oi_bm25_doc_ids(h), h->d_times, h->d_sig_flags, V, P, d_edges, n_buckets, source, d_counts);
     ++h->launches;
-    MN_CK(cudaGetLastError());
+    OI_CK(cudaGetLastError());
   }
-  MN_CK(cudaMemcpyAsync(out_counts, d_counts, bytes, cudaMemcpyDeviceToHost, st));
-  MN_CK(call_end(h, st));
-  MN_CK(cudaStreamSynchronize(st));
+  OI_CK(cudaMemcpyAsync(out_counts, d_counts, bytes, cudaMemcpyDeviceToHost, st));
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
   return OI_OK;
 }
-#undef MN_CK

@@ -1,6 +1,6 @@
 // oi_postings.cuh — shared device helpers of the per-posting kernels over the BM25 CSR: the term of a posting (the
-// warp-tile walk of bm25.cu's weight and validation kernels, also used by mention.cu's counts) and the time bucket of
-// a post (mention.cu's timelines and counts, SPEC §8b).
+// warp-tile walk of bm25.cu's weight and validation kernels, also used by mention.cu's counts), and the staged edges
+// and the time bucket of a post (mention.cu's timelines and counts, SPEC §8b).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -28,6 +28,19 @@ __device__ __forceinline__ TileTerms bm25_tile_terms(const u64 *__restrict__ ter
   t.lo = __shfl_sync(0xFFFFFFFFu, b, 0);
   t.hi = __shfl_sync(0xFFFFFFFFu, b, 31) + 1;
   return t;
+}
+
+// The edges E[0 .. nb] of a bucketed kernel, staged in the block's dynamic shared memory when nb < kEdgesInSmem (the
+// launch gives (nb + 1) * 8 bytes then, else none) and read from global memory otherwise.  Every thread of the block
+// calls it; -> the edges the block reads.
+constexpr int kEdgesInSmem = 4096;
+__device__ __forceinline__ const int64_t *oi_stage_edges(const int64_t *edges, uint32_t nb) {
+  extern __shared__ int64_t s_dyn_edges[];
+  const bool staged = nb < kEdgesInSmem;
+  if (staged)
+    for (uint32_t k = threadIdx.x; k <= nb; k += blockDim.x) s_dyn_edges[k] = edges[k];
+  __syncthreads();
+  return staged ? s_dyn_edges : edges;
 }
 
 // The bucket of time t among the strictly increasing edges E[0 .. nb]: b with E[b] <= t < E[b + 1], or nb when t is

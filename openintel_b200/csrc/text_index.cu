@@ -257,12 +257,6 @@ __global__ void union_map_kernel(const uint8_t *lv, const u64 *lv_off, const u64
   }
 }
 
-unsigned grid_of(u64 n, int num_sms) {
-  u64 b = (n + 255) / 256;
-  if (b > (u64)num_sms * 16) b = (u64)num_sms * 16;
-  return (unsigned)(b ? b : 1);
-}
-
 // cub temporary storage: one buffer, grown when a call needs more
 struct CubTmp {
   void *p = nullptr;
@@ -311,7 +305,7 @@ struct RecordSort {
     RS_CK(cudaMalloc(&d_keys2, n * sizeof(u64)));
     RS_CK(cudaMalloc(&d_vals, n * sizeof(uint32_t)));
     RS_CK(cudaMalloc(&d_vals2, n * sizeof(uint32_t)));
-    text_keys_kernel<<<grid_of(n, num_sms), 256, 0, st>>>(arena, off, n, d_keys, d_vals);
+    text_keys_kernel<<<oi_grid(n, 256, num_sms), 256, 0, st>>>(arena, off, n, d_keys, d_vals);
     ++launches;
     RS_CK(cudaGetLastError());
     cub::DoubleBuffer<u64> kb(d_keys, d_keys2);
@@ -337,7 +331,7 @@ struct RecordSort {
     RS_CK(cudaStreamSynchronize(st));
     if (m) {
       RS_CK(cudaMalloc(&d_sub, (size_t)m * sizeof(uint32_t)));
-      gather_kernel<<<grid_of(m, num_sms), 256, 0, st>>>(order, d_pos, m, d_sub);
+      gather_kernel<<<oi_grid(m, 256, num_sms), 256, 0, st>>>(order, d_pos, m, d_sub);
       ++launches;
       RS_CK(cudaGetLastError());
       const TokenLess less{arena, off};
@@ -346,7 +340,7 @@ struct RecordSort {
       RS_CK(cub::DeviceMergeSort::StableSortKeys(tmp.p, tb, d_sub, (int64_t)m, less, st));
       launches += 3;  // partition + block sort + merge passes (counted once)
       // the selected slots hold whole runs of equal keys, in key order: the full-byte order refines it in place
-      scatter_kernel<<<grid_of(m, num_sms), 256, 0, st>>>(d_sub, d_pos, m, order);
+      scatter_kernel<<<oi_grid(m, 256, num_sms), 256, 0, st>>>(d_sub, d_pos, m, order);
       ++launches;
       RS_CK(cudaGetLastError());
     }
@@ -456,7 +450,7 @@ extern "C" oi_status oi_index_build_bm25_text(oi_index *h, const uint8_t *texts,
 
   // ---- 5: boundaries -> CSR + vocabulary
   TX_CK(cudaMalloc(&d_flags, T * sizeof(u64)));
-  text_flags_kernel<<<grid_of(T, h->num_sms), 256, 0, st>>>(keys, occ, d_arena, d_occ_off, d_occ_doc, T, d_flags);
+  text_flags_kernel<<<oi_grid(T, 256, h->num_sms), 256, 0, st>>>(keys, occ, d_arena, d_occ_off, d_occ_doc, T, d_flags);
   ++h->launches;
   TX_CK(cudaGetLastError());
   TX_CK(cub::DeviceScan::InclusiveSum(nullptr, tb, d_flags, d_flags, (int64_t)T, st));
@@ -473,12 +467,12 @@ extern "C" oi_status oi_index_build_bm25_text(oi_index *h, const uint8_t *texts,
   TX_CK(cudaMalloc(&d_tfs, P * sizeof(uint32_t)));
   TX_CK(cudaMalloc(&d_pstart, (P + 1) * sizeof(uint32_t)));
   TX_CK(cudaMalloc(&d_first, (size_t)V * sizeof(uint32_t)));
-  text_csr_kernel<<<grid_of(T, h->num_sms), 256, 0, st>>>(d_flags, occ, d_occ_doc, T, d_term_off, d_doc_ids, d_pstart, d_first);
-  text_tf_kernel<<<grid_of(P, h->num_sms), 256, 0, st>>>(d_pstart, P, d_tfs);
+  text_csr_kernel<<<oi_grid(T, 256, h->num_sms), 256, 0, st>>>(d_flags, occ, d_occ_doc, T, d_term_off, d_doc_ids, d_pstart, d_first);
+  text_tf_kernel<<<oi_grid(P, 256, h->num_sms), 256, 0, st>>>(d_pstart, P, d_tfs);
   h->launches += 2;
   TX_CK(cudaGetLastError());
   TX_CK(cudaMalloc(&d_vocab_off, ((size_t)V + 1) * sizeof(u64)));
-  text_vocab_len_kernel<<<grid_of((u64)V + 1, h->num_sms), 256, 0, st>>>(d_first, d_occ_off, V, d_vocab_off);
+  text_vocab_len_kernel<<<oi_grid((u64)V + 1, 256, h->num_sms), 256, 0, st>>>(d_first, d_occ_off, V, d_vocab_off);
   ++h->launches;
   TX_CK(cudaGetLastError());
   TX_CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_vocab_off, d_vocab_off, (int64_t)V + 1, st));
@@ -489,7 +483,7 @@ extern "C" oi_status oi_index_build_bm25_text(oi_index *h, const uint8_t *texts,
   TX_CK(cudaMemcpyAsync(&vocab_bytes, d_vocab_off + V, sizeof(u64), cudaMemcpyDeviceToHost, st));
   TX_CK(cudaStreamSynchronize(st));
   TX_CK(cudaMalloc(&d_vocab, vocab_bytes));
-  text_vocab_copy_kernel<<<grid_of(V, h->num_sms), 256, 0, st>>>(d_first, d_occ_off, d_arena, d_vocab_off, V, d_vocab);
+  text_vocab_copy_kernel<<<oi_grid(V, 256, h->num_sms), 256, 0, st>>>(d_first, d_occ_off, d_arena, d_vocab_off, V, d_vocab);
   ++h->launches;
   TX_CK(cudaGetLastError());
   TX_CK(cudaStreamSynchronize(st));
@@ -571,7 +565,7 @@ extern "C" oi_status oi_index_bm25_union_vocabulary(oi_index *h, const uint8_t *
   UN_CK(cudaMemsetAsync(d_err, 0xFF, 2 * sizeof(unsigned long long), st));
   // the device offsets are absolute: the kernels see the entries through a pointer rebased by offsets[0]
   const uint8_t *d_terms = d_bytes - offsets[0];
-  union_check_kernel<<<grid_of(n, h->num_sms), 256, 0, st>>>(d_terms, d_off, n, d_err);
+  union_check_kernel<<<oi_grid(n, 256, h->num_sms), 256, 0, st>>>(d_terms, d_off, n, d_err);
   ++h->launches;
   UN_CK(cudaGetLastError());
   unsigned long long bad = 0;
@@ -585,7 +579,7 @@ extern "C" oi_status oi_index_bm25_union_vocabulary(oi_index *h, const uint8_t *
   // ---- union: byte order (step 4), boundaries, vocabulary
   UN_CK(sorted.run(d_terms, d_off, n, tmp, st, h->num_sms, h->launches));
   UN_CK(cudaMalloc(&d_flags, n * sizeof(uint32_t)));
-  union_flags_kernel<<<grid_of(n, h->num_sms), 256, 0, st>>>(sorted.keys, sorted.order, d_terms, d_off, n, d_flags);
+  union_flags_kernel<<<oi_grid(n, 256, h->num_sms), 256, 0, st>>>(sorted.keys, sorted.order, d_terms, d_off, n, d_flags);
   ++h->launches;
   UN_CK(cudaGetLastError());
   UN_CK(cub::DeviceScan::InclusiveSum(nullptr, tb, d_flags, d_flags, (int64_t)n, st));
@@ -596,11 +590,11 @@ extern "C" oi_status oi_index_bm25_union_vocabulary(oi_index *h, const uint8_t *
   UN_CK(cudaMemcpyAsync(&V, d_flags + n - 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
   UN_CK(cudaStreamSynchronize(st));
   UN_CK(cudaMalloc(&d_first, (size_t)V * sizeof(uint32_t)));
-  union_first_kernel<<<grid_of(n, h->num_sms), 256, 0, st>>>(d_flags, sorted.order, n, d_first);
+  union_first_kernel<<<oi_grid(n, 256, h->num_sms), 256, 0, st>>>(d_flags, sorted.order, n, d_first);
   ++h->launches;
   UN_CK(cudaGetLastError());
   UN_CK(cudaMalloc(&d_vocab_off, ((size_t)V + 1) * sizeof(u64)));
-  text_vocab_len_kernel<<<grid_of((u64)V + 1, h->num_sms), 256, 0, st>>>(d_first, d_off, V, d_vocab_off);
+  text_vocab_len_kernel<<<oi_grid((u64)V + 1, 256, h->num_sms), 256, 0, st>>>(d_first, d_off, V, d_vocab_off);
   ++h->launches;
   UN_CK(cudaGetLastError());
   UN_CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_vocab_off, d_vocab_off, (int64_t)V + 1, st));
@@ -611,14 +605,14 @@ extern "C" oi_status oi_index_bm25_union_vocabulary(oi_index *h, const uint8_t *
   UN_CK(cudaMemcpyAsync(&vocab_bytes, d_vocab_off + V, sizeof(u64), cudaMemcpyDeviceToHost, st));
   UN_CK(cudaStreamSynchronize(st));
   UN_CK(cudaMalloc(&d_vocab, vocab_bytes));
-  text_vocab_copy_kernel<<<grid_of(V, h->num_sms), 256, 0, st>>>(d_first, d_off, d_terms, d_vocab_off, V, d_vocab);
+  text_vocab_copy_kernel<<<oi_grid(V, 256, h->num_sms), 256, 0, st>>>(d_first, d_off, d_terms, d_vocab_off, V, d_vocab);
   ++h->launches;
   UN_CK(cudaGetLastError());
 
   // ---- this shard's lists under the global term ids: lengths scattered to their global ids, exclusive scan
   UN_CK(cudaMalloc(&d_term_off, ((size_t)V + 1) * sizeof(u64)));
   UN_CK(cudaMemsetAsync(d_term_off, 0, ((size_t)V + 1) * sizeof(u64), st));
-  union_map_kernel<<<grid_of(n_local, h->num_sms), 256, 0, st>>>(h->d_vocab, h->d_vocab_off, term_off, n_local, d_vocab,
+  union_map_kernel<<<oi_grid(n_local, 256, h->num_sms), 256, 0, st>>>(h->d_vocab, h->d_vocab_off, term_off, n_local, d_vocab,
                                                                   d_vocab_off, V, d_term_off, d_err + 1);
   ++h->launches;
   UN_CK(cudaGetLastError());

@@ -441,6 +441,17 @@ class ShardedStoreIndex:
         self.close()
 
 
+def _mentions_by_source(state):
+    """{source name: post count} of a mention state (capi.MENTION_STATE_DTYPE), {} for none"""
+    return {} if state is None else {SOURCES[s]: int(state["by_source"][s]) for s in range(len(SOURCES))}
+
+
+def _social_block(state, summary):
+    """the "social" block (analyze.social_block) of a mention state and its summary; None, None: no post"""
+    from . import analyze
+    return analyze.social_block(analyze.empty_summary() if summary is None else summary, _mentions_by_source(state))
+
+
 class MentionIndex:
     """Per-ticker social reports from the index (SPEC §8a): the posts that mention a ticker are its posting list, so
     the reference's `analyze --mention` report of many tickers takes one device call (one relay over the ranks of a
@@ -476,29 +487,36 @@ class MentionIndex:
 
     def reports(self, tickers, source=None, markets=None, cfg=fusion.EngineConfig()):
         """one report per ticker, in the order given: analyze.build_report of the ticker's posts (of `source` only, when
-        given).  A ticker is normalised like select_posts' mention (leading '$' dropped, lower case); `markets` maps
-        tickers, normalised the same way, to fusion.MarketSummary.  A ticker with no post and no market snapshot -- what
-        analyze refuses with NoData -- gives None."""
+        given).  A ticker is normalised like select_posts' mention (analyze.ticker_key); `markets` maps tickers,
+        normalised the same way, to fusion.MarketSummary.  A ticker with no post and no market snapshot -- what analyze
+        refuses with NoData -- gives None."""
         from . import analyze, sharding
-        keys = [t.lstrip("$").lower() for t in tickers]
-        mk = {k.lstrip("$").lower(): v for k, v in (markets or {}).items()}
-        known = [k for k in dict.fromkeys(keys) if k in self.term_id]  # a ticker outside the vocabulary has no post
-        states, sums = sharding.relay_mention_summary(
-            self.dist, self.ix, np.array([self.term_id[k] for k in known], dtype=np.uint32),
-            None if source is None else SOURCES.index(source), cfg.bull_bear_threshold, device=self.device)
-        found = {k: (st, sm) for k, st, sm in zip(known, states, sums)}
+        mk = {analyze.ticker_key(k): v for k, v in (markets or {}).items()}
         out = []
-        for k in keys:
-            if k in found:
-                st, sm = found[k]
-                by_source = {SOURCES[s]: int(st["by_source"][s]) for s in range(len(SOURCES))}
-            else:
-                sm, by_source = analyze.empty_summary(), {}
+        for k, st, sm in self._relay(tickers, sharding.relay_mention_summary, source, cfg):
             try:
-                out.append(analyze.build_report(sm, by_source, mk.get(k), cfg))
+                out.append(analyze.build_report(analyze.empty_summary() if sm is None else sm, _mentions_by_source(st),
+                                                mk.get(k), cfg))
             except analyze.NoData:
                 out.append(None)
         return out
+
+    @staticmethod
+    def _source_code(source):
+        """a source name (store.SOURCES) -> its code; None (all posts) stays None"""
+        return None if source is None else SOURCES.index(source)
+
+    def _relay(self, tickers, relay, source, cfg, *args):
+        """`relay` (sharding.relay_mention_summary, or relay_mention_timeline with the edges in `args`) over the distinct
+        tickers in the vocabulary, normalised by analyze.ticker_key.  -> per ticker, in the order given, (normalised
+        ticker, states, summaries); (ticker, None, None) for one outside the vocabulary, which has no post"""
+        from . import analyze
+        keys = [analyze.ticker_key(t) for t in tickers]
+        known = [k for k in dict.fromkeys(keys) if k in self.term_id]
+        states, sums = relay(self.dist, self.ix, np.array([self.term_id[k] for k in known], dtype=np.uint32), *args,
+                             self._source_code(source), cfg.bull_bear_threshold, device=self.device)
+        found = dict(zip(known, zip(states, sums)))
+        return [(k,) + found.get(k, (None, None)) for k in keys]
 
     def _load_times(self):
         """parses this shard's created_at and loads it next to the BM25 part.  Sharded, the ranks agree first on whether
@@ -524,6 +542,15 @@ class MentionIndex:
         self.ix.load_post_times(times)
         self.times_loaded = True
 
+    def _edges(self, edges):
+        """the bucket edges as ints, checked; the post times are read from the store and loaded on the first call"""
+        edges = [int(e) for e in edges]
+        if len(edges) < 2 or any(a >= b for a, b in zip(edges, edges[1:])):
+            raise ValueError("edges must be at least two strictly increasing times")
+        if not self.times_loaded:
+            self._load_times()
+        return edges
+
     def timeline(self, tickers, edges, source=None, cfg=fusion.EngineConfig()):
         """per ticker, in the order given, a list of len(edges) - 1 "social" blocks (analyze.social_block): block b
         summarises the ticker's posts (of `source` only, when given) created in [edges[b], edges[b + 1]), seconds since
@@ -531,26 +558,14 @@ class MentionIndex:
         reports as "social".  Tickers are normalised like reports(); one outside the vocabulary gets empty blocks.  The
         post times are read from the store and loaded on the first call; sharded, every rank calls with the same
         arguments."""
-        from . import analyze, sharding
-        edges = [int(e) for e in edges]
-        if len(edges) < 2 or any(a >= b for a, b in zip(edges, edges[1:])):
-            raise ValueError("edges must be at least two strictly increasing times")
-        if not self.times_loaded:
-            self._load_times()
-        keys = [t.lstrip("$").lower() for t in tickers]
-        known = [k for k in dict.fromkeys(keys) if k in self.term_id]
-        states, sums = sharding.relay_mention_timeline(
-            self.dist, self.ix, np.array([self.term_id[k] for k in known], dtype=np.uint32), edges,
-            None if source is None else SOURCES.index(source), cfg.bull_bear_threshold, device=self.device)
-        found = {k: (st, sm) for k, st, sm in zip(known, states, sums)}
+        return self._timeline(tickers, self._edges(edges), source, cfg)
+
+    def _timeline(self, tickers, edges, source, cfg):
+        from . import sharding
         out = []
-        for k in keys:
-            if k not in found:
-                out.append([analyze.social_block(analyze.empty_summary(), {}) for _ in range(len(edges) - 1)])
-                continue
-            st, sm = found[k]
-            out.append([analyze.social_block(sm[b], {SOURCES[s]: int(st[b]["by_source"][s]) for s in range(len(SOURCES))})
-                        for b in range(len(edges) - 1)])
+        for _, states, sums in self._relay(tickers, sharding.relay_mention_timeline, source, cfg, edges):
+            pairs = zip(states, sums) if sums is not None else [(None, None)] * (len(edges) - 1)  # no post
+            out.append([_social_block(st, sm) for st, sm in pairs])
         return out
 
     def mention_counts(self, edges, source=None):
@@ -560,12 +575,7 @@ class MentionIndex:
         first call; sharded, every rank calls with the same arguments.  -> int64 [len(vocab)][len(edges) - 1], the same
         on every rank"""
         from . import sharding
-        edges = [int(e) for e in edges]
-        if len(edges) < 2 or any(a >= b for a, b in zip(edges, edges[1:])):
-            raise ValueError("edges must be at least two strictly increasing times")
-        if not self.times_loaded:
-            self._load_times()
-        counts = self.ix.mention_counts(edges, None if source is None else SOURCES.index(source))
+        counts = self.ix.mention_counts(self._edges(edges), self._source_code(source))
         return sharding.all_reduce_counts(self.dist, counts, device=self.device)
 
     def trending(self, since, until, baseline_since, k, min_mentions=1, source=None, universe=None, cfg=fusion.EngineConfig()):
@@ -575,29 +585,18 @@ class MentionIndex:
         terms with at least min_mentions mentions in the window are ranked; `universe` (tickers, normalised like
         reports()) restricts the ranking to its entries, and one outside the vocabulary is never ranked.  Times are
         seconds since the Unix epoch; sharded, every rank calls with the same arguments and gets the same list."""
-        from . import analyze, sharding, trending
-        t0, t1, t2 = int(baseline_since), int(since), int(until)
-        if not t0 < t1 < t2:
-            raise ValueError("the times must satisfy baseline_since < since < until")
-        if int(k) < 1 or int(min_mentions) < 1:
-            raise ValueError("k and min_mentions must be at least 1")
+        from . import analyze, trending
+        t0, t1, t2, k, min_mentions = trending.check_args(baseline_since, since, until, k, min_mentions)
         counts = self.mention_counts([t0, t1, t2], source)
         mask = None
         if universe is not None:
             mask = np.zeros(len(self.vocab), dtype=bool)
-            mask[[self.term_id[w] for w in (u.lstrip("$").lower() for u in universe) if w in self.term_id]] = True
+            mask[[self.term_id[w] for w in map(analyze.ticker_key, universe) if w in self.term_id]] = True
         ids, expected, surge = trending.rank(counts[:, 1], counts[:, 0], t0, t1, t2, k, min_mentions, mask)
-        states, sums = sharding.relay_mention_timeline(self.dist, self.ix, ids.astype(np.uint32), [t0, t1, t2],
-                                                       None if source is None else SOURCES.index(source),
-                                                       cfg.bull_bear_threshold, device=self.device)
-        out = []
-        for i, t in enumerate(ids):
-            blocks = [analyze.social_block(sums[i][b], {SOURCES[s]: int(states[i][b]["by_source"][s]) for s in range(len(SOURCES))})
-                      for b in range(2)]
-            out.append({"ticker": self.vocab[t], "mentions": int(counts[t, 1]), "baseline_mentions": int(counts[t, 0]),
-                        "expected": float(expected[i]), "surge": float(surge[i]),
-                        "social": {"baseline": blocks[0], "window": blocks[1]}})
-        return out
+        blocks = self._timeline([self.vocab[t] for t in ids], [t0, t1, t2], source, cfg)
+        return [{"ticker": self.vocab[t], "mentions": int(counts[t, 1]), "baseline_mentions": int(counts[t, 0]),
+                 "expected": float(x), "surge": float(sg), "social": {"baseline": b[0], "window": b[1]}}
+                for t, x, sg, b in zip(ids, expected, surge, blocks)]
 
     def close(self):
         self.ix.close()

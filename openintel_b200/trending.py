@@ -20,6 +20,16 @@ import sys
 import numpy as np
 
 
+def check_args(t0, t1, t2, k, min_mentions):
+    """the times and sizes of a ranking as ints, checked: t0 < t1 < t2, k >= 1 and min_mentions >= 1"""
+    t0, t1, t2, k, min_mentions = int(t0), int(t1), int(t2), int(k), int(min_mentions)
+    if not t0 < t1 < t2:
+        raise ValueError("the times must satisfy baseline_since < since < until")
+    if k < 1 or min_mentions < 1:
+        raise ValueError("k and min_mentions must be at least 1")
+    return t0, t1, t2, k, min_mentions
+
+
 def rank(c, m, t0, t1, t2, k, min_mentions=1, candidates=None):
     """The SPEC §8c ranking.  c / m: per-term mention counts in the window [t1, t2) and in the baseline [t0, t1), term
     id = index; candidates: a bool mask over the terms, or None for all.  A candidate has c >= min_mentions (and its
@@ -28,11 +38,7 @@ def rank(c, m, t0, t1, t2, k, min_mentions=1, candidates=None):
         surge    = ((double)c - expected) / sqrt(expected + 1.0)
     Order: surge descending, ties by ascending term id; the first k.
     -> (term ids int64 [<= k], expected f64, surge f64), in rank order"""
-    t0, t1, t2, k, min_mentions = int(t0), int(t1), int(t2), int(k), int(min_mentions)
-    if not t0 < t1 < t2:
-        raise ValueError("the times must satisfy baseline_since < since < until")
-    if k < 1 or min_mentions < 1:
-        raise ValueError("k and min_mentions must be at least 1")
+    t0, t1, t2, k, min_mentions = check_args(t0, t1, t2, k, min_mentions)
     c = np.asarray(c).reshape(-1)
     m = np.asarray(m).reshape(-1)
     if c.shape != m.shape:

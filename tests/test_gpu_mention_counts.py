@@ -4,42 +4,19 @@ a document-sharded index -- and store.MentionIndex.trending and the `trending` C
 with the social blocks of `analyze --mention --since --until` for the baseline and the window."""
 import json
 import math
-import os
-import struct
 import subprocess
 import sys
 
 import numpy as np
 import pytest
 
-from test_gpu_mention_summary import _free_port, _synthetic
-from test_gpu_mention_timeline import T0, DAY, _fixture, _timed_store
+from mention_util import G, oi  # noqa: F401  (fixtures)
+from mention_util import (DAY, ROOT, SMALL_EDGES, T0, bits as _bits, fixture_store, make_store, run_ranks, sharded_corpus,
+                          small_corpus, synthetic as _synthetic)
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SOURCES = (None, "reddit", "bluesky")
-
-
-@pytest.fixture(scope="module")
-def oi():
-    import __graft_entry__ as ge  # noqa: F401
-    import openintel_b200
-    openintel_b200.load_library()
-    import runpy
-    from openintel_b200 import hostlib
-    runpy.run_path(os.path.join(os.path.dirname(hostlib.__file__), "host", "build.py"), run_name="__build__")
-    return openintel_b200
-
-
-@pytest.fixture(scope="module")
-def G():
-    with open(os.path.join(ROOT, "tests", "golden", "reference_lexicon_goldens.json"), encoding="utf-8") as f:
-        return json.load(f)
-
-
-def _bits(x):
-    return struct.pack("<d", float(x))
 
 
 class HostCounts:
@@ -101,7 +78,7 @@ def _check_counts(mi, oracle, edges):
 # ---- 1 + 2. counts == the timeline totals == the host oracle -------------------------------------------------------
 def test_fixture_counts_equal_timeline_totals_and_the_host_oracle(oi, G, tmp_path):
     from openintel_b200 import store
-    conn, _, hours = _fixture(G, str(tmp_path / "fixture.db"))
+    conn, _, hours = fixture_store(G, str(tmp_path / "fixture.db"))
     n = len(hours)
     layouts = [[T0, T0 + 3600 * n],  # one bucket around all posts
                [T0 + 3600 * h for h in range(n + 1)],  # one post per bucket, every post on an edge
@@ -129,7 +106,7 @@ def synthetic(oi, tmp_path_factory):
     on_edge = rng.random(N_SYN) < 0.1
     times[on_edge] = T0 + DAY * rng.integers(-1, 367, int(on_edge.sum()))  # posts exactly on the daily edges
     times[(times >= T0 + 100 * DAY) & (times < T0 + 103 * DAY)] -= 5 * DAY  # three empty days
-    conn = _timed_store(str(tmp_path_factory.mktemp("counts") / "syn.db"), texts, sources, times)
+    conn = make_store(str(tmp_path_factory.mktemp("counts") / "syn.db"), texts, sources, times)
     mi = store.MentionIndex(conn)
     yield dict(conn=conn, mi=mi, oracle=HostCounts(conn, mi.vocab), tickers=tickers)
     mi.close()
@@ -168,45 +145,31 @@ def test_synthetic_trending_equals_the_rule_over_the_host_counts(oi, synthetic):
 
 
 # ---- 3. the sharded index: the shards' counts summed over gloo ranks (all on device 0) ------------------------------
-N_SHARD = 3000
 E_SHARD = [T0 - DAY, T0 + 3 * DAY, T0 + 6 * DAY, T0 + 7 * DAY, T0 + 9 * DAY]
 
 
-def _sharded_worker(rank, world, port, path, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        from openintel_b200 import store
-        conn = store.open_store(path)
-        with store.MentionIndex(conn, dist) as mi:
-            out = {"counts": {str(src): mi.mention_counts(E_SHARD, src).tolist() for src in SOURCES},
-                   "trending": {str(src): json.dumps(mi.trending(T0 + 6 * DAY, T0 + 7 * DAY, T0, 15, source=src))
-                                for src in SOURCES},
-                   "universe": json.dumps(mi.trending(T0 + 6 * DAY, T0 + 7 * DAY, T0, 5, universe=["onlyfirst", "$CALLS", "nope"]))}
-        conn.close()
-        q.put((rank, out))
-    finally:
-        dist.destroy_process_group()
+def _sharded_worker(dist, path):
+    from openintel_b200 import store
+    conn = store.open_store(path)
+    with store.MentionIndex(conn, dist) as mi:
+        out = {"counts": {str(src): mi.mention_counts(E_SHARD, src).tolist() for src in SOURCES},
+               "trending": {str(src): json.dumps(mi.trending(T0 + 6 * DAY, T0 + 7 * DAY, T0, 15, source=src))
+                            for src in SOURCES},
+               "universe": json.dumps(mi.trending(T0 + 6 * DAY, T0 + 7 * DAY, T0, 5, universe=["onlyfirst", "$CALLS", "nope"]))}
+    conn.close()
+    return out
 
 
 @pytest.mark.parametrize("world,tokenless", [(2, False), (3, False), (3, True)])
 def test_sharded_counts_and_trending_equal_the_unsharded_ones(oi, tmp_path, world, tokenless):
-    """`onlyfirst` appears on the first shard only; with `tokenless`, the middle shard's posts hold no token at all"""
-    import torch.multiprocessing as mp
-    from openintel_b200 import sharding, store
-    texts, sources, _ = _synthetic(N_SHARD, 17 + world, n_tickers=60)
-    texts[3] += " onlyfirst moon"
-    texts[10] += " onlyfirst dump"
-    if tokenless:
-        base, n = sharding.shard_range(N_SHARD, world, 1)
-        for i in range(base, base + n):
-            texts[i] = ("!!!", "ÿþ ???", "... — !!", "\U0001f680 $$")[i % 4]
-    times = T0 + np.random.default_rng(world).integers(-2 * DAY, 10 * DAY, N_SHARD)
+    """the sharded corpus of mention_util.sharded_corpus: `onlyfirst` on the first shard only, a token-free middle
+    shard with `tokenless`"""
+    from openintel_b200 import store
+    texts, sources, _ = sharded_corpus(17 + world, world, tokenless)
+    times = T0 + np.random.default_rng(world).integers(-2 * DAY, 10 * DAY, len(texts))
     times[[3, 10]] = T0 + 6 * DAY + 5  # onlyfirst: two posts in the window, none in the baseline
     path = str(tmp_path / "posts.db")
-    _timed_store(path, texts, sources, times).close()
+    make_store(path, texts, sources, times).close()
     conn = store.open_store(path)
     with store.MentionIndex(conn) as mi:
         want = {"counts": {str(src): mi.mention_counts(E_SHARD, src).tolist() for src in SOURCES},
@@ -215,15 +178,7 @@ def test_sharded_counts_and_trending_equal_the_unsharded_ones(oi, tmp_path, worl
         ranked = {e["ticker"]: e for e in json.loads(want["universe"])}
         assert set(ranked) == {"onlyfirst", "calls"} and ranked["onlyfirst"]["surge"] == 2.0  # m = 0: surge = c
     conn.close()
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_sharded_worker, args=(r, world, port, path, q)) for r in range(world)]
-    [p.start() for p in procs]
-    res = sorted([q.get(timeout=600) for _ in procs], key=lambda t: t[0])
-    [p.join(timeout=60) for p in procs]
-    assert all(p.exitcode == 0 for p in procs)
-    for rank, got in res:
+    for rank, got in run_ranks(world, _sharded_worker, path):
         assert got == want, rank
 
 
@@ -263,7 +218,7 @@ def planted(oi, G, tmp_path_factory):
             texts[i] += " " + word
             times[i] = (TB + DAY * j + 11 if (word != "newbie" and j < 3) else TW + 3600 * j + 7)
     path = str(tmp_path_factory.mktemp("planted") / "planted.db")
-    conn = _timed_store(path, texts, sources, times)
+    conn = make_store(path, texts, sources, times)
     mi = store.MentionIndex(conn)
     m = G["fixture_posts"]["mock_market"]
     mk = fusion.MarketSummary.from_snapshot(m["last_price"], m["previous_close"], m["volume"], m["avg_volume"], m["iv_rank"])
@@ -333,35 +288,11 @@ def _raw_counts(ix, edges, nb, source=-1, out=None):
 
 
 def test_errors_and_state(oi):
-    import oracle as O
-    from openintel_b200 import capi
-    texts = ["$GME to the moon", "gme puts", "calls on AMC", "nothing here", "GME GME dump", "amc squeeze yolo"]
-    pol = np.array([O.lexicon_score(t)[0] for t in texts])
-    spec = np.array([O.lexicon_score(t)[1] for t in texts], dtype=np.uint8)
-    src = np.array([0, 1, 0, 1, 1, 0], dtype=np.uint8)
-    times = T0 + np.array([50, 10, 20, 30, 40, 0]) * 3600
-    edges = [T0, T0 + 24 * 3600, T0 + 48 * 3600]
-    with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
-        ix.load_post_signals(pol, spec, src)
-        ix.load_post_times(times)
-        with pytest.raises(oi.OiError) as e:  # signals and times, no BM25 part
-            ix.mention_counts(edges)
-        assert e.value.status == 5 and "BM25" in e.value.message
-    with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
-        ix.build_bm25_text(texts)
-        with pytest.raises(oi.OiError) as e:  # no signals, no times
-            ix.mention_counts(edges)
-        assert e.value.status == 5 and "signals" in e.value.message
-        ix.load_post_times(times)
-        with pytest.raises(oi.OiError) as e:  # times, no signals
-            ix.mention_counts(edges)
-        assert e.value.status == 5 and "signals" in e.value.message
+    texts, pol, spec, src, times = small_corpus()
+    edges = SMALL_EDGES
     with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
         vocab = ix.build_bm25_text(texts)
         ix.load_post_signals(pol, spec, src)
-        with pytest.raises(oi.OiError) as e:  # signals, no times
-            ix.mention_counts(edges)
-        assert e.value.status == 5 and "times" in e.value.message
         ix.load_post_times(times)
         c0 = ix.mention_counts(edges)
         gme, amc, the = vocab.index("gme"), vocab.index("amc"), vocab.index("the")
@@ -437,7 +368,7 @@ def test_trending_cli(oi, planted, tmp_path):
                                                               universe=["$" + P["surging"][0], "twina", "twinb", "notaword"])))
     assert {e["ticker"] for e in out["ranked"]} <= {P["surging"][0], "twina", "twinb"}
     # a created_at without an offset: error and exit 1
-    conn = _timed_store(str(tmp_path / "bad.db"), ["gme moon"], ["reddit"], [T0])
+    conn = make_store(str(tmp_path / "bad.db"), ["gme moon"], ["reddit"], [T0])
     conn.execute("UPDATE posts SET created_at = '2024-01-01 00:00:00'")
     conn.commit()
     conn.close()

@@ -3,7 +3,6 @@
 for bit -- unsharded, relayed over the shards of a document-sharded index, and through store.MentionIndex.timeline and
 the `timeline` CLI."""
 import json
-import os
 import subprocess
 import sys
 
@@ -11,60 +10,17 @@ import numpy as np
 import pytest
 
 import oracle as O
-from test_gpu_mention_summary import _free_port, _lists, _same_summary, _shard_pair, _synthetic
+from mention_util import G, oi  # noqa: F401  (fixtures)
+from mention_util import (DAY, ROOT, SMALL_EDGES, T0, fixture_store, iso as _iso, lists, make_store, run_ranks,
+                          same_summary, shard_pair, sharded_corpus, small_corpus, synthetic as _synthetic)
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-T0 = 1704067200  # 2024-01-01T00:00:00Z
-DAY = 86400
-
-
-def _iso(t):
-    from openintel_b200 import timeline
-    return timeline.format_time(int(t))
-
-
-@pytest.fixture(scope="module")
-def oi():
-    import __graft_entry__ as ge  # noqa: F401
-    import openintel_b200
-    openintel_b200.load_library()
-    import runpy
-    from openintel_b200 import hostlib
-    runpy.run_path(os.path.join(os.path.dirname(hostlib.__file__), "host", "build.py"), run_name="__build__")
-    return openintel_b200
-
-
-@pytest.fixture(scope="module")
-def G():
-    with open(os.path.join(ROOT, "tests", "golden", "reference_lexicon_goldens.json"), encoding="utf-8") as f:
-        return json.load(f)
-
-
-def _timed_store(path, texts, sources, times):
-    from openintel_b200 import store
-    conn = store.open_store(path)
-    store.insert_posts(conn, [dict(id="p%d" % i, source=s, author="a%d" % (i % 97), text=t, created_at=_iso(c), engagement=i % 50)
-                              for i, (t, s, c) in enumerate(zip(texts, sources, times))])
-    return conn
-
-
-def _fixture(G, path):
-    """the reference fixture posts, distinct hourly times not in doc order"""
-    from openintel_b200 import fusion
-    fx = G["fixture_posts"]["posts"]
-    hours = np.random.default_rng(5).permutation(len(fx))
-    conn = _timed_store(path, [p["text"] for p in fx], [p["source"] for p in fx], T0 + 3600 * hours)
-    m = G["fixture_posts"]["mock_market"]
-    return conn, fusion.MarketSummary.from_snapshot(m["last_price"], m["previous_close"], m["volume"], m["avg_volume"],
-                                                    m["iv_rank"]), hours
 
 
 # ---- 1. the reference fixture: MentionIndex.timeline == analyze_posts over select_posts(mention, since, until) ------
 def test_fixture_timeline_equals_analyze_per_bucket(oi, G, tmp_path):
     from openintel_b200 import analyze, capi, store
-    conn, mk, hours = _fixture(G, str(tmp_path / "fixture.db"))
+    conn, mk, hours = fixture_store(G, str(tmp_path / "fixture.db"))
     n = len(hours)
     layouts = [[T0, T0 + 3600 * n],  # one bucket around all posts
                [T0 + 3600 * h for h in range(n + 1)],  # one post per bucket, every post on an edge
@@ -101,7 +57,7 @@ def test_one_bucket_equals_mention_summary(oi):
             s_tl, m_tl = ix.mention_timeline(ids, [T0, T0 + 30 * DAY], source=src)
             assert s_tl.shape == (len(ids), 1) and s_tl[:, 0].tobytes() == s_sum.tobytes()
             for a, b in zip(m_tl, m_sum):
-                _same_summary(a[0], b)
+                same_summary(a[0], b)
 
 
 # ---- 3. a synthetic corpus with times not in doc order, against the oracle -----------------------------------------
@@ -117,7 +73,7 @@ def synthetic(oi, tmp_path_factory):
     on_edge = rng.random(N_SYN) < 0.1
     times[on_edge] = T0 + DAY * rng.integers(-1, 367, int(on_edge.sum()))  # posts exactly on the daily edges
     times[(times >= T0 + 100 * DAY) & (times < T0 + 103 * DAY)] -= 5 * DAY  # three empty days
-    conn = _timed_store(str(tmp_path_factory.mktemp("timeline") / "syn.db"), texts, sources, times)
+    conn = make_store(str(tmp_path_factory.mktemp("timeline") / "syn.db"), texts, sources, times)
     scores = [O.lexicon_score(t) for t in texts]
     posts_of = {}
     for d, t in enumerate(texts):
@@ -146,7 +102,7 @@ def _check(S, ids, words, sums, states, edges, src, thr):
         b = np.searchsorted(edges, S["times"][d], side="right") - 1
         for k in range(len(edges) - 1):
             dk = d[b == k]  # doc order kept
-            _same_summary(sums[i][k], O.social_summary(S["pol"][dk], S["spec"][dk], thr), (w, k, src, thr))
+            same_summary(sums[i][k], O.social_summary(S["pol"][dk], S["spec"][dk], thr), (w, k, src, thr))
             assert int(states[i, k]["total"]) == len(dk)
             assert [int(states[i, k]["by_source"][s]) for s in (0, 1)] == [int(np.sum(S["src"][dk] == s)) for s in (0, 1)]
 
@@ -176,61 +132,34 @@ def test_timeline_equals_the_oracle_over_the_selected_posts(oi, synthetic, n_buc
 
 
 # ---- 4. the sharded relay over gloo ranks (all on device 0) -------------------------------------------------------
-N_SHARD = 3000
 EDGES_SHARD = [T0 + 6 * 3600 * k for k in range(29)]  # 7 days in 6-hour buckets, posts over 8 days
 
 
-def _relay_worker(rank, world, port, path, tickers, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        from openintel_b200 import store
-        conn = store.open_store(path)
-        with store.MentionIndex(conn, dist) as mi:
-            try:
-                out = {src: json.dumps(mi.timeline(tickers, EDGES_SHARD, source=src)) for src in (None, "reddit", "bluesky")}
-            except ValueError as e:
-                out = "ValueError: %s" % e
-        conn.close()
-        q.put((rank, out))
-    finally:
-        dist.destroy_process_group()
-
-
-def _run_ranks(world, path, ask):
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_relay_worker, args=(r, world, port, path, ask, q)) for r in range(world)]
-    [p.start() for p in procs]
-    res = sorted([q.get(timeout=600) for _ in procs], key=lambda t: t[0])
-    [p.join(timeout=60) for p in procs]
-    assert all(p.exitcode == 0 for p in procs)
-    return res
+def _relay_worker(dist, path, tickers):
+    from openintel_b200 import store
+    conn = store.open_store(path)
+    with store.MentionIndex(conn, dist) as mi:
+        try:
+            out = {src: json.dumps(mi.timeline(tickers, EDGES_SHARD, source=src)) for src in (None, "reddit", "bluesky")}
+        except ValueError as e:
+            out = "ValueError: %s" % e
+    conn.close()
+    return out
 
 
 @pytest.mark.parametrize("world,tokenless", [(2, False), (3, False), (3, True)])
 def test_relay_over_the_shards_equals_the_unsharded_timeline(oi, tmp_path, world, tokenless):
-    from openintel_b200 import sharding, store
-    texts, sources, tickers = _synthetic(N_SHARD, 7 + world, n_tickers=60)
-    texts[3] += " onlyfirst moon"
-    texts[10] += " onlyfirst dump"
-    if tokenless:
-        base, n = sharding.shard_range(N_SHARD, world, 1)
-        for i in range(base, base + n):
-            texts[i] = ("!!!", "ÿþ ???", "... — !!", "\U0001f680 $$")[i % 4]
-    times = T0 + np.random.default_rng(world).integers(-DAY, 8 * DAY, N_SHARD)
+    from openintel_b200 import store
+    texts, sources, tickers = sharded_corpus(7 + world, world, tokenless)
+    times = T0 + np.random.default_rng(world).integers(-DAY, 8 * DAY, len(texts))
     path = str(tmp_path / "posts.db")
-    _timed_store(path, texts, sources, times).close()
+    make_store(path, texts, sources, times).close()
     ask = ["$" + t.upper() for t in tickers[:40]] + ["onlyfirst", "calls", "$nothere", tickers[0]]
     conn = store.open_store(path)
     with store.MentionIndex(conn) as mi:
         want = {src: json.dumps(mi.timeline(ask, EDGES_SHARD, source=src)) for src in (None, "reddit", "bluesky")}
     conn.close()
-    for rank, got in _run_ranks(world, path, ask):
+    for rank, got in run_ranks(world, _relay_worker, path, ask):
         assert got == want, rank
 
 
@@ -240,7 +169,7 @@ def test_a_bad_time_on_one_shard_raises_on_every_rank(oi, tmp_path):
     from openintel_b200 import store
     texts, sources, tickers = _synthetic(600, 5, n_tickers=20)
     path = str(tmp_path / "posts.db")
-    conn = _timed_store(path, texts, sources, T0 + np.arange(600) * 60)
+    conn = make_store(path, texts, sources, T0 + np.arange(600) * 60)
     conn.execute("UPDATE posts SET created_at = '2024-01-01T00:00:00' WHERE doc_id = 555")
     conn.commit()
     with store.MentionIndex(conn) as mi:
@@ -249,7 +178,7 @@ def test_a_bad_time_on_one_shard_raises_on_every_rank(oi, tmp_path):
             mi.timeline([tickers[0]], [T0, T0 + DAY])
         assert "doc_id 555" in str(e.value)
     conn.close()
-    res = _run_ranks(2, path, [tickers[0]])
+    res = run_ranks(2, _relay_worker, path, [tickers[0]])
     assert res[1][1].startswith("ValueError") and "doc_id 555" in res[1][1]
     assert res[0][1].startswith("ValueError") and "another shard" in res[0][1]
 
@@ -258,7 +187,7 @@ def test_a_bad_time_on_one_shard_raises_on_every_rank(oi, tmp_path):
 def test_carry_continues_the_chain_across_two_shards(oi):
     texts, sources, tickers = _synthetic(20_000, 99, n_tickers=50)
     cut = 12_345
-    full, (a, b), vocab, pol, spec = _shard_pair(oi, texts, sources, cut)
+    full, (a, b), vocab, pol, spec = shard_pair(oi, texts, sources, cut)
     times = T0 + np.random.default_rng(1).integers(0, 10 * DAY, len(texts))
     full.load_post_times(times)
     a.load_post_times(times[:cut])
@@ -266,7 +195,7 @@ def test_carry_continues_the_chain_across_two_shards(oi):
     edges = [T0 + DAY, T0 + 2 * DAY, T0 + 2 * DAY + 1, T0 + 5 * DAY, T0 + 9 * DAY]
     ids = [vocab.index(t) for t in tickers[:30] if t in vocab] + [vocab.index("calls")]
     srcs = np.array([0 if s == "reddit" else 1 for s in sources])
-    to, di = _lists(full)
+    to, di = lists(full)
     for src in (None, 0, 1):
         s_all, m_all = full.mention_timeline(ids, edges, source=src)
         s_a, m_a = a.mention_timeline(ids, edges, source=src)
@@ -274,7 +203,7 @@ def test_carry_continues_the_chain_across_two_shards(oi):
         assert s_b.tobytes() == s_all.tobytes()
         for x, y in zip(m_b, m_all):
             for xk, yk in zip(x, y):
-                _same_summary(xk, yk)
+                same_summary(xk, yk)
         # the first shard's summary is the summary of the prefix
         for i, t in enumerate(ids):
             d = di[to[t]:to[t + 1]]
@@ -284,7 +213,7 @@ def test_carry_continues_the_chain_across_two_shards(oi):
             bk = np.searchsorted(edges, times[d], side="right") - 1
             for k in range(len(edges) - 1):
                 dk = d[bk == k]
-                _same_summary(m_a[i][k], O.social_summary(pol[dk], spec[dk].astype(np.int32)), (t, k, src))
+                same_summary(m_a[i][k], O.social_summary(pol[dk], spec[dk].astype(np.int32)), (t, k, src))
     for ix in (full, a, b):
         ix.close()
 
@@ -298,33 +227,11 @@ def _raw_call(ix, terms, n, edges, nb, source=-1, carry=None, out_state=None, ou
 
 def test_errors_and_state(oi):
     from openintel_b200 import capi
-    texts = ["$GME to the moon", "gme puts", "calls on AMC", "nothing here", "GME GME dump", "amc squeeze yolo"]
-    pol = np.array([O.lexicon_score(t)[0] for t in texts])
-    spec = np.array([O.lexicon_score(t)[1] for t in texts], dtype=np.uint8)
-    src = np.array([0, 1, 0, 1, 1, 0], dtype=np.uint8)
-    times = T0 + np.array([50, 10, 20, 30, 40, 0]) * 3600
-    edges = [T0, T0 + 24 * 3600, T0 + 48 * 3600]
-    with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
-        ix.load_post_signals(pol, spec, src)
-        ix.load_post_times(times)
-        with pytest.raises(oi.OiError) as e:  # signals and times, no BM25 part
-            ix.mention_timeline([0], edges)
-        assert e.value.status == 5
-    with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
-        vocab = ix.build_bm25_text(texts)
-        with pytest.raises(oi.OiError) as e:  # no signals, no times
-            ix.mention_timeline([0], edges)
-        assert e.value.status == 5 and "signals" in e.value.message
-        ix.load_post_times(times)
-        with pytest.raises(oi.OiError) as e:  # times, no signals
-            ix.mention_timeline([0], edges)
-        assert e.value.status == 5 and "signals" in e.value.message
+    texts, pol, spec, src, times = small_corpus()
+    edges = SMALL_EDGES
     with oi.GpuIndex(n_docs=len(texts), dim=4, max_k=1) as ix:
         vocab = ix.build_bm25_text(texts)
         ix.load_post_signals(pol, spec, src)
-        with pytest.raises(oi.OiError) as e:  # signals, no times
-            ix.mention_timeline([0], edges)
-        assert e.value.status == 5 and "times" in e.value.message
         with pytest.raises(ValueError):
             ix.load_post_times(times[:-1])
         assert ix.L.oi_index_load_post_times(ix.h, None) == 1
@@ -379,7 +286,7 @@ def _cli(module, *args):
 
 def test_timeline_cli_equals_analyze_per_bucket(oi, G, tmp_path):
     db = str(tmp_path / "fixture.db")
-    conn, _, hours = _fixture(G, db)
+    conn, _, hours = fixture_store(G, db)
     conn.close()
     m = G["fixture_posts"]["mock_market"]
     snap = "%r,%r,%d,%d,%r" % (m["last_price"], m["previous_close"], m["volume"], m["avg_volume"], m["iv_rank"])
@@ -401,7 +308,7 @@ def test_timeline_cli_equals_analyze_per_bucket(oi, G, tmp_path):
     r = _cli("timeline", "--store", db, "--since", since, "--until", until, "--every", "1d", "--source", "reddit", "aapl")
     assert r.returncode == 0 and json.loads(r.stdout)["tickers"][0]["timeline"][0]["mentions_by_source"] == {"reddit": 4}
     # errors: stderr and exit 1 for a bad store row, usage errors for bad arguments
-    conn = _timed_store(str(tmp_path / "bad.db"), ["gme moon"], ["reddit"], [T0])
+    conn = make_store(str(tmp_path / "bad.db"), ["gme moon"], ["reddit"], [T0])
     conn.execute("UPDATE posts SET created_at = '2024-01-01 00:00:00'")
     conn.commit()
     conn.close()
