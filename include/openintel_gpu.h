@@ -38,6 +38,7 @@ extern "C" {
 
 #define OI_NO_DOC 0xFFFFFFFFu
 #define OI_MAX_K 1024u
+#define OI_MAX_DIM 24576u /* widest row the cosine kernels search: the wide-row scan keeps the query in 96 KB of shared memory */
 #define OI_UNIQUE_ID_BYTES 128
 #define OI_P2P_HANDLE_BYTES 64
 
@@ -62,7 +63,7 @@ typedef struct {
   int32_t device;       /* CUDA device ordinal */
   uint64_t n_docs;      /* documents held by THIS shard */
   uint64_t doc_base;    /* global id of this shard's first document (SPEC §5) */
-  uint32_t dim;         /* embedding dimension; dim*sizeof(dtype) must be a multiple of 16 */
+  uint32_t dim;         /* embedding dimension <= OI_MAX_DIM; dim*sizeof(dtype) must be a multiple of 16 */
   uint32_t dtype;       /* OI_DTYPE_F32 | OI_DTYPE_BF16: storage type of the embedding matrix */
   uint32_t max_k;       /* largest k any search call will ask for (<= OI_MAX_K) */
   uint32_t max_batch;   /* largest number of queries per search call */

@@ -72,6 +72,9 @@ extern "C" oi_status oi_index_create(const oi_index_desc *desc, oi_index **out) 
   if (desc->dtype != OI_DTYPE_F32 && desc->dtype != OI_DTYPE_BF16) return create_fail(OI_ERR_INVALID_ARG, "dtype must be OI_DTYPE_F32 or OI_DTYPE_BF16");
   const uint32_t esize = desc->dtype == OI_DTYPE_F32 ? 4 : 2;
   if (desc->dim == 0 || (desc->dim * esize) % 16 != 0) return create_fail(OI_ERR_INVALID_ARG, "dim * sizeof(dtype) must be a non-zero multiple of 16 bytes");
+  if (desc->dim > OI_MAX_DIM)
+    return create_fail(OI_ERR_INVALID_ARG, "dim = " + std::to_string(desc->dim) + " exceeds OI_MAX_DIM = " + std::to_string(OI_MAX_DIM) +
+                                               ": no cosine kernel searches rows that wide");
   if (desc->max_k == 0 || desc->max_k > OI_MAX_K) return create_fail(OI_ERR_INVALID_ARG, "max_k must be in 1..1024");
   if (desc->max_batch == 0 || desc->max_batch > 65536) return create_fail(OI_ERR_INVALID_ARG, "max_batch must be in 1..65536");
   if (desc->n_docs + desc->doc_base > 0xFFFFFFFEull) return create_fail(OI_ERR_INVALID_ARG, "doc ids must fit in u32 (doc_base + n_docs <= 2^32 - 2)");

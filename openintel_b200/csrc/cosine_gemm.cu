@@ -124,14 +124,16 @@ __device__ __forceinline__ u64 warp_compact_list(u64 *list, uint32_t n, uint32_t
 // and a tile with a survivor cost the whole SM thousands of cycles.  Returns the new list length.
 __device__ __noinline__ uint32_t gemm_open_group(uint32_t s0, uint32_t s1, uint32_t s2, uint32_t s3, uint32_t s4, uint32_t s5,
                                                  uint32_t s6, uint32_t s7, u64 *buf, uint32_t cnt, float thr_s, u64 thr_key,
-                                                 uint32_t doc, uint32_t doc_end, float nxt_s, const float *lvl, uint32_t *lvl_cnt,
+                                                 uint32_t doc, uint32_t n_in, float nxt_s, const float *lvl, uint32_t *lvl_cnt,
                                                  uint32_t lv) {
   const uint32_t sv[8] = {s0, s1, s2, s3, s4, s5, s6, s7};
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     const float sc = __uint_as_float(sv[e]);
     const u64 key = oi_make_key(sc, doc + e);
-    const bool in_range = doc + e < doc_end;  // rows past the end of the shard are zero-filled by the TMA unit
+    // rows past the end of the shard are zero-filled by the TMA unit.  Counted from the group's first column, not by
+    // global id: doc_base + n_docs may be 2^32 - 2, and the ids of those rows would wrap to 0.
+    const bool in_range = (uint32_t)e < n_in;
     const bool ok = in_range && sc >= thr_s && key > thr_key;
     if (ok) buf[cnt] = key;
     cnt += ok ? 1u : 0u;
@@ -428,9 +430,10 @@ __device__ __forceinline__ void cosine_gemm_body(const CUtensorMap &tmap, const 
             const float cnt_s = climb ? nxt_s : INFINITY;
 #pragma unroll
             for (int g = 0; g < NG; ++g) {
+              const uint32_t c0 = (uint32_t)(hf * W + 8 * g);
               if (__any_sync(0xFFFFFFFFu, gm[g] >= thr_s))
                 cnt = gemm_open_group(v[8 * g], v[8 * g + 1], v[8 * g + 2], v[8 * g + 3], v[8 * g + 4], v[8 * g + 5], v[8 * g + 6],
-                                      v[8 * g + 7], buf, cnt, thr_s, thr_key, p.doc_base + doc0 + hf * W + 8 * g, p.doc_base + p.n_rows,
+                                      v[8 * g + 7], buf, cnt, thr_s, thr_key, p.doc_base + doc0 + c0, n_valid > c0 ? n_valid - c0 : 0u,
                                       cnt_s, my_lvl, my_cnt, lv);
             }
           }

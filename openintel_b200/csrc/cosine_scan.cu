@@ -834,6 +834,8 @@ cudaError_t dispatch_ldg(const OiScanParams &p, uint32_t grid, cudaStream_t st) 
     case 7:
     case 8: return launch_ldg<T, 8, 1>(p, grid, st);
     default: {
+      // the query as f32 (nv * QF = dim floats); oi_index_create refuses dim > OI_MAX_DIM, so this always fits
+      static_assert(OI_MAX_DIM * sizeof(float) <= 96 * 1024, "OI_MAX_DIM must fit the wide-row kernel's query buffer");
       size_t smem = (size_t)p.nv * Elem<T>::QF * sizeof(float);
       if (smem > 96 * 1024) return cudaErrorInvalidValue;
       cudaError_t e = cudaFuncSetAttribute(cosine_scan_generic_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -14,6 +14,7 @@ pub const OI_ERR_COMM: oi_status = 6;
 pub const OI_ERR_UNSUPPORTED: oi_status = 7;
 pub const OI_NO_DOC: u32 = 0xFFFF_FFFF;
 pub const OI_MAX_K: u32 = 1024;
+pub const OI_MAX_DIM: u32 = 24576;
 pub const OI_UNIQUE_ID_BYTES: usize = 128;
 pub const OI_P2P_HANDLE_BYTES: usize = 64;
 pub const OI_DTYPE_F32: u32 = 0;
