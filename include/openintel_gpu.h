@@ -279,6 +279,38 @@ oi_status oi_index_mention_timeline(oi_index *h, const uint32_t *terms, uint32_t
 oi_status oi_index_mention_counts(oi_index *h, const int64_t *edges, uint32_t n_buckets, int32_t source,
                                   uint32_t *out_counts);
 
+/* ---- co-mentions: the posts that mention two terms, counted and summarised (docs/SPEC.md §8d) ---
+ * window[0 .. 1] = [since, until), seconds since the Unix epoch, since < until: the one bucket of the §8b rules, and
+ * only posts inside it (and of `source`, when >= 0) count.  co(a, u) = the number of this shard's posts that mention
+ * both a and u; a post that repeats either term counts once.  co(a, a) = a's own count in the window, and co(a, u) =
+ * co(u, a).  The posts that mention an anchor are marked in a per-post bit mask (one bit per anchor, shard-local doc
+ * ids), so at most OI_MAX_COMENTION_ANCHORS anchors go in one call.  A document-sharded index sums the shards' counts
+ * (integers) and relays the pair states in rank order exactly as oi_index_mention_summary does; a shard without a
+ * posting returns zero counts and the carried states.  Duplicate anchors or pairs are allowed and give identical rows.
+ * OI_ERR_STATE: no BM25 part, no signals or no times loaded.  A refused call changes nothing.  Blocking; reads the
+ * posting lists only, so it works before and after oi_index_bm25_finalize. */
+#define OI_MAX_COMENTION_ANCHORS 64
+
+/* out_counts[i * n_terms + u] = co(anchors[i], u) on this shard, anchor-major, for every term u of the BM25 part
+ * (n_terms as oi_index_read_bm25 reports it), host memory.  n_anchors == 0 is a no-op.
+ * OI_ERR_INVALID_ARG: NULL anchors / window / out_counts, since >= until, source outside -1 .. OI_N_SOURCES - 1, an
+ * anchor id >= the BM25 part's n_terms, more than OI_MAX_COMENTION_ANCHORS anchors.  OI_ERR_OUT_OF_MEMORY: no room for
+ * the counts on the device. */
+oi_status oi_index_comention_counts(oi_index *h, const uint32_t *anchors, uint32_t n_anchors,
+                                    const int64_t *window /* [since, until) */, int32_t source, uint32_t *out_counts);
+
+/* pair j = (anchor_terms[j], terms[j]): the §8a social summary of this shard's posts counted in co(anchor_terms[j],
+ * terms[j]), in doc order, continued from carry_in[j] (NULL = nothing before this shard).  out_state (may be NULL) /
+ * out_summary: [n_pairs]; the state's total is co(a, u), and (a, a) gives the state and summary of
+ * oi_index_mention_timeline for (a, [since, until)) bit for bit.  n_pairs == 0 is a no-op.
+ * OI_ERR_INVALID_ARG: NULL anchor_terms / terms / window / out_summary, since >= until, source outside
+ * -1 .. OI_N_SOURCES - 1, a term or anchor id >= the BM25 part's n_terms, more than OI_MAX_COMENTION_ANCHORS distinct
+ * anchor terms. */
+oi_status oi_index_comention_summary(oi_index *h, const uint32_t *anchor_terms, const uint32_t *terms, uint32_t n_pairs,
+                                     const int64_t *window, int32_t source, double bull_bear_threshold,
+                                     const oi_mention_state *carry_in, oi_mention_state *out_state,
+                                     oi_social_summary *out_summary);
+
 /* ---- tuning / introspection (bench + tests) ------------------------------------------------ */
 /* number of kernels this handle has launched since creation (bench "gpu_launches") */
 uint64_t oi_index_launch_count(const oi_index *h);

@@ -7,6 +7,7 @@ import os
 import numpy as np
 
 NO_DOC = 0xFFFFFFFF
+MAX_COMENTION_ANCHORS = 64  # OI_MAX_COMENTION_ANCHORS: one bit of the per-post mask per anchor
 DTYPE_F32, DTYPE_BF16 = 0, 1
 UNIQUE_ID_BYTES = 128
 P2P_HANDLE_BYTES = 64
@@ -112,6 +113,8 @@ def load_library():
         "oi_index_load_post_times": (st, [H, _vp]),
         "oi_index_mention_timeline": (st, [H, _u32p, C.c_uint32, _vp, C.c_uint32, C.c_int32, C.c_double, _vp, _vp, _vp]),
         "oi_index_mention_counts": (st, [H, _vp, C.c_uint32, C.c_int32, _u32p]),
+        "oi_index_comention_counts": (st, [H, _u32p, C.c_uint32, _vp, C.c_int32, _u32p]),
+        "oi_index_comention_summary": (st, [H, _u32p, _u32p, C.c_uint32, _vp, C.c_int32, C.c_double, _vp, _vp, _vp]),
         "oi_index_launch_count": (C.c_uint64, [H]),
         "oi_index_set_option": (st, [H, C.c_char_p, C.c_int64]),
         "oi_debug_cosine_gemm_scores": (st, [H, _f32p, C.c_uint32, _f32p]),
@@ -320,6 +323,35 @@ class GpuIndex:
         out = np.zeros((getattr(self, "n_terms", 0), nb), dtype=np.uint32)  # no BM25 part: the call refuses
         self._ck(self.L.oi_index_mention_counts(self.h, _addr(e), nb, _source_code(source), _addr(out)))
         return out
+
+    # -- co-mentions (SPEC §8d)
+    def comention_counts(self, anchor_ids, window, source=None):
+        """co[i][u] = the number of this shard's posts in window = [since, until) (of `source` only, when given) that
+        mention both anchor_ids[i] and term u, for every term u of the BM25 part (oi_index_comention_counts; at most
+        MAX_COMENTION_ANCHORS anchors).  -> uint32 [n_anchors][n_terms]"""
+        anchors = np.ascontiguousarray(anchor_ids, dtype=np.uint32).reshape(-1)
+        w = np.ascontiguousarray(window, dtype=np.int64).reshape(-1)
+        if len(w) != 2:
+            raise ValueError("the window is [since, until): two times, not %d" % len(w))
+        out = np.zeros((len(anchors), getattr(self, "n_terms", 0)), dtype=np.uint32)  # no BM25 part: the call refuses
+        self._ck(self.L.oi_index_comention_counts(self.h, _addr(anchors), len(anchors), _addr(w), _source_code(source),
+                                                   _addr(out)))
+        return out
+
+    def comention_summary(self, anchor_ids, term_ids, window, source=None, threshold=0.2, carry=None):
+        """the social summary of this shard's posts in window = [since, until) that mention both anchor_ids[j] and
+        term_ids[j], per pair j (oi_index_comention_summary; at most MAX_COMENTION_ANCHORS distinct anchors), continued
+        from `carry` (the states of the previous shard, or None).  -> (states: MENTION_STATE_DTYPE [n], summaries: list
+        of dicts shaped like GpuLexicon's summary)"""
+        anchors = np.ascontiguousarray(anchor_ids, dtype=np.uint32).reshape(-1)
+        terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
+        w = np.ascontiguousarray(window, dtype=np.int64).reshape(-1)
+        if len(anchors) != len(terms) or len(w) != 2:
+            raise ValueError("need one anchor per term (%d, %d) and a window of two times (%d)" % (len(anchors), len(terms), len(w)))
+        states, sums, cin = self._mention_outputs((len(terms),), carry)
+        self._ck(self.L.oi_index_comention_summary(self.h, _addr(anchors), _addr(terms), len(terms), _addr(w),
+                                                    _source_code(source), threshold, _addr(cin), _addr(states), _addr(sums)))
+        return states, summaries_from_array(sums)
 
     # -- multi-GPU
     @staticmethod

@@ -99,7 +99,8 @@ struct oi_index {
   unsigned char *d_mention_io = nullptr;
   size_t mention_io_bytes = 0;
   // per-post creation times (seconds since the Unix epoch, [n_docs]) for the timelines, independent of the BM25 part
-  // and of the signals; d_timeline_ws: the timeline call's grow-on-demand keys / sort / segment workspace
+  // and of the signals; d_timeline_ws: the grow-on-demand keys / sort / segment workspace of the timeline call, and the
+  // post mask and selection workspace of the co-mention calls
   int64_t *d_times = nullptr;
   bool has_times = false;
   unsigned char *d_timeline_ws = nullptr;

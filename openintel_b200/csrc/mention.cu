@@ -14,8 +14,14 @@
 // the segment offsets, and the same summary body runs once per segment.  The chains of all segments run side by side,
 // so a call costs about its largest segment's chain, plus a fixed cost per segment that dominates when there are
 // millions of tiny ones (DESIGN §4.4).
+//
+// Co-mentions (SPEC §8d): the posts of up to 64 anchors' lists inside a window are marked in a per-post u64 mask (bit i
+// = anchor i).  One pass over all postings, the one of the mention counts, then counts for every term the marked posts
+// of its list; and the marked postings of the pairs' term lists, kept in (pair, doc) order by a stable selection, are
+// the segments the timeline's summary kernel runs over.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
 #include <cstring>
 #include <vector>
 
@@ -122,6 +128,75 @@ __global__ void __launch_bounds__(256) mention_counts_kernel(const u64 *__restri
   }
 }
 
+// ---- co-mentions (SPEC §8d)
+// One thread per posting of the requested anchor lists (start[0 .. n]: their starts in the concatenation, start[n] =
+// total, read here so the host does not wait for it): a post of anchor i's list inside [since, until) and of the source
+// gets bit i of mask[doc].  The window is applied here, so the passes that read the mask read no times.
+__global__ void __launch_bounds__(256) comention_mark_kernel(const u64 *term_off, const uint32_t *doc_ids, const int64_t *times,
+                                                             const uint8_t *flags, const uint32_t *anchors, const u64 *start,
+                                                             uint32_t n, int64_t since, int64_t until, int source, u64 *mask) {
+  const u64 total = start[n];
+  for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
+    uint32_t a = 0, b = n;  // the anchor: start[a] <= p < start[b], as in timeline_keys_kernel
+    while (b - a > 1) {
+      const uint32_t m = (a + b) >> 1;
+      if (start[m] <= p) a = m; else b = m;
+    }
+    const uint32_t doc = doc_ids[term_off[anchors[a]] + (p - start[a])];
+    const int64_t t = times[doc];
+    if (t >= since && t < until && (source < 0 || (flags[doc] >> 1) == source)) atomicOr(mask + doc, 1ull << a);
+  }
+}
+
+// One pass over all postings of the shard with the tile walk of mention_counts_kernel: counts[i * n_terms + t] gets
+// the postings of term t whose post carries bit i of the mask.  The doc ids are streamed and the mask gathered.  The
+// lanes that share the term and the mask word -- the intersection of two matches -- add their popcount with one atomic
+// per set bit, so a head term does not serialise on its counters; a warp whose 32 posts carry no bit does no match.
+__global__ void __launch_bounds__(256) comention_counts_kernel(const u64 *__restrict__ term_off, const uint32_t *__restrict__ doc_ids,
+                                                               const u64 *__restrict__ mask, uint32_t n_terms, u64 n_postings,
+                                                               uint32_t *counts) {
+  const int lane = threadIdx.x & 31;
+  const u64 warp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((u64)gridDim.x * blockDim.x) >> 5;
+  for (u64 tile = warp * OI_BM25_TILE; tile < n_postings; tile += n_warps * OI_BM25_TILE) {
+    const TileTerms tt = bm25_tile_terms(term_off, n_terms, tile, n_postings, lane);
+    uint32_t lo = tt.lo;
+    for (uint32_t u = 0; u < OI_BM25_TILE / 32; ++u) {
+      if (tile + 32u * u >= n_postings) break;  // warp-uniform: the whole warp stays in for the matches below
+      const u64 p = tile + 32u * u + (uint32_t)lane;
+      u64 m = 0;  // no bit: past the end, or a post no anchor marked
+      if (p < n_postings) {
+        lo = bm25_term_of(term_off, lo, tt.hi, p);
+        m = mask[__ldcs(doc_ids + p)];
+      }
+      if (!__any_sync(0xFFFFFFFFu, m != 0)) continue;
+      const uint32_t peers = __match_any_sync(0xFFFFFFFFu, lo) & __match_any_sync(0xFFFFFFFFu, m);
+      if (m && lane == __ffs(peers) - 1) {
+        const uint32_t c = (uint32_t)__popc(peers);
+        for (u64 r = m; r; r &= r - 1) atomicAdd(counts + (u64)(__ffsll((long long)r) - 1) * n_terms + lo, c);
+      }
+    }
+  }
+}
+
+// posting p of the concatenated pair lists (start[0 .. n], start[n] = total) -> key j (pair j), value = the doc id,
+// keep = whether the post carries the mask bit anchor_bit[j] of the pair's anchor
+__global__ void __launch_bounds__(256) comention_pair_keys_kernel(const u64 *term_off, const uint32_t *doc_ids, const u64 *mask,
+                                                                  const uint32_t *terms, const uint32_t *anchor_bit,
+                                                                  const u64 *start, uint32_t n, u64 total, uint32_t *keys,
+                                                                  uint32_t *vals, uint8_t *keep) {
+  for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
+    uint32_t a = 0, b = n;
+    while (b - a > 1) {
+      const uint32_t m = (a + b) >> 1;
+      if (start[m] <= p) a = m; else b = m;
+    }
+    const uint32_t doc = doc_ids[term_off[terms[a]] + (p - start[a])];
+    keys[p] = a;
+    vals[p] = doc;
+    keep[p] = (uint8_t)((mask[doc] >> anchor_bit[a]) & 1u);
+  }
+}
+
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 // the dynamic shared memory of a kernel that stages nb + 1 edges (oi_stage_edges)
@@ -140,15 +215,18 @@ cudaError_t grow(unsigned char *&buf, size_t &cap, size_t want, cudaStream_t st)
   return e;
 }
 
-// What a mention call takes: term ids (summary, timeline), bucket edges and the post times (timeline, counts), and
-// the messages of its NULL-argument and no-bucket refusals.
+// What a mention call takes: term ids (summary, timeline, co-mentions), bucket edges and the post times (timeline,
+// counts, co-mentions: their window is one bucket), the messages of its NULL-argument and no-bucket refusals, and the
+// name of its term ids in a refusal (nullptr: "terms").
 struct MentionCall {
   bool terms, edges;
-  const char *null_args, *no_bucket;
+  const char *null_args, *no_bucket, *ids;
 };
 constexpr MentionCall kSummary{true, false, "NULL terms / out_summary", nullptr};
 constexpr MentionCall kTimeline{true, true, "NULL terms / edges / out_summary", "n_buckets = 0: a timeline needs a bucket"};
 constexpr MentionCall kCounts{false, true, "NULL edges / out_counts", "n_buckets = 0: counts need a bucket"};
+constexpr MentionCall kComentionCounts{true, true, "NULL anchors / window / out_counts", nullptr, "anchors"};
+constexpr MentionCall kComentionPairs{true, true, "NULL anchor_terms / terms / window / out_summary", nullptr, "terms"};
 
 // The state and argument checks of the mention calls, in the order they find a fault: the BM25 part, the signals and
 // the times; no term (OI_OK, nothing to do -- with any pointers); a NULL argument, no bucket, more (term, bucket)
@@ -174,8 +252,29 @@ oi_status mention_check(oi_index *h, const MentionCall &c, const uint32_t *terms
   const uint32_t V = oi_bm25_n_terms(h);
   if (c.terms)
     for (uint32_t i = 0; i < n_terms; ++i)
-      if (terms[i] >= V) return h->fail(OI_ERR_INVALID_ARG, "terms[%u] = %u: the BM25 part has %u terms", i, terms[i], V);
+      if (terms[i] >= V)
+        return h->fail(OI_ERR_INVALID_ARG, "%s[%u] = %u: the BM25 part has %u terms", c.ids ? c.ids : "terms", i, terms[i], V);
   return OI_OK;
+}
+
+// the mask of the co-mention calls: clear it, then bit i of mask[doc] for every post of anchors[i]'s list in [since,
+// until) and of the source.  d_anchors: n <= 64 term ids on the device; d_start: n + 1 u64 for their lists' starts;
+// scan_tmp: the scan's temporaries (scan_bytes of them).
+cudaError_t comention_mark(oi_index *h, cudaStream_t st, const uint32_t *d_anchors, uint32_t n, u64 *d_start, void *scan_tmp,
+                           size_t scan_bytes, const int64_t *window, int32_t source, u64 *d_mask) {
+  const u64 *term_off = oi_bm25_term_offsets(h);
+  cudaError_t e = cudaMemsetAsync(d_mask, 0, (h->desc.n_docs ? h->desc.n_docs : 1) * sizeof(u64), st);
+  if (e != cudaSuccess) return e;
+  timeline_lengths_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(term_off, d_anchors, n, d_start);
+  ++h->launches;
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, d_start, d_start, (int64_t)n + 1, st)) != cudaSuccess) return e;
+  h->launches += 2;
+  // the anchors' postings are not known on the host: a resident grid strides over them
+  comention_mark_kernel<<<4 * h->num_sms, 256, 0, st>>>(term_off, oi_bm25_doc_ids(h), h->d_times, h->d_sig_flags, d_anchors,
+                                                        d_start, n, window[0], window[1], source, d_mask);
+  ++h->launches;
+  return cudaGetLastError();
 }
 
 }  // namespace
@@ -440,6 +539,165 @@ extern "C" oi_status oi_index_mention_counts(oi_index *h, const int64_t *edges, 
     OI_CK(cudaGetLastError());
   }
   OI_CK(cudaMemcpyAsync(out_counts, d_counts, bytes, cudaMemcpyDeviceToHost, st));
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_comention_counts(oi_index *h, const uint32_t *anchors, uint32_t n_anchors, const int64_t *window,
+                                               int32_t source, uint32_t *out_counts) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  const oi_status s = mention_check(h, kComentionCounts, anchors, n_anchors, window, 1, source, out_counts);
+  if (s || n_anchors == 0) return s;
+  if (n_anchors > OI_MAX_COMENTION_ANCHORS)
+    return h->fail(OI_ERR_INVALID_ARG, "n_anchors = %u: at most %d anchors, one mask bit each", n_anchors, OI_MAX_COMENTION_ANCHORS);
+  const uint32_t V = oi_bm25_n_terms(h);
+  const u64 n_out = (u64)n_anchors * V, na1 = (u64)n_anchors + 1;
+  // d_mention_io: anchors u32 [64] | starts u64 [65] | counts u32 [n V] | scan temporaries; the byte count cannot wrap
+  size_t scan_tmp = 0;
+  OI_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)na1, h->stream));
+  const size_t o_start = align16(OI_MAX_COMENTION_ANCHORS * sizeof(uint32_t));
+  const size_t o_counts = align16(o_start + (OI_MAX_COMENTION_ANCHORS + 1) * sizeof(u64));
+  if (n_out > (~(u64)0 - 64 - o_counts - scan_tmp) / sizeof(uint32_t))
+    return h->fail(OI_ERR_OUT_OF_MEMORY, "%u anchors x %u terms of counts do not fit the address space", n_anchors, V);
+  OI_CK(cudaSetDevice(h->desc.device));
+  cudaStream_t st = h->stream;
+  OI_CK(call_begin(h, st));
+  const size_t bytes = n_out * sizeof(uint32_t), o_tmp = align16(o_counts + bytes);
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
+  unsigned char *io = h->d_mention_io;
+  uint32_t *d_anchors = reinterpret_cast<uint32_t *>(io), *d_counts = reinterpret_cast<uint32_t *>(io + o_counts);
+  OI_CK(cudaMemsetAsync(d_counts, 0, bytes, st));
+  const u64 P = oi_bm25_n_postings(h);
+  if (P) {  // a shard without a posting (the token-free shard of a sharded lift) counts nothing
+    // d_timeline_ws: the mask u64 [n_docs]
+    OI_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, (h->desc.n_docs ? h->desc.n_docs : 1) * sizeof(u64), st));
+    u64 *d_mask = reinterpret_cast<u64 *>(h->d_timeline_ws);
+    OI_CK(cudaMemcpyAsync(d_anchors, anchors, n_anchors * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    OI_CK(comention_mark(h, st, d_anchors, n_anchors, reinterpret_cast<u64 *>(io + o_start), io + o_tmp, scan_tmp, window,
+                         source, d_mask));
+    int per_sm = 0;
+    OI_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, comention_counts_kernel, 256, 0));
+    const u64 tiles = (P + OI_BM25_TILE - 1) / OI_BM25_TILE, want = (tiles + 7) / 8;  // 8 warps per CTA
+    const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
+    comention_counts_kernel<<<(unsigned)(want < resident ? want : resident), 256, 0, st>>>(oi_bm25_term_offsets(h), oi_bm25_doc_ids(h),
+                                                                                            d_mask, V, P, d_counts);
+    ++h->launches;
+    OI_CK(cudaGetLastError());
+  }
+  OI_CK(cudaMemcpyAsync(out_counts, d_counts, bytes, cudaMemcpyDeviceToHost, st));
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_comention_summary(oi_index *h, const uint32_t *anchor_terms, const uint32_t *terms, uint32_t n_pairs,
+                                                const int64_t *window, int32_t source, double bull_bear_threshold,
+                                                const oi_mention_state *carry_in, oi_mention_state *out_state,
+                                                oi_social_summary *out_summary) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  // a NULL anchor_terms is refused with the other NULL arguments.  The pairs are keyed by u32 j < n_pairs <= 2^32 - 1.
+  const oi_status s = mention_check(h, kComentionPairs, terms, n_pairs, window, 1, source, anchor_terms ? out_summary : nullptr);
+  if (s || n_pairs == 0) return s;
+  const uint32_t V = oi_bm25_n_terms(h);
+  // the distinct anchor terms, first-seen order, and each pair's mask bit: its anchor's place among them
+  std::vector<uint32_t> anchors, bit(n_pairs);
+  for (uint32_t j = 0; j < n_pairs; ++j) {
+    const uint32_t a = anchor_terms[j];
+    if (a >= V) return h->fail(OI_ERR_INVALID_ARG, "anchor_terms[%u] = %u: the BM25 part has %u terms", j, a, V);
+    uint32_t i = 0;
+    while (i < anchors.size() && anchors[i] != a) ++i;
+    if (i == anchors.size()) {
+      if (i == OI_MAX_COMENTION_ANCHORS)
+        return h->fail(OI_ERR_INVALID_ARG, "anchor_terms[%u] = %u: at most %d distinct anchor terms, one mask bit each", j, a,
+                       OI_MAX_COMENTION_ANCHORS);
+      anchors.push_back(a);
+    }
+    bit[j] = i;
+  }
+  const u64 *term_off = oi_bm25_term_offsets(h);
+  OI_CK(cudaSetDevice(h->desc.device));
+  cudaStream_t st = h->stream;
+  OI_CK(call_begin(h, st));
+
+  // d_mention_io: anchors u32 [64] | anchor starts u64 [65] | terms u32 [n] | mask bits u32 [n] | starts u64 [n + 1] |
+  // carries [n] (when given) | states [n] | summaries [n] | scan temporaries
+  const size_t n = n_pairs, na = anchors.size();
+  size_t scan_tmp = 0, scan_a = 0;
+  OI_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)n + 1, st));
+  OI_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_a, (u64 *)nullptr, (u64 *)nullptr, (int64_t)na + 1, st));
+  if (scan_a > scan_tmp) scan_tmp = scan_a;
+  const size_t o_astart = align16(OI_MAX_COMENTION_ANCHORS * sizeof(uint32_t));
+  const size_t o_terms = align16(o_astart + (OI_MAX_COMENTION_ANCHORS + 1) * sizeof(u64));
+  const size_t o_bit = align16(o_terms + n * sizeof(uint32_t)), o_start = align16(o_bit + n * sizeof(uint32_t));
+  const size_t o_carry = align16(o_start + (n + 1) * sizeof(u64));
+  const size_t o_state = align16(o_carry + (carry_in ? n * sizeof(oi_mention_state) : 0));
+  const size_t o_sum = align16(o_state + n * sizeof(oi_mention_state));
+  const size_t o_tmp = align16(o_sum + n * sizeof(oi_social_summary));
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
+  unsigned char *io = h->d_mention_io;
+  uint32_t *d_anchors = reinterpret_cast<uint32_t *>(io), *d_terms = reinterpret_cast<uint32_t *>(io + o_terms);
+  uint32_t *d_bit = reinterpret_cast<uint32_t *>(io + o_bit);
+  u64 *d_start = reinterpret_cast<u64 *>(io + o_start);
+  oi_mention_state *d_carry = carry_in ? reinterpret_cast<oi_mention_state *>(io + o_carry) : nullptr;
+  oi_mention_state *d_state = reinterpret_cast<oi_mention_state *>(io + o_state);
+  oi_social_summary *d_sum = reinterpret_cast<oi_social_summary *>(io + o_sum);
+  OI_CK(cudaMemcpyAsync(d_anchors, anchors.data(), na * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  OI_CK(cudaMemcpyAsync(d_terms, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  OI_CK(cudaMemcpyAsync(d_bit, bit.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  if (carry_in) OI_CK(cudaMemcpyAsync(d_carry, carry_in, n * sizeof(oi_mention_state), cudaMemcpyHostToDevice, st));
+  timeline_lengths_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(term_off, d_terms, n_pairs, d_start);
+  ++h->launches;
+  OI_CK(cudaGetLastError());
+  OI_CK(cub::DeviceScan::ExclusiveSum(io + o_tmp, scan_tmp, d_start, d_start, (int64_t)n + 1, st));
+  h->launches += 2;
+  u64 total = 0;
+  OI_CK(cudaMemcpyAsync(&total, d_start + n, sizeof(u64), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
+
+  // d_timeline_ws: mask u64 [n_docs] | keys u32 [P] | doc ids u32 [P] | kept keys u32 [P] | kept doc ids u32 [P] |
+  // keep u8 [P] | kept count i64 | segment offsets u64 [n + 1] | select temporaries
+  size_t sel_tmp = 0;
+  if (total)
+    OI_CK(cub::DeviceSelect::Flagged(nullptr, sel_tmp, (const uint32_t *)nullptr, (const uint8_t *)nullptr, (uint32_t *)nullptr,
+                                     (int64_t *)nullptr, (int64_t)total, st));
+  const size_t o_keys = align16((h->desc.n_docs ? h->desc.n_docs : 1) * sizeof(u64));
+  const size_t o_keep = align16(o_keys + 4 * total * sizeof(uint32_t)), o_nsel = align16(o_keep + total);
+  const size_t o_seg = align16(o_nsel + sizeof(int64_t)), o_stmp = align16(o_seg + (n + 1) * sizeof(u64));
+  OI_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, o_stmp + sel_tmp, st));
+  unsigned char *ws = h->d_timeline_ws;
+  u64 *d_mask = reinterpret_cast<u64 *>(ws), *d_seg = reinterpret_cast<u64 *>(ws + o_seg);
+  uint32_t *d_keys = reinterpret_cast<uint32_t *>(ws + o_keys);
+  uint32_t *kept_keys = d_keys + 2 * total, *kept_docs = d_keys + 3 * total;
+  if (total) {
+    OI_CK(comention_mark(h, st, d_anchors, (uint32_t)na, reinterpret_cast<u64 *>(io + o_astart), io + o_tmp, scan_tmp, window,
+                         source, d_mask));
+    comention_pair_keys_kernel<<<oi_grid(total, 256, h->num_sms), 256, 0, st>>>(
+        term_off, oi_bm25_doc_ids(h), d_mask, d_terms, d_bit, d_start, n_pairs, total, d_keys, d_keys + total, ws + o_keep);
+    ++h->launches;
+    OI_CK(cudaGetLastError());
+    // the kept keys past the kept count read 0xFFFFFFFF, above every pair, so the segment search runs over all P of them.
+    // Stable: the concatenation is in (pair, doc) order, so each pair's kept posts stay in doc order.
+    OI_CK(cudaMemsetAsync(kept_keys, 0xFF, total * sizeof(uint32_t), st));
+    int64_t *d_nsel = reinterpret_cast<int64_t *>(ws + o_nsel);
+    OI_CK(cub::DeviceSelect::Flagged(ws + o_stmp, sel_tmp, d_keys, ws + o_keep, kept_keys, d_nsel, (int64_t)total, st));
+    OI_CK(cub::DeviceSelect::Flagged(ws + o_stmp, sel_tmp, d_keys + total, ws + o_keep, kept_docs, d_nsel, (int64_t)total, st));
+    h->launches += 4;  // init + select, twice
+  }
+  timeline_segments_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(kept_keys, total, n, d_seg);
+  ++h->launches;
+  OI_CK(cudaGetLastError());
+  int per_sm = 0;
+  OI_CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mention_timeline_kernel, 128, 0));
+  const u64 resident = (u64)h->num_sms * (u64)(per_sm > 0 ? per_sm : 1);
+  mention_timeline_kernel<<<(unsigned)(n < resident ? n : resident), 128, 0, st>>>(
+      h->d_sig_pol, h->d_sig_flags, total ? kept_docs : nullptr, d_seg, n, source, bull_bear_threshold, d_carry, d_state, d_sum);
+  ++h->launches;
+  OI_CK(cudaGetLastError());
+  if (out_state) OI_CK(cudaMemcpyAsync(out_state, d_state, n * sizeof(oi_mention_state), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaMemcpyAsync(out_summary, d_sum, n * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
   OI_CK(call_end(h, st));
   OI_CK(cudaStreamSynchronize(st));
   return OI_OK;

@@ -151,6 +151,21 @@ def all_reduce_counts(dist, counts, device="cpu"):
     return t.cpu().numpy()
 
 
+def relay_comention_summary(dist, ix, anchor_ids, term_ids, window, source=None, threshold=0.2, device="cpu"):
+    """The shared-post summaries of the pairs (anchor_ids[j], term_ids[j]) over a document-sharded index (SPEC §8d), the
+    same on every rank: the relay of relay_mention_summary over the states of GpuIndex.comention_summary.  The post
+    masks are shard-local; only the states cross ranks.  Every rank passes the same pairs and window.  -> (states,
+    summaries) as GpuIndex.comention_summary returns them."""
+    if dist is None or dist.get_world_size() == 1 or len(term_ids) == 0:
+        return ix.comention_summary(anchor_ids, term_ids, window, source, threshold)
+
+    def run(carry):
+        states, sums = ix.comention_summary(anchor_ids, term_ids, window, source, threshold, carry)
+        return states, capi.summaries_to_array(sums)
+    states, raw = _relay_states(dist, len(term_ids), run, device)
+    return states, capi.summaries_from_array(raw)
+
+
 def broadcast_unique_id(dist, device="cpu"):
     """rank 0 creates the NCCL unique id (C ABI), everybody receives it."""
     import torch

@@ -461,7 +461,9 @@ class MentionIndex:
     embeddings), scores its posts with the GPU PostAnalyzer and loads the signals and source codes next to the BM25
     part.  reports() returns on every rank exactly what analyze.analyze_posts returns for select_posts(source,
     mention=ticker).  timeline() splits the same summaries by creation time (SPEC §8b); mention_counts() counts every
-    term's mentions by creation time and trending() ranks the terms by the surge of their counts (SPEC §8c).  These read
+    term's mentions by creation time and trending() ranks the terms by the surge of their counts (SPEC §8c);
+    comention_counts() counts every term's posts together with tickers in a window and related() ranks the terms by
+    their excess over independence, with the social block of the shared posts (SPEC §8d).  These read
     the post times from `conn` on their first call, so `conn` stays open while the index is used."""
 
     def __init__(self, conn, dist=None, device_index=0):
@@ -480,7 +482,8 @@ class MentionIndex:
                                 (self.doc_base, self.doc_base + self.n_local)).fetchall()
             with capi.GpuLexicon(device_index) as lx:
                 pol, spec, _, _ = lx.analyze([r[1] for r in rows])
-            self.ix.load_post_signals(pol, spec, [SOURCES.index(r[0]) for r in rows])
+            self.source_codes = np.array([SOURCES.index(r[0]) for r in rows], dtype=np.uint8)
+            self.ix.load_post_signals(pol, spec, self.source_codes)
         except Exception:
             self.ix.close()
             raise
@@ -540,7 +543,7 @@ class MentionIndex:
         if err is not None:
             raise ValueError(err)
         self.ix.load_post_times(times)
-        self.times_loaded = True
+        self.times, self.times_loaded = times, True
 
     def _edges(self, edges):
         """the bucket edges as ints, checked; the post times are read from the store and loaded on the first call"""
@@ -585,18 +588,100 @@ class MentionIndex:
         terms with at least min_mentions mentions in the window are ranked; `universe` (tickers, normalised like
         reports()) restricts the ranking to its entries, and one outside the vocabulary is never ranked.  Times are
         seconds since the Unix epoch; sharded, every rank calls with the same arguments and gets the same list."""
-        from . import analyze, trending
+        from . import trending
         t0, t1, t2, k, min_mentions = trending.check_args(baseline_since, since, until, k, min_mentions)
         counts = self.mention_counts([t0, t1, t2], source)
-        mask = None
-        if universe is not None:
-            mask = np.zeros(len(self.vocab), dtype=bool)
-            mask[[self.term_id[w] for w in map(analyze.ticker_key, universe) if w in self.term_id]] = True
-        ids, expected, surge = trending.rank(counts[:, 1], counts[:, 0], t0, t1, t2, k, min_mentions, mask)
+        ids, expected, surge = trending.rank(counts[:, 1], counts[:, 0], t0, t1, t2, k, min_mentions,
+                                             self._universe_mask(universe))
         blocks = self._timeline([self.vocab[t] for t in ids], [t0, t1, t2], source, cfg)
         return [{"ticker": self.vocab[t], "mentions": int(counts[t, 1]), "baseline_mentions": int(counts[t, 0]),
                  "expected": float(x), "surge": float(sg), "social": {"baseline": b[0], "window": b[1]}}
                 for t, x, sg, b in zip(ids, expected, surge, blocks)]
+
+    def _universe_mask(self, universe):
+        """a bool mask over the vocabulary of the universe's entries, normalised like reports(); None for all terms.  An
+        entry outside the vocabulary marks nothing."""
+        from . import analyze
+        if universe is None:
+            return None
+        mask = np.zeros(len(self.vocab), dtype=bool)
+        mask[[self.term_id[w] for w in map(analyze.ticker_key, universe) if w in self.term_id]] = True
+        return mask
+
+    def _comention_batches(self, keys, window, source):
+        """the co-mention counts of the normalised tickers `keys` (distinct, all in the vocabulary) against every term,
+        in device calls of at most capi.MAX_COMENTION_ANCHORS anchors, all-reduced over the shards.  -> per batch,
+        (its keys, int64 [len(keys)][len(vocab)])"""
+        from . import sharding
+        for i in range(0, len(keys), capi.MAX_COMENTION_ANCHORS):
+            batch = keys[i:i + capi.MAX_COMENTION_ANCHORS]
+            counts = self.ix.comention_counts([self.term_id[k] for k in batch], window, self._source_code(source))
+            yield batch, sharding.all_reduce_counts(self.dist, counts, device=self.device)
+
+    def comention_counts(self, tickers, since, until, source=None):
+        """co[i][u] = the number of posts (of `source` only, when given) created in [since, until), seconds since the
+        Unix epoch, that mention both tickers[i] and term u of the vocabulary (SPEC §8d): one device call per shard and
+        batch of at most 64 distinct tickers, and an all-reduce of the shards' counts.  Tickers are normalised like
+        reports(); one outside the vocabulary is never sent to the device and gets a row of zeros.  The post times are
+        read from the store and loaded on the first call; sharded, every rank calls with the same arguments.
+        -> int64 [len(tickers)][len(vocab)], the same on every rank"""
+        from . import analyze
+        window = self._edges([since, until])
+        keys = [analyze.ticker_key(t) for t in tickers]
+        rows = {}
+        for batch, counts in self._comention_batches([k for k in dict.fromkeys(keys) if k in self.term_id], window, source):
+            rows.update(zip(batch, counts))
+        out = np.zeros((len(keys), len(self.vocab)), dtype=np.int64)
+        for i, k in enumerate(keys):
+            if k in rows:
+                out[i] = rows[k]
+        return out
+
+    def _window_posts(self, since, until, source):
+        """N of SPEC §8d: the posts (of `source` only, when given) created in [since, until), over all shards"""
+        from . import sharding
+        inside = (self.times >= since) & (self.times < until)
+        if source is not None:
+            inside &= self.source_codes == self._source_code(source)
+        return int(sharding.all_reduce_counts(self.dist, np.array([np.count_nonzero(inside)]), device=self.device)[0])
+
+    def related(self, tickers, since, until, k, min_co_mentions=1, source=None, universe=None, cfg=fusion.EngineConfig()):
+        """per anchor ticker, in the order given, the terms mentioned together with it in the window [since, until)
+        more often than independence predicts, ranked by SPEC §8d (related.rank): {ticker, mentions (n_a), posts (N),
+        related: at most k entries {ticker, co_mentions, mentions (n_u), expected, score, social}}.  `social` is the
+        "social" block of the posts in the window that mention both, so its total_mentions is co_mentions.  Only terms
+        with at least min_co_mentions co-mentions are ranked; `universe` (tickers, normalised like reports()) restricts
+        the ranking to its entries, and one outside the vocabulary is never ranked.  An anchor outside the vocabulary,
+        or with no post in the window, ranks nothing.  Times are seconds since the Unix epoch; one device call per shard
+        and batch of 64 anchors for the counts, one relay per batch for the social blocks; sharded, every rank calls
+        with the same arguments and gets the same result."""
+        from . import analyze, related, sharding
+        since, until, k, min_co_mentions = related.check_args(since, until, k, min_co_mentions)
+        n_u = self.mention_counts([since, until], source)[:, 0]
+        n_posts = self._window_posts(since, until, source)
+        mask = self._universe_mask(universe)
+        keys = [analyze.ticker_key(t) for t in tickers]
+        found = {}
+        for batch, counts in self._comention_batches([t for t in dict.fromkeys(keys) if t in self.term_id], [since, until],
+                                                     source):
+            ranked = []
+            for key, co in zip(batch, counts):
+                a = self.term_id[key]
+                ranked.append((key, co, int(co[a])) + related.rank(co, n_u, co[a], n_posts, a, k, min_co_mentions, mask))
+            pairs = [(self.term_id[key], int(u)) for key, _, _, ids, _, _ in ranked for u in ids]
+            states, sums = sharding.relay_comention_summary(
+                self.dist, self.ix, np.array([p[0] for p in pairs], dtype=np.uint32),
+                np.array([p[1] for p in pairs], dtype=np.uint32), [since, until], self._source_code(source),
+                cfg.bull_bear_threshold, device=self.device)
+            j = 0
+            for key, co, n_a, ids, expected, score in ranked:
+                found[key] = (n_a, [{"ticker": self.vocab[u], "co_mentions": int(co[u]), "mentions": int(n_u[u]),
+                                     "expected": float(x), "score": float(sc),
+                                     "social": _social_block(states[j + i], sums[j + i])}
+                                    for i, (u, x, sc) in enumerate(zip(ids, expected, score))])
+                j += len(ids)
+        return [{"ticker": key, "mentions": found.get(key, (0, []))[0], "posts": n_posts, "related": found.get(key, (0, []))[1]}
+                for key in keys]
 
     def close(self):
         self.ix.close()

@@ -21,6 +21,8 @@ pub const OI_DTYPE_F32: u32 = 0;
 pub const OI_DTYPE_BF16: u32 = 1;
 /// post sources in store-schema order: 0 = reddit, 1 = bluesky
 pub const OI_N_SOURCES: usize = 2;
+/// anchors of one co-mention call: one bit of the per-post mask each (docs/SPEC.md §8d)
+pub const OI_MAX_COMENTION_ANCHORS: u32 = 64;
 
 #[repr(C)]
 pub struct oi_index {
@@ -148,6 +150,16 @@ extern "C" {
     /// (docs/SPEC.md §8c); edges has n_buckets + 1 entries
     pub fn oi_index_mention_counts(h: *mut oi_index, edges: *const i64, n_buckets: u32, source: i32,
                                    out_counts: *mut u32) -> oi_status;
+    /// co-mention counts of at most OI_MAX_COMENTION_ANCHORS anchors against every term of the BM25 part,
+    /// [n_anchors][n_terms] anchor-major, over the posts in window = [since, until) (docs/SPEC.md §8d)
+    pub fn oi_index_comention_counts(h: *mut oi_index, anchors: *const u32, n_anchors: u32, window: *const i64, source: i32,
+                                     out_counts: *mut u32) -> oi_status;
+    /// per pair (anchor_terms[j], terms[j]): the social summary of the posts in the window that mention both, relayed
+    /// like oi_index_mention_summary
+    pub fn oi_index_comention_summary(h: *mut oi_index, anchor_terms: *const u32, terms: *const u32, n_pairs: u32,
+                                      window: *const i64, source: i32, bull_bear_threshold: f64,
+                                      carry_in: *const oi_mention_state, out_state: *mut oi_mention_state,
+                                      out_summary: *mut oi_social_summary) -> oi_status;
 
     pub fn oi_index_launch_count(h: *const oi_index) -> u64;
     pub fn oi_index_set_option(h: *mut oi_index, name: *const c_char, value: i64) -> oi_status;
