@@ -311,6 +311,38 @@ oi_status oi_index_comention_summary(oi_index *h, const uint32_t *anchor_terms, 
                                      const oi_mention_state *carry_in, oi_mention_state *out_state,
                                      oi_social_summary *out_summary);
 
+/* ---- per-author mention runs: who talks about a term (docs/SPEC.md §8e) ---------------------
+ * An author is the pair (source, author name), numbered by the caller with dense global ids in (source code, UTF-8
+ * name) order.  The run of (term, author) holds the posts of this shard in window = [since, until) (and of `source`,
+ * when >= 0) that mention the term and were written by the author; a post that repeats the term counts once.  All its
+ * fields are integers, so a document-sharded index merges the shards' runs by (term, author): counts and engagement
+ * summed, first_at the min, last_at the max, in any order. */
+
+/* per-post author ids and engagement of THIS shard, n = n_docs, host memory.  The largest id + 1 sets the key width of
+ * oi_index_mention_authors.  Independent of the BM25 part, of the signals and of the times; a rebuilt BM25 part keeps
+ * them.  OI_ERR_INVALID_ARG: NULL author / engagement; a refused call keeps the previous data. */
+oi_status oi_index_load_post_authors(oi_index *h, const uint32_t *author, const uint32_t *engagement);
+
+/* one (term, author) run: `term` is the index into the call's terms[], posts = bullish + bearish + neutral by the
+ * bull/bear threshold, engagement the u64 sum, first_at / last_at the min / max created_at of its posts */
+typedef struct {
+  uint32_t term, author;
+  uint64_t posts, bullish, bearish, speculative, engagement;
+  int64_t first_at, last_at;
+} oi_author_run;
+
+/* the runs of terms[0 .. n_terms) on this shard, sorted by (term index, author id): term i's runs are
+ * out_runs[out_term_runs[i] .. out_term_runs[i + 1]) (out_term_runs: [n_terms + 1], host memory).  Duplicate term ids
+ * each get their own runs.  *out_n_runs = the number of runs.  n_terms == 0 is a no-op.  More runs than `capacity`:
+ * OI_ERR_INVALID_ARG with *out_n_runs = the number needed and nothing else written, so the caller can size its buffer.
+ * OI_ERR_STATE: no BM25 part, no signals, no times or no authors loaded.  OI_ERR_INVALID_ARG: NULL terms / window /
+ * out_term_runs / out_runs / out_n_runs, since >= until, source outside -1 .. OI_N_SOURCES - 1, a term id >= the BM25
+ * part's n_terms, more than 2^31 - 1 postings in the requested lists.  A refused call changes nothing.  Blocking;
+ * reads the posting lists only, so it works before and after oi_index_bm25_finalize. */
+oi_status oi_index_mention_authors(oi_index *h, const uint32_t *terms, uint32_t n_terms, const int64_t *window,
+                                   int32_t source, double bull_bear_threshold, uint64_t capacity, uint64_t *out_term_runs,
+                                   oi_author_run *out_runs, uint64_t *out_n_runs);
+
 /* ---- tuning / introspection (bench + tests) ------------------------------------------------ */
 /* number of kernels this handle has launched since creation (bench "gpu_launches") */
 uint64_t oi_index_launch_count(const oi_index *h);

@@ -54,6 +54,9 @@ MENTION_STATE_DTYPE = np.dtype([("total", "<u8"), ("bullish", "<u8"), ("bearish"
                                 ("speculative", "<u8"), ("by_source", "<u8", (N_SOURCES,)), ("sum", "<f8")])
 # ... and of oi_social_summary
 SOCIAL_SUMMARY_DTYPE = np.dtype([(f, "<u8" if t is C.c_uint64 else "<f8") for f, t in SocialSummary._fields_])
+# oi_author_run: one (term, author) run of SPEC §8e; `term` indexes the call's term ids
+AUTHOR_RUN_DTYPE = np.dtype([("term", "<u4"), ("author", "<u4"), ("posts", "<u8"), ("bullish", "<u8"), ("bearish", "<u8"),
+                             ("speculative", "<u8"), ("engagement", "<u8"), ("first_at", "<i8"), ("last_at", "<i8")])
 
 
 def lib_path():
@@ -115,6 +118,9 @@ def load_library():
         "oi_index_mention_counts": (st, [H, _vp, C.c_uint32, C.c_int32, _u32p]),
         "oi_index_comention_counts": (st, [H, _u32p, C.c_uint32, _vp, C.c_int32, _u32p]),
         "oi_index_comention_summary": (st, [H, _u32p, _u32p, C.c_uint32, _vp, C.c_int32, C.c_double, _vp, _vp, _vp]),
+        "oi_index_load_post_authors": (st, [H, _u32p, _u32p]),
+        "oi_index_mention_authors": (st, [H, _u32p, C.c_uint32, _vp, C.c_int32, C.c_double, C.c_uint64, _u64p, _vp,
+                                          C.POINTER(C.c_uint64)]),
         "oi_index_launch_count": (C.c_uint64, [H]),
         "oi_index_set_option": (st, [H, C.c_char_p, C.c_int64]),
         "oi_debug_cosine_gemm_scores": (st, [H, _f32p, C.c_uint32, _f32p]),
@@ -352,6 +358,37 @@ class GpuIndex:
         self._ck(self.L.oi_index_comention_summary(self.h, _addr(anchors), _addr(terms), len(terms), _addr(w),
                                                     _source_code(source), threshold, _addr(cin), _addr(states), _addr(sums)))
         return states, summaries_from_array(sums)
+
+    # -- author runs (SPEC §8e)
+    def load_post_authors(self, author, engagement):
+        """per-post author ids (dense, global: SPEC §8e) and engagement of this shard, in doc order.  A refused call keeps
+        the previous data."""
+        a = np.ascontiguousarray(author, dtype=np.uint32)
+        e = np.ascontiguousarray(engagement, dtype=np.uint32)
+        if a.ndim != 1 or not len(a) == len(e) == self.n_docs:
+            raise ValueError("need %d author ids and engagements, got %d / %d" % (self.n_docs, a.size, e.size))
+        self._ck(self.L.oi_index_load_post_authors(self.h, _addr(a), _addr(e)))
+
+    def mention_authors(self, term_ids, window, source=None, threshold=0.2, capacity=4096):
+        """the (term, author) runs of this shard's posts in window = [since, until) (of `source` only, when given) that
+        mention term_ids[i] (oi_index_mention_authors), sorted by (term index, author id).  When the runs do not fit
+        `capacity`, the call is made once more with the number the refusal reports.  -> (term_runs uint64 [n + 1]: term
+        i's runs are runs[term_runs[i]:term_runs[i + 1]], runs: AUTHOR_RUN_DTYPE [term_runs[n]])"""
+        terms = np.ascontiguousarray(term_ids, dtype=np.uint32).reshape(-1)
+        w = np.ascontiguousarray(window, dtype=np.int64).reshape(-1)
+        if len(w) != 2:
+            raise ValueError("the window is [since, until): two times, not %d" % len(w))
+        term_runs = np.zeros(len(terms) + 1, dtype=np.uint64)
+        for attempt in range(2):
+            runs = np.zeros(max(int(capacity), 1), dtype=AUTHOR_RUN_DTYPE)
+            n = C.c_uint64(0)
+            s = self.L.oi_index_mention_authors(self.h, _addr(terms), len(terms), _addr(w), _source_code(source), threshold,
+                                                int(capacity), _addr(term_runs), _addr(runs), C.byref(n))
+            if s == 1 and n.value > capacity and attempt == 0:
+                capacity = n.value
+                continue
+            self._ck(s)
+            return term_runs, runs[:n.value]
 
     # -- multi-GPU
     @staticmethod

@@ -105,6 +105,11 @@ struct oi_index {
   bool has_times = false;
   unsigned char *d_timeline_ws = nullptr;
   size_t timeline_ws_bytes = 0;
+  // per-post author ids and engagement ([n_docs] each) for the author runs, independent of the rest; n_authors = the
+  // largest id + 1 (at least 1): the author part of the (term, author) keys
+  uint32_t *d_author = nullptr, *d_engagement = nullptr;
+  u64 n_authors = 0;
+  bool has_authors = false;
 
   // multi-GPU
   OiComm *comm = nullptr;

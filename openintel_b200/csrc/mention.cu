@@ -19,7 +19,12 @@
 // = anchor i).  One pass over all postings, the one of the mention counts, then counts for every term the marked posts
 // of its list; and the marked postings of the pairs' term lists, kept in (pair, doc) order by a stable selection, are
 // the segments the timeline's summary kernel runs over.
+//
+// Author runs (SPEC §8e): with an author id per post, each requested posting inside a window is keyed by (term, author)
+// in a u64; one stable radix sort and a run-length encoding give the (term, author) runs and their post counts, and one
+// pass over the sorted postings, balanced over postings rather than runs, adds the runs' integer fields with atomics.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_run_length_encode.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <cstring>
@@ -197,6 +202,120 @@ __global__ void __launch_bounds__(256) comention_pair_keys_kernel(const u64 *ter
   }
 }
 
+// ---- author runs (SPEC §8e)
+// posting p of the concatenated lists (start[0 .. n], start[n] = total) -> key i * n_authors + author[doc] (term i), or
+// the sentinel n * n_authors for a post outside [since, until) or of another source; value = the doc id
+__global__ void __launch_bounds__(256) author_keys_kernel(const u64 *term_off, const uint32_t *doc_ids, const int64_t *times,
+                                                          const uint8_t *flags, const uint32_t *author, const uint32_t *terms,
+                                                          const u64 *start, uint32_t n, u64 total, int64_t since,
+                                                          int64_t until, int source, u64 n_authors, u64 *keys, uint32_t *vals) {
+  for (u64 p = blockIdx.x * (u64)blockDim.x + threadIdx.x; p < total; p += (u64)gridDim.x * blockDim.x) {
+    uint32_t a = 0, b = n;  // the term: start[a] <= p < start[b], as in timeline_keys_kernel
+    while (b - a > 1) {
+      const uint32_t m = (a + b) >> 1;
+      if (start[m] <= p) a = m; else b = m;
+    }
+    const uint32_t doc = doc_ids[term_off[terms[a]] + (p - start[a])];
+    const int64_t t = times[doc];
+    const bool in = t >= since && t < until && (source < 0 || (flags[doc] >> 1) == source);
+    keys[p] = in ? (u64)a * n_authors + author[doc] : (u64)n * n_authors;
+    vals[p] = doc;
+  }
+}
+
+// term_runs[i] = the first of the n_unique sorted run keys that is >= i * n_authors, i = 0 .. n: term i's runs are
+// [term_runs[i], term_runs[i + 1]), and term_runs[n] -- the sentinel's place -- is the number of runs without the
+// sentinel's
+__global__ void author_term_runs_kernel(const u64 *unique, const int *n_unique, uint32_t n, u64 n_authors, u64 *term_runs) {
+  for (u64 i = blockIdx.x * (u64)blockDim.x + threadIdx.x; i <= n; i += (u64)gridDim.x * blockDim.x) {
+    u64 lo = 0, hi = (u64)*n_unique;
+    const u64 want = i * n_authors;
+    while (lo < hi) {
+      const u64 m = (lo + hi) >> 1;
+      if (unique[m] < want) lo = m + 1; else hi = m;
+    }
+    term_runs[i] = lo;
+  }
+}
+
+// run r: its term and author from its key, its post count from the run length, and the neutral elements of the sums,
+// the min and the max that author_aggregate_kernel fills
+__global__ void author_runs_init_kernel(const u64 *unique, const uint32_t *lengths, u64 n_runs, u64 n_authors,
+                                        oi_author_run *runs) {
+  for (u64 r = blockIdx.x * (u64)blockDim.x + threadIdx.x; r < n_runs; r += (u64)gridDim.x * blockDim.x) {
+    const u64 term = unique[r] / n_authors;
+    oi_author_run x;
+    x.term = (uint32_t)term;
+    x.author = (uint32_t)(unique[r] - term * n_authors);
+    x.posts = lengths[r];
+    x.bullish = x.bearish = x.speculative = x.engagement = 0;
+    x.first_at = INT64_MAX;
+    x.last_at = INT64_MIN;
+    runs[r] = x;
+  }
+}
+
+// One pass over the sorted postings, load-balanced over the postings rather than the runs: one author with tens of
+// thousands of posts is spread over many warps.  A warp takes 32 consecutive postings; the lanes of one run are
+// contiguous because the keys are sorted, so __match_any_sync finds them and a segmented shuffle reduction over
+// [leader, last] gives their engagement sum and time range.  The leader finds its run among the unique keys and adds
+// the popcounts of its peers' bullish / bearish / speculative votes, the sum and the range with one integer atomic
+// each.  The sentinel's postings sort last, so a warp that meets only them is done.
+__global__ void __launch_bounds__(256) author_aggregate_kernel(const u64 *__restrict__ keys, const uint32_t *__restrict__ docs,
+                                                               u64 total, u64 sentinel, const u64 *__restrict__ unique, u64 n_runs,
+                                                               const double *__restrict__ polarity, const uint8_t *__restrict__ flags,
+                                                               const int64_t *__restrict__ times,
+                                                               const uint32_t *__restrict__ engagement, double thr,
+                                                               oi_author_run *runs) {
+  const int lane = threadIdx.x & 31;
+  const u64 warp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((u64)gridDim.x * blockDim.x) >> 5;
+  for (u64 base = warp * 32; base < total; base += n_warps * 32) {
+    const u64 p = base + (uint32_t)lane;
+    const u64 key = p < total ? __ldcs(keys + p) : sentinel;
+    const bool on = key < sentinel;
+    if (!__any_sync(0xFFFFFFFFu, on)) break;  // warp-uniform: every later posting is the sentinel's too
+    bool bull = false, bear = false, spec = false;
+    u64 eng = 0;
+    int64_t t_lo = INT64_MAX, t_hi = INT64_MIN;
+    if (on) {
+      const uint32_t doc = __ldcs(docs + p);
+      const double x = polarity[doc];
+      bull = x > thr;
+      bear = x < -thr;
+      spec = flags[doc] & 1u;
+      eng = engagement[doc];
+      t_lo = t_hi = times[doc];
+    }
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, on ? key : ~0ull);
+    const int last = 31 - __clz(peers);
+    for (int o = 1; o < 32; o <<= 1) {  // lane l ends with [l, min(l + 31, last)]: the leader with its whole segment
+      const u64 e2 = __shfl_down_sync(0xFFFFFFFFu, eng, o);
+      const int64_t lo2 = __shfl_down_sync(0xFFFFFFFFu, t_lo, o), hi2 = __shfl_down_sync(0xFFFFFFFFu, t_hi, o);
+      if (lane + o <= last) {
+        eng += e2;
+        t_lo = lo2 < t_lo ? lo2 : t_lo;
+        t_hi = hi2 > t_hi ? hi2 : t_hi;
+      }
+    }
+    const uint32_t b_bull = __ballot_sync(0xFFFFFFFFu, bull), b_bear = __ballot_sync(0xFFFFFFFFu, bear);
+    const uint32_t b_spec = __ballot_sync(0xFFFFFFFFu, spec);
+    if (on && lane == __ffs(peers) - 1) {
+      u64 lo = 0, hi = n_runs;  // the run: unique[lo] == key
+      while (lo < hi) {
+        const u64 m = (lo + hi) >> 1;
+        if (unique[m] < key) lo = m + 1; else hi = m;
+      }
+      oi_author_run *r = runs + lo;
+      if (const uint32_t c = __popc(b_bull & peers)) atomicAdd(reinterpret_cast<unsigned long long *>(&r->bullish), (u64)c);
+      if (const uint32_t c = __popc(b_bear & peers)) atomicAdd(reinterpret_cast<unsigned long long *>(&r->bearish), (u64)c);
+      if (const uint32_t c = __popc(b_spec & peers)) atomicAdd(reinterpret_cast<unsigned long long *>(&r->speculative), (u64)c);
+      if (eng) atomicAdd(reinterpret_cast<unsigned long long *>(&r->engagement), eng);
+      atomicMin(reinterpret_cast<long long *>(&r->first_at), (long long)t_lo);
+      atomicMax(reinterpret_cast<long long *>(&r->last_at), (long long)t_hi);
+    }
+  }
+}
+
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 // the dynamic shared memory of a kernel that stages nb + 1 edges (oi_stage_edges)
@@ -215,27 +334,30 @@ cudaError_t grow(unsigned char *&buf, size_t &cap, size_t want, cudaStream_t st)
   return e;
 }
 
-// What a mention call takes: term ids (summary, timeline, co-mentions), bucket edges and the post times (timeline,
-// counts, co-mentions: their window is one bucket), the messages of its NULL-argument and no-bucket refusals, and the
-// name of its term ids in a refusal (nullptr: "terms").
+// What a mention call takes: term ids (summary, timeline, co-mentions, authors), bucket edges and the post times
+// (timeline, counts, co-mentions and authors: their window is one bucket), the messages of its NULL-argument and
+// no-bucket refusals, the name of its term ids in a refusal (nullptr: "terms"), and the post authors (author runs).
 struct MentionCall {
   bool terms, edges;
   const char *null_args, *no_bucket, *ids;
+  bool authors;
 };
 constexpr MentionCall kSummary{true, false, "NULL terms / out_summary", nullptr};
 constexpr MentionCall kTimeline{true, true, "NULL terms / edges / out_summary", "n_buckets = 0: a timeline needs a bucket"};
 constexpr MentionCall kCounts{false, true, "NULL edges / out_counts", "n_buckets = 0: counts need a bucket"};
 constexpr MentionCall kComentionCounts{true, true, "NULL anchors / window / out_counts", nullptr, "anchors"};
 constexpr MentionCall kComentionPairs{true, true, "NULL anchor_terms / terms / window / out_summary", nullptr, "terms"};
+constexpr MentionCall kAuthors{true, true, "NULL terms / window / out_term_runs / out_runs / out_n_runs", nullptr, "terms", true};
 
-// The state and argument checks of the mention calls, in the order they find a fault: the BM25 part, the signals and
-// the times; no term (OI_OK, nothing to do -- with any pointers); a NULL argument, no bucket, more (term, bucket)
+// The state and argument checks of the mention calls, in the order they find a fault: the BM25 part, the signals, the
+// times and the authors; no term (OI_OK, nothing to do -- with any pointers); a NULL argument, no bucket, more (term, bucket)
 // segments than 32-bit keys hold, edges that do not increase strictly, the source, the term ids.  Under the lock.
 oi_status mention_check(oi_index *h, const MentionCall &c, const uint32_t *terms, uint32_t n_terms, const int64_t *edges,
                         uint32_t n_buckets, int32_t source, const void *out) {
   if (!oi_bm25_term_offsets(h)) return h->fail(OI_ERR_STATE, "no BM25 part: the posting lists are the mentions");
   if (!h->has_signals) return h->fail(OI_ERR_STATE, "no post signals loaded (oi_index_load_post_signals)");
   if (c.edges && !h->has_times) return h->fail(OI_ERR_STATE, "no post times loaded (oi_index_load_post_times)");
+  if (c.authors && !h->has_authors) return h->fail(OI_ERR_STATE, "no post authors loaded (oi_index_load_post_authors)");
   if (c.terms && n_terms == 0) return OI_OK;
   if ((c.terms && !terms) || (c.edges && !edges) || !out) return h->fail(OI_ERR_INVALID_ARG, "%s", c.null_args);
   if (c.edges && n_buckets == 0) return h->fail(OI_ERR_INVALID_ARG, "%s", c.no_bucket);
@@ -294,6 +416,12 @@ void oi_mention_free(oi_index *h) {
   h->has_times = false;
   h->d_timeline_ws = nullptr;
   h->timeline_ws_bytes = 0;
+  cudaFree(h->d_author);
+  cudaFree(h->d_engagement);
+  h->d_author = nullptr;
+  h->d_engagement = nullptr;
+  h->n_authors = 0;
+  h->has_authors = false;
 }
 
 extern "C" oi_status oi_index_load_post_signals(oi_index *h, const double *polarity, const uint8_t *speculative,
@@ -700,5 +828,144 @@ extern "C" oi_status oi_index_comention_summary(oi_index *h, const uint32_t *anc
   OI_CK(cudaMemcpyAsync(out_summary, d_sum, n * sizeof(oi_social_summary), cudaMemcpyDeviceToHost, st));
   OI_CK(call_end(h, st));
   OI_CK(cudaStreamSynchronize(st));
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_load_post_authors(oi_index *h, const uint32_t *author, const uint32_t *engagement) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  if (!author || !engagement) return h->fail(OI_ERR_INVALID_ARG, "NULL author / engagement");
+  const u64 n = h->desc.n_docs;
+  uint32_t top = 0;
+  for (u64 i = 0; i < n; ++i) top = author[i] > top ? author[i] : top;
+  OI_CK(cudaSetDevice(h->desc.device));
+  if (!h->d_author) {
+    cudaError_t e = cudaMalloc(&h->d_author, (n ? n : 1) * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMalloc(&h->d_engagement, (n ? n : 1) * sizeof(uint32_t));
+    if (e != cudaSuccess) {
+      cudaFree(h->d_author);
+      h->d_author = nullptr;
+      h->d_engagement = nullptr;
+      return h->fail(e == cudaErrorMemoryAllocation ? OI_ERR_OUT_OF_MEMORY : OI_ERR_CUDA, "allocating the post authors failed: %s",
+                     cudaGetErrorString(e));
+    }
+  }
+  OI_CK(call_begin(h, h->stream));
+  h->has_authors = false;  // until the copies have landed
+  if (n) {
+    OI_CK(cudaMemcpyAsync(h->d_author, author, n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    OI_CK(cudaMemcpyAsync(h->d_engagement, engagement, n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  }
+  OI_CK(call_end(h, h->stream));
+  OI_CK(cudaStreamSynchronize(h->stream));
+  h->n_authors = (u64)top + 1;
+  h->has_authors = true;
+  return OI_OK;
+}
+
+extern "C" oi_status oi_index_mention_authors(oi_index *h, const uint32_t *terms, uint32_t n_terms, const int64_t *window,
+                                              int32_t source, double bull_bear_threshold, uint64_t capacity,
+                                              uint64_t *out_term_runs, oi_author_run *out_runs, uint64_t *out_n_runs) {
+  if (!h) return OI_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(h->mu);
+  const oi_status s = mention_check(h, kAuthors, terms, n_terms, window, 1, source,
+                                    out_term_runs && out_runs && out_n_runs ? out_runs : nullptr);
+  if (s || n_terms == 0) return s;
+  const u64 *term_off = oi_bm25_term_offsets(h);
+  const u64 n_authors = h->n_authors, sentinel = (u64)n_terms * n_authors;  // < 2^64: n_terms < 2^32, n_authors <= 2^32
+  OI_CK(cudaSetDevice(h->desc.device));
+  cudaStream_t st = h->stream;
+  OI_CK(call_begin(h, st));
+
+  // d_mention_io: terms u32 [n] | starts u64 [n + 1] | term runs u64 [n + 1] | scan temporaries
+  const size_t n = n_terms;
+  size_t scan_tmp = 0;
+  OI_CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (u64 *)nullptr, (u64 *)nullptr, (int64_t)n + 1, st));
+  const size_t o_start = align16(n * sizeof(uint32_t)), o_truns = align16(o_start + (n + 1) * sizeof(u64));
+  const size_t o_tmp = align16(o_truns + (n + 1) * sizeof(u64));
+  OI_CK(grow(h->d_mention_io, h->mention_io_bytes, o_tmp + scan_tmp, st));
+  unsigned char *io = h->d_mention_io;
+  uint32_t *d_terms = reinterpret_cast<uint32_t *>(io);
+  u64 *d_start = reinterpret_cast<u64 *>(io + o_start), *d_truns = reinterpret_cast<u64 *>(io + o_truns);
+  OI_CK(cudaMemcpyAsync(d_terms, terms, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  timeline_lengths_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(term_off, d_terms, n_terms, d_start);
+  ++h->launches;
+  OI_CK(cudaGetLastError());
+  OI_CK(cub::DeviceScan::ExclusiveSum(io + o_tmp, scan_tmp, d_start, d_start, (int64_t)n + 1, st));
+  h->launches += 2;
+  u64 total = 0;
+  OI_CK(cudaMemcpyAsync(&total, d_start + n, sizeof(u64), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
+  if (total > 0x7FFFFFFFull)  // the run-length encoding counts items in an int
+    return h->fail(OI_ERR_INVALID_ARG, "the requested lists hold %llu postings: at most 2^31 - 1 in one call",
+                   (unsigned long long)total);
+
+  // d_timeline_ws: keys u64 [P] x 2 | doc ids u32 [P] x 2 | run keys u64 [P] | run lengths u32 [P] | run count i32 |
+  // sort / encode temporaries
+  int end_bit = 0;
+  while (end_bit < 64 && (sentinel >> end_bit)) ++end_bit;  // the bits of the largest key, the sentinel
+  size_t sort_tmp = 0, rle_tmp = 0;
+  if (total) {
+    cub::DoubleBuffer<u64> kb(nullptr, nullptr);
+    cub::DoubleBuffer<uint32_t> vb(nullptr, nullptr);
+    OI_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+    OI_CK(cub::DeviceRunLengthEncode::Encode(nullptr, rle_tmp, (const u64 *)nullptr, (u64 *)nullptr, (uint32_t *)nullptr,
+                                             (int *)nullptr, (int)total, st));
+  }
+  const size_t o_vals = align16(2 * total * sizeof(u64)), o_uniq = align16(o_vals + 2 * total * sizeof(uint32_t));
+  const size_t o_len = align16(o_uniq + total * sizeof(u64)), o_nruns = align16(o_len + total * sizeof(uint32_t));
+  const size_t o_wtmp = align16(o_nruns + sizeof(int));
+  OI_CK(grow(h->d_timeline_ws, h->timeline_ws_bytes, o_wtmp + (sort_tmp > rle_tmp ? sort_tmp : rle_tmp), st));
+  unsigned char *ws = h->d_timeline_ws;
+  u64 *d_keys = reinterpret_cast<u64 *>(ws), *d_uniq = reinterpret_cast<u64 *>(ws + o_uniq);
+  uint32_t *d_vals = reinterpret_cast<uint32_t *>(ws + o_vals), *d_len = reinterpret_cast<uint32_t *>(ws + o_len);
+  int *d_nruns = reinterpret_cast<int *>(ws + o_nruns);
+  const u64 *sorted_keys = d_keys;
+  const uint32_t *sorted_docs = d_vals;
+  if (total) {
+    author_keys_kernel<<<oi_grid(total, 256, h->num_sms), 256, 0, st>>>(
+        term_off, oi_bm25_doc_ids(h), h->d_times, h->d_sig_flags, h->d_author, d_terms, d_start, n_terms, total, window[0],
+        window[1], source, n_authors, d_keys, d_vals);
+    ++h->launches;
+    OI_CK(cudaGetLastError());
+    cub::DoubleBuffer<u64> kb(d_keys, d_keys + total);
+    cub::DoubleBuffer<uint32_t> vb(d_vals, d_vals + total);
+    OI_CK(cub::DeviceRadixSort::SortPairs(ws + o_wtmp, sort_tmp, kb, vb, (int64_t)total, 0, end_bit, st));
+    h->launches += 1 + (end_bit + 7) / 8;  // histogram + one pass per 8 bits
+    sorted_keys = kb.Current();
+    sorted_docs = vb.Current();
+    OI_CK(cub::DeviceRunLengthEncode::Encode(ws + o_wtmp, rle_tmp, sorted_keys, d_uniq, d_len, d_nruns, (int)total, st));
+    h->launches += 2;
+  } else {
+    OI_CK(cudaMemsetAsync(d_nruns, 0, sizeof(int), st));
+  }
+  author_term_runs_kernel<<<oi_grid(n + 1, 256, h->num_sms), 256, 0, st>>>(d_uniq, d_nruns, n_terms, n_authors, d_truns);
+  ++h->launches;
+  OI_CK(cudaGetLastError());
+  std::vector<u64> term_runs(n + 1);
+  OI_CK(cudaMemcpyAsync(term_runs.data(), d_truns, (n + 1) * sizeof(u64), cudaMemcpyDeviceToHost, st));
+  OI_CK(cudaStreamSynchronize(st));
+  const u64 n_runs = term_runs[n];
+  *out_n_runs = n_runs;
+  if (n_runs > capacity)
+    return h->fail(OI_ERR_INVALID_ARG, "%llu runs do not fit capacity = %llu", (unsigned long long)n_runs,
+                   (unsigned long long)capacity);
+  if (n_runs) {
+    // d_mention_io (its terms and starts are spent): runs [R]
+    OI_CK(grow(h->d_mention_io, h->mention_io_bytes, n_runs * sizeof(oi_author_run), st));
+    oi_author_run *d_runs = reinterpret_cast<oi_author_run *>(h->d_mention_io);
+    author_runs_init_kernel<<<oi_grid(n_runs, 256, h->num_sms), 256, 0, st>>>(d_uniq, d_len, n_runs, n_authors, d_runs);
+    ++h->launches;
+    OI_CK(cudaGetLastError());
+    author_aggregate_kernel<<<oi_grid(total, 256, h->num_sms), 256, 0, st>>>(
+        sorted_keys, sorted_docs, total, sentinel, d_uniq, n_runs, h->d_sig_pol, h->d_sig_flags, h->d_times, h->d_engagement,
+        bull_bear_threshold, d_runs);
+    ++h->launches;
+    OI_CK(cudaGetLastError());
+    OI_CK(cudaMemcpyAsync(out_runs, d_runs, n_runs * sizeof(oi_author_run), cudaMemcpyDeviceToHost, st));
+  }
+  OI_CK(call_end(h, st));
+  OI_CK(cudaStreamSynchronize(st));
+  memcpy(out_term_runs, term_runs.data(), (n + 1) * sizeof(u64));
   return OI_OK;
 }

@@ -166,6 +166,16 @@ def relay_comention_summary(dist, ix, anchor_ids, term_ids, window, source=None,
     return states, capi.summaries_from_array(raw)
 
 
+def all_gather_runs(dist, runs, device="cpu"):
+    """Every rank's author runs (capi.AUTHOR_RUN_DTYPE, any number per rank) -> the list of all ranks' runs in rank
+    order, the same on every rank (SPEC §8e), as the bytes of all_gather_packed.  `dist` = torch.distributed
+    (initialised) or None for a single shard."""
+    raw = np.ascontiguousarray(runs, dtype=capi.AUTHOR_RUN_DTYPE).view(np.uint8)
+    blob, offs = all_gather_packed(dist, raw, np.array([0, len(raw)]), device=device)
+    offs = offs.astype(np.int64)
+    return [blob[offs[r]:offs[r + 1]].copy().view(capi.AUTHOR_RUN_DTYPE) for r in range(len(offs) - 1)]
+
+
 def broadcast_unique_id(dist, device="cpu"):
     """rank 0 creates the NCCL unique id (C ABI), everybody receives it."""
     import torch

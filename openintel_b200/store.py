@@ -463,8 +463,9 @@ class MentionIndex:
     mention=ticker).  timeline() splits the same summaries by creation time (SPEC §8b); mention_counts() counts every
     term's mentions by creation time and trending() ranks the terms by the surge of their counts (SPEC §8c);
     comention_counts() counts every term's posts together with tickers in a window and related() ranks the terms by
-    their excess over independence, with the social block of the shared posts (SPEC §8d).  These read
-    the post times from `conn` on their first call, so `conn` stays open while the index is used."""
+    their excess over independence, with the social block of the shared posts (SPEC §8d); authors() groups the tickers'
+    posts by author and measures how concentrated the talk is (SPEC §8e).  These read the post times (and authors() the
+    post authors) from `conn` on their first call, so `conn` stays open while the index is used."""
 
     def __init__(self, conn, dist=None, device_index=0):
         self.dist = dist if (dist is not None and dist.get_world_size() > 1) else None
@@ -476,7 +477,7 @@ class MentionIndex:
         self.vocab = sh["vocab"]
         self.term_id = {w: i for i, w in enumerate(self.vocab)}
         self.doc_base, self.n_local = sh["doc_base"], sh["n_local"]
-        self.conn, self.times_loaded = conn, False
+        self.conn, self.times_loaded, self.authors_loaded = conn, False, False
         try:
             rows = conn.execute("SELECT source, text FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
                                 (self.doc_base, self.doc_base + self.n_local)).fetchall()
@@ -682,6 +683,60 @@ class MentionIndex:
                 j += len(ids)
         return [{"ticker": key, "mentions": found.get(key, (0, []))[0], "posts": n_posts, "related": found.get(key, (0, []))[1]}
                 for key in keys]
+
+    def _load_authors(self):
+        """reads this shard's source, author and engagement, numbers the authors and loads the ids next to the BM25 part.
+        An author is (source, name); the ids are global and dense in (source code, UTF-8 name) order (SPEC §8e), so
+        sharded the ranks all-gather their sorted distinct authors, packed as one source byte + the name, and every rank
+        numbers their sorted union."""
+        from . import sharding
+        rows = self.conn.execute("SELECT source, author, engagement FROM posts WHERE doc_id >= ? AND doc_id < ? ORDER BY doc_id",
+                                 (self.doc_base, self.doc_base + self.n_local)).fetchall()
+        keys = [bytes([SOURCES.index(src)]) + name.encode("utf-8") for src, name, _ in rows]
+        mine = sorted(set(keys))
+        if self.dist is not None:
+            blob, offs = capi.pack_texts(mine)
+            blob, offs = sharding.all_gather_packed(self.dist, blob[:int(offs[-1])], offs, device=self.device)
+            raw, offs = blob.tobytes(), offs.astype(np.int64)
+            mine = sorted({raw[offs[i]:offs[i + 1]] for i in range(len(offs) - 1)})
+        ids = {key: i for i, key in enumerate(mine)}
+        self.ix.load_post_authors(np.array([ids[key] for key in keys], dtype=np.uint32),
+                                  np.array([r[2] for r in rows], dtype=np.uint32))
+        self.author_keys = [(SOURCES[key[0]], key[1:].decode("utf-8")) for key in mine]
+        self.authors_loaded = True
+
+    def authors(self, tickers, since, until, k, source=None, cfg=fusion.EngineConfig()):
+        """per ticker, in the order given, who posted about it in the window [since, until) (of `source` only, when
+        given) and how concentrated that talk is (SPEC §8e): {ticker, mentions (P), authors (A), effective_authors, hhi,
+        top_share, engagement, top: at most k entries {source, author, posts, bullish, bearish, neutral, speculative,
+        engagement, first_at, last_at}}, ranked by posts, then engagement, descending, then author.  Tickers are
+        normalised like reports(); one outside the vocabulary, or without a post in the window, gets zeros and no
+        entry.  Times are seconds since the Unix epoch; one device call per shard for all tickers, and the shards' runs
+        are gathered and merged; sharded, every rank calls with the same arguments and gets the same result."""
+        from . import analyze, authors, sharding
+        since, until, k = authors.check_args(since, until, k)
+        window = self._edges([since, until])
+        if not self.authors_loaded:
+            self._load_authors()
+        keys = [analyze.ticker_key(t) for t in tickers]
+        known = [t for t in dict.fromkeys(keys) if t in self.term_id]
+        _, runs = self.ix.mention_authors(np.array([self.term_id[t] for t in known], dtype=np.uint32), window,
+                                          self._source_code(source), cfg.bull_bear_threshold)
+        if self.dist is not None:
+            runs = authors.merge(sharding.all_gather_runs(self.dist, runs, device=self.device))
+        cut = np.searchsorted(runs["term"], np.arange(len(known) + 1))
+        found = {}
+        for i, key in enumerate(known):
+            r = authors.rank(runs[cut[i]:cut[i + 1]], k)
+            top = [{"source": self.author_keys[int(x["author"])][0], "author": self.author_keys[int(x["author"])][1],
+                    "posts": int(x["posts"]), "bullish": int(x["bullish"]), "bearish": int(x["bearish"]),
+                    "neutral": int(x["posts"]) - int(x["bullish"]) - int(x["bearish"]), "speculative": int(x["speculative"]),
+                    "engagement": int(x["engagement"]), "first_at": int(x["first_at"]), "last_at": int(x["last_at"])}
+                   for x in r["top"]]
+            found[key] = {"mentions": r["mentions"], "authors": r["authors"], "effective_authors": r["effective_authors"],
+                          "hhi": r["hhi"], "top_share": r["top_share"], "engagement": r["engagement"], "top": top}
+        none = {"mentions": 0, "authors": 0, "effective_authors": 0.0, "hhi": 0.0, "top_share": 0.0, "engagement": 0, "top": []}
+        return [dict({"ticker": key}, **found.get(key, none)) for key in keys]
 
     def close(self):
         self.ix.close()

@@ -61,6 +61,21 @@ pub struct oi_mention_state {
     pub sum: f64,
 }
 
+/// one (term, author) run of oi_index_mention_authors (docs/SPEC.md §8e); `term` indexes the call's term ids
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct oi_author_run {
+    pub term: u32,
+    pub author: u32,
+    pub posts: u64,
+    pub bullish: u64,
+    pub bearish: u64,
+    pub speculative: u64,
+    pub engagement: u64,
+    pub first_at: i64,
+    pub last_at: i64,
+}
+
 #[repr(C)]
 pub struct oi_index_desc {
     pub struct_size: u32,
@@ -160,6 +175,13 @@ extern "C" {
                                       window: *const i64, source: i32, bull_bear_threshold: f64,
                                       carry_in: *const oi_mention_state, out_state: *mut oi_mention_state,
                                       out_summary: *mut oi_social_summary) -> oi_status;
+    /// per-post author ids (dense, global) and engagement of this shard (docs/SPEC.md §8e)
+    pub fn oi_index_load_post_authors(h: *mut oi_index, author: *const u32, engagement: *const u32) -> oi_status;
+    /// the (term, author) runs of the posts in window = [since, until), sorted by (term index, author id); term i's runs
+    /// are out_runs[out_term_runs[i] .. out_term_runs[i + 1]); more runs than `capacity`: refused with the count needed
+    pub fn oi_index_mention_authors(h: *mut oi_index, terms: *const u32, n_terms: u32, window: *const i64, source: i32,
+                                    bull_bear_threshold: f64, capacity: u64, out_term_runs: *mut u64,
+                                    out_runs: *mut oi_author_run, out_n_runs: *mut u64) -> oi_status;
 
     pub fn oi_index_launch_count(h: *const oi_index) -> u64;
     pub fn oi_index_set_option(h: *mut oi_index, name: *const c_char, value: i64) -> oi_status;
